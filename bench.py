@@ -3,6 +3,7 @@
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W
   python bench.py --config c2|c4|c5 ...                     (the other BASELINE.json configurations as the headline)
+  python bench.py --dump-outputs DIR ...                    (+ the results of the last timed step as DIR/<name>.npy)
 
 Headline workload (BASELINE.json configs[2], "c3", the one the metric is quoted on): a batch of 256 synthetic
 KITTI-shape HDL-64 scans (120 000 points each, 112 x 1440 range image), 10 cut pedestrians / cyclists to insert per
@@ -410,6 +411,9 @@ def run_side(args, json_out):
     print(json.dumps(res), file=json_out, flush=True)
 
 
+DUMP_BYTES = 60 * 10 ** 6          # --dump-outputs: bytes of all arrays at most (under 64 MB with the .npy headers)
+
+
 class Bench:
     """One workload on this rank's GPU: engines, the staged (pinned) batch and the three measurements."""
 
@@ -487,6 +491,45 @@ class Bench:
         self.barrier()
         dev_ms = self.max_over_ranks(max(ev0.elapsed_time(ev) for ev in ev_end))
         return dev_ms, self.eng.launch_count() - launches0
+
+    def dump_outputs(self, steps, out_dir):
+        """Write what the last device-resident step computed, as a caller receives it (Real3DEngine.unpack), to
+        `out_dir/<name>.npy` (float32 / float64): status, output sizes and inserted objects of every scan, and the
+        clouds of a sample of the scans, taken in a seeded order for as long as the dump stays within DUMP_BYTES (so
+        two builds whose outputs have the same sizes dump the same scans)."""
+        eng = self.res_engines[(steps - 1) % len(self.res_engines)]      # _resident_steps deals step i to engine i % n
+        res = eng.unpack(eng.fetch_raw(), raise_on_error=False)
+        ss = self.w["task"] == "ss"
+        obj_id = {name: i for i, name in enumerate(eng.obj_names)}
+        ins = [(s, obj_id[name], rot, eng.classes.index(cls), vis, box) for s, r in enumerate(res)
+               for (name, rot, cls), vis, box in zip(r.inserted, r.visible, r.boxes)]
+        f64 = lambda rows, cols: np.array(rows, dtype=np.float64).reshape(-1, cols)
+        out = {"status": f64([r.status for r in res], 1)[:, 0],
+               "points_per_scan": f64([len(r.velodyne) for r in res], 1)[:, 0],
+               "check_rows_per_scan": f64([len(r.check) for r in res], 1)[:, 0],
+               # scan, object index in the cut-object database, rotation step, class index, visible points
+               "inserted": f64([i[:5] for i in ins], 5),
+               # center x y z, rotation quaternion x y z w, length, width, height
+               "inserted_boxes": f64([[*b["center"].values(), *b["rotation"].values(), b["length"], b["width"], b["height"]]
+                                      for *_, b in ins], 10)}
+        # float32 velodyne + check rows, float64 labels; 8 B per scan reserved for `sample_scans`
+        cloud_bytes = lambda r: 4 * r.velodyne.size + 4 * r.check.size + (8 * len(r.velodyne) if ss else 0)
+        budget = DUMP_BYTES - sum(a.nbytes for a in out.values()) - 8 * self.n_scans
+        pick = []
+        for s in np.random.default_rng(0).permutation(self.n_scans):
+            budget -= cloud_bytes(res[s])
+            if budget < 0:
+                break
+            pick.append(int(s))
+        pick.sort()
+        out["sample_scans"] = np.array(pick, dtype=np.float64)
+        out["velodyne"] = np.concatenate([np.zeros((0, 4), np.float32)] + [res[s].velodyne for s in pick]).astype(np.float32)
+        out["check"] = np.concatenate([np.zeros((0, 5 if ss else 4), np.float32)] + [res[s].check for s in pick]).astype(np.float32)
+        if ss:
+            out["labels"] = np.concatenate([np.zeros(0)] + [res[s].labels for s in pick]).astype(np.float64)
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in out.items():
+            np.save(os.path.join(out_dir, name + ".npy"), a)
 
     # ---- one step alone on one engine + the per-kernel CUDA-event times of exactly that mode -------------------
     def serial(self, steps):
@@ -663,7 +706,14 @@ def main():
     ap.add_argument("--side", default=None, choices=["rich_map_od", "rich_map_ss", "cut_objects"],
                     help="instead of the headline bench: one of the offline tools either side of the path (SURVEY 8f rows "
                          "3-4), GPU numbers from tools/bench_*.py plus the CPU baseline (numpy oracle port, one host core)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (rank 0's batch) to DIR/<name>.npy, so "
+                         "that two builds can be compared output for output on the same seeded inputs")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.side or args.impl != "b200"):
+        ap.error("--dump-outputs applies to the headline B200 path only (not to --side or --impl reference)")
     if args.side:
         run_side(args, json_out)
         return
@@ -705,6 +755,8 @@ def main():
     # ---- device-resident throughput ("value"): the whole device path from the raw points, steps overlapped ----------
     dev_ms, launches = b.resident(args.steps, args.warmup, sampler)
     value = world * n_scans * args.steps / (dev_ms / 1000.0)
+    if args.dump_outputs and rank == 0:
+        b.dump_outputs(args.steps, args.dump_outputs)
     # ---- the same step alone on one engine, and the per-kernel times of exactly that mode ---------------------------
     prof_steps = max(3, min(args.steps, 10))
     serial_ms, prof, stats, results = b.serial(prof_steps)

@@ -4,6 +4,7 @@ import json
 import os
 
 import numpy as np
+import pytest
 
 import bench
 
@@ -75,3 +76,59 @@ def test_timed_mode_model_adds_walker_slot_time_and_streaming_kernels():
     assert abs(m["streaming_kernels_ms_per_step"] - 1.89) < 1e-9
     assert abs(m["sum_ms"] - (m["walker_slot_ms_per_step"] + 1.89)) < 1e-3 and m["measured_ms_per_step"] == 2.95
     assert bench.timed_mode_model("ss", 256, table, cyc, 10, {}, 13.0, sm_count=148)["walker_cta_slots"] == 296
+
+
+@pytest.mark.parametrize("task", ["od", "ss"])
+def test_dump_outputs_writes_the_last_steps_results(tmp_path, monkeypatch, task):
+    """--dump-outputs: the engine that ran the last timed step, float32 / float64 files only, per-scan records of every
+    scan, and the clouds of the scans that fit the byte budget in the seeded order."""
+    from types import SimpleNamespace
+    from pcl_augmentation_b200.engine import ScanResult
+    ss = task == "ss"
+    rng = np.random.default_rng(5)
+    box = {"center": {"x": 1.0, "y": 2.0, "z": 3.0}, "rotation": {"x": 0.0, "y": 0.0, "z": 0.6, "w": 0.8},
+           "length": 4.0, "width": 5.0, "height": 6.0, "class": "Cyclist"}
+
+    def engine(tag):
+        res = [ScanResult(velodyne=rng.normal(size=(10 + s, 4)).astype(np.float32),
+                          labels=rng.integers(0, 260, 10 + s).astype(np.uint32) if ss else np.zeros(0, np.uint32),
+                          check=np.full((s % 3, 5 if ss else 4), tag, np.float32), inserted=[("b.npz", 7 * s, "Cyclist")] * (s % 2),
+                          lines=[], boxes=[box] * (s % 2), visible=[s] * (s % 2), status=tag) for s in range(40)]
+        return SimpleNamespace(obj_names=["a.npz", "b.npz"], classes=["Pedestrian", "Cyclist"],
+                               fetch_raw=lambda: None, unpack=lambda buffers, raise_on_error: res, res=res)
+    engines = [engine(0), engine(1), engine(2)]
+    fake = SimpleNamespace(res_engines=engines, w={"task": task}, n_scans=40)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 8000)
+    bench.Bench.dump_outputs(fake, 5, str(tmp_path))                    # steps 0..4 dealt to engines 0 1 2 0 1
+    got = {p.stem: np.load(p) for p in tmp_path.iterdir()}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert sum(a.nbytes for a in got.values()) <= 8000
+    res = engines[1].res
+    assert np.all(got["status"] == 1) and got["points_per_scan"].tolist() == [10.0 + s for s in range(40)]
+    assert got["check_rows_per_scan"].tolist() == [float(s % 3) for s in range(40)]
+    np.testing.assert_array_equal(got["inserted"], [[s, 1, 7 * s, 1, s] for s in range(1, 40, 2)])
+    np.testing.assert_array_equal(got["inserted_boxes"], [[1, 2, 3, 0, 0, 0.6, 0.8, 4, 5, 6]] * 20)
+    # the longest prefix of the seeded scan order whose clouds fit next to the per-scan records
+    left, want = 8000 - 3360 - 8 * 40, []
+    for s in np.random.default_rng(0).permutation(40):
+        left -= (10 + s) * (24 if ss else 16) + (s % 3) * (20 if ss else 16)
+        if left < 0:
+            break
+        want.append(s)
+    pick = got["sample_scans"].astype(int)
+    assert len(want) >= 3 and pick.tolist() == sorted(want)
+    np.testing.assert_array_equal(got["velodyne"], np.concatenate([res[s].velodyne for s in pick]))
+    assert got["check"].shape == (sum(s % 3 for s in pick), 5 if ss else 4)
+    if ss:
+        np.testing.assert_array_equal(got["labels"], np.concatenate([res[s].labels for s in pick]))
+    else:
+        assert "labels" not in got
+
+
+@pytest.mark.parametrize("extra", [["--side", "cut_objects"], ["--impl", "reference"], ["--steps", "0"]])
+def test_arguments_the_headline_path_cannot_honour_are_refused(tmp_path, extra):
+    import subprocess
+    import sys
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--dump-outputs", str(tmp_path / "d")] + extra,
+                       capture_output=True, text=True, timeout=120)
+    assert p.returncode == 2 and "error" in p.stderr and not (tmp_path / "d").exists()

@@ -96,7 +96,7 @@ def test_full_size_frames_vs_oracle(tmp_path):
         assert n >= 20, (task, n)
 
 
-def test_tilted_boxes_counts_and_indices_vs_cut_bounding_box():
+def test_tilted_boxes_counts_and_indices_vs_cut_bounding_box(tmp_path):
     """General (non yaw-only) quaternions, overlapping boxes, emitted indices and the field-of-view count."""
     from scipy.spatial.transform import Rotation as R
     pcl, labels = synth.make_scan(95, synth.KITTI_SHAPE, synth.make_scene_cars(95, 5))
@@ -123,8 +123,8 @@ def test_tilted_boxes_counts_and_indices_vs_cut_bounding_box():
     pcl = np.vstack((pcl, far))
     labels = np.concatenate((labels, np.full(len(far), 7, dtype=labels.dtype)))
     pts5 = np.hstack((pcl.astype(np.float64), labels.reshape(-1, 1).astype(np.float64)))
-    (calib_path := "/tmp/r3d_calib_test.txt") and open(calib_path, "w").write("\n".join(KITTI_CALIB_LINES) + "\n")
-    calib = coo.read_calib(calib_path)
+    (tmp_path / "calib.txt").write_text("\n".join(KITTI_CALIB_LINES) + "\n")
+    calib = coo.read_calib(str(tmp_path / "calib.txt"))
     cam = co.camera_record(calib, KITTI_IMAGE_SHAPE)
     cuts = co.cut_boxes_batch([(pcl, labels)], [boxes], [[co.EMIT_ANY] * len(boxes)], cameras=[cam], want_index=True)[0]
     hits = 0

@@ -85,11 +85,12 @@ def test_filter_objects_bookkeeping_matches_reference_run():
 
 def test_reference_arm_recipe_lists_existing_reference_files():
     """oracle/build_ref.py (the recipe behind `bench.py --impl reference`, kind "reference"): every file it names exists
-    in the reference tree, and the copy under oracle/_ref is byte-identical (skipped where /root/reference is absent)."""
+    in the reference tree, and the copy under oracle/_ref is byte-identical (skipped where the original project's source
+    tree, build_ref.SRC, is absent: the repository does not carry those source files)."""
     import filecmp
     from oracle import build_ref
     if not os.path.isdir(build_ref.SRC):
-        pytest.skip("no /root/reference here")
+        pytest.skip("the original project's source tree (oracle/build_ref.py SRC) is not present")
     assert build_ref.build(verbose=False)
     for rel in build_ref.FILES:
         src = os.path.join(build_ref.SRC, rel)
