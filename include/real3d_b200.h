@@ -357,6 +357,55 @@ int r3d_engine_walk_profile(r3d_engine* eng, int64_t* cycles, int32_t* tries, in
 /* the engine's cudaStream_t (so callers can bracket work with their own CUDA events) */
 void* r3d_engine_stream(r3d_engine* eng);
 
+/* ------------------------------------------------------------------------------- resident dataset (online) */
+/* A dataset laid out in device memory, owned by the caller, from which r3d_engine_load_resident gathers batches
+ * without any per-point host -> device traffic.  Device arrays (scan i of the store):
+ *   xyzi [point_offsets[i] .. point_offsets[i+1]) x 4 float32 (16-byte aligned), labels the same rows as uint16
+ *   (semantic label & 0xFFFF); boxes [box_offsets[i] .. box_offsets[i+1]) x R3D_BOX_DOUBLES (the records of
+ *   r3d_batch.boxes); OD: maps / map_offsets (n_scans * 2 + 1, byte offsets into maps) / map_dims (n_scans x 2 x 4) in
+ *   the r3d_batch layout; semseg: poses (n_scans x 16).  h_point_offsets / h_box_offsets: HOST copies of the
+ *   offsets (capacity checks and the per-batch maxima without a device read). */
+typedef struct r3d_resident_store {
+    int32_t n_scans;
+    const float* xyzi;
+    const uint16_t* labels;
+    const int64_t* point_offsets;
+    const double* boxes;
+    const int32_t* box_offsets;
+    const uint8_t* maps;
+    const int64_t* map_offsets;
+    const int32_t* map_dims;
+    const double* poses;
+    const int64_t* h_point_offsets;
+    const int32_t* h_box_offsets;
+} r3d_resident_store;
+
+/* How r3d_engine_load_resident draws the class counts of a scan (the insertion keys of the YAML, generate_seed
+ * od/ins:171-187): random != 0 -> number_of_object independent uniform class draws; otherwise fixed_counts[n_classes]
+ * (number_of_classes). */
+int r3d_engine_set_schedule_policy(r3d_engine* eng, int32_t random, int32_t number_of_object, const int32_t* fixed_counts);
+/* Load the store scans indices[0 .. n) (HOST array; duplicates allowed) as the engine's batch and draw their schedules
+ * on the device: class counts and, per (event, class), a uniformly random ordered head of min(max_tries, list length)
+ * distinct sample indices followed by -1 (random.shuffle od/ins:400), from Philox4x32-10 keyed by (seed, epoch, store
+ * index, event, class) — never by the position in the batch, so a scan's draws do not depend on how scans are batched
+ * or sharded.  Input errors are reported before anything is enqueued.  The only host -> device copy is the index list;
+ * everything else is enqueued on the engine stream.  The OD maps are read from the store in place (keep it alive while
+ * the batch is in use). */
+int r3d_engine_load_resident(r3d_engine* eng, const r3d_resident_store* store, const int32_t* indices, int32_t n,
+                             uint64_t seed, uint64_t epoch);
+/* r3d_engine_set_ss_map on a map already in DEVICE memory (no copy; the engine only reads it; keep it alive). */
+int r3d_engine_set_ss_map_device(r3d_engine* eng, const uint8_t* map, int32_t size_x, int32_t size_y, int64_t move_x,
+                                 int64_t move_y);
+/* device -> host copy of the schedule tables of the loaded batch: counts (n x n_classes), perms (n x *n_events x
+ * n_classes x max_tries; may be NULL), *n_events. */
+int r3d_engine_schedule_read(r3d_engine* eng, int32_t* counts, int32_t* perms, int32_t* n_events);
+/* The inserted objects of the last run in DEVICE memory (the r3d_engine_output_device pattern, but enqueued on the
+ * engine stream without a host wait): n_inserted (n), inserted (n x max_events x 4, as r3d_batch_result.inserted),
+ * inserted_box (n x max_events x 8, likewise) and box7 (n x max_events x 7 float32: x, y, z_bottom, length, width,
+ * height, yaw = atan2(m10, m00) in the lidar frame; rows past n_inserted are 0).  Valid until the next load / run. */
+int r3d_engine_inserted_device(r3d_engine* eng, const int32_t** n_inserted, const int32_t** inserted,
+                               const double** inserted_box, const float** box7);
+
 /* debug / parity taps on the resident state of one scan (device -> host), used by the tests */
 int r3d_engine_debug_image(r3d_engine* eng, int scan, double* smooth_out /* rows*cols */);
 int r3d_engine_debug_candidates(r3d_engine* eng, int scan, uint8_t* flags_out /* yaw_steps+1 */,

@@ -57,6 +57,13 @@ class BatchResult(C.Structure):
                 ("inserted_box", C.c_void_p), ("status", C.c_void_p), ("rounds", C.c_void_p), ("out_labels16", C.c_void_p)]
 
 
+class ResidentStore(C.Structure):
+    _fields_ = [("n_scans", C.c_int32), ("xyzi", C.c_void_p), ("labels", C.c_void_p), ("point_offsets", C.c_void_p),
+                ("boxes", C.c_void_p), ("box_offsets", C.c_void_p), ("maps", C.c_void_p), ("map_offsets", C.c_void_p),
+                ("map_dims", C.c_void_p), ("poses", C.c_void_p), ("h_point_offsets", C.c_void_p),
+                ("h_box_offsets", C.c_void_p)]
+
+
 # name -> (restype, argtypes); must list every symbol declared in include/real3d_b200.h
 PROTOTYPES = {
     "r3d_version": (C.c_int, []),
@@ -124,6 +131,12 @@ PROTOTYPES = {
     "r3d_engine_stream": (C.c_void_p, [C.c_void_p]),
     "r3d_engine_debug_image": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "r3d_engine_debug_candidates": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "r3d_engine_set_schedule_policy": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
+    "r3d_engine_load_resident": (C.c_int, [C.c_void_p, C.POINTER(ResidentStore), C.c_void_p, C.c_int32, C.c_uint64, C.c_uint64]),
+    "r3d_engine_set_ss_map_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_int64]),
+    "r3d_engine_schedule_read": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32)]),
+    "r3d_engine_inserted_device": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
+                                             C.POINTER(C.c_void_p)]),
 }
 
 _lib = None

@@ -2,6 +2,7 @@
 // the C ABI declared in include/real3d_b200.h.
 #include "r3d_engine_kernels.cuh"
 #include "r3d_host.h"
+#include "r3d_resident.h"
 
 #include <cmath>
 #include <chrono>
@@ -111,6 +112,14 @@ struct r3d_engine {
     unsigned long long* d_words = nullptr;   // device alias of h_words
     unsigned seq = 0;
     long long* h_offsets = nullptr;     // pinned, 2 * (max_scans + 1)
+    // resident-dataset loads (r3d_engine_load_resident): schedule policy, the pinned index list and the event after its
+    // copy (the list is rewritten only once the previous copy has left it), detection targets of the last run
+    SchedulePolicy policy;
+    bool policy_set = false;
+    int* h_idx = nullptr;
+    cudaEvent_t ev_idx = nullptr;
+    DevBuf<int> idx_dev, n_ins_dev;
+    DevBuf<float> box7;
     // profiling
     bool profile = false;
     double prof_ms[KID_COUNT] = {0};
@@ -397,6 +406,8 @@ extern "C" int r3d_engine_destroy(r3d_engine* eng) {
     }
     if (eng->ev_armed) cudaEventDestroy(eng->ev_armed);
     if (eng->ev_wait) cudaEventDestroy(eng->ev_wait);
+    if (eng->ev_idx) cudaEventDestroy(eng->ev_idx);
+    if (eng->h_idx) cudaFreeHost(eng->h_idx);
     for (int i = 0; i < R3D_MAX_SUB; ++i) if (eng->round_graph[i].exec) cudaGraphExecDestroy(eng->round_graph[i].exec);
     cudaStreamDestroy(eng->stream);
     delete eng;
@@ -526,8 +537,9 @@ static int arm_batch(r3d_engine* eng, bool ingest) {
         eng->fresh = false;
         k_reset_alive<<<dim3(std::max(chunks, 1), n), 256, 0, st>>>(d, n); r3d_count_launch();
         // scene boxes: drop the boxes appended by the previous run
-        R3D_CUDA(cudaMemcpyAsync(eng->boxes.p, eng->boxes0.p, eng->h_boxes.size() * sizeof(Box), cudaMemcpyDeviceToDevice, st));
-        k_box_tests<<<(int)((eng->h_boxes.size() + 127) / 128), 128, 0, st>>>(eng->boxes.p, eng->box_tests.p, (int)eng->h_boxes.size());
+        const size_t slots = (size_t)n * d.max_boxes;
+        R3D_CUDA(cudaMemcpyAsync(eng->boxes.p, eng->boxes0.p, slots * sizeof(Box), cudaMemcpyDeviceToDevice, st));
+        k_box_tests<<<(int)((slots + 127) / 128), 128, 0, st>>>(eng->boxes.p, eng->box_tests.p, (int)slots);
         r3d_count_launch();
     }
     eng->ran = false;
@@ -640,6 +652,106 @@ extern "C" int r3d_engine_load_batch(r3d_engine* eng, const r3d_batch* bt) {
     return arm_batch(eng, true);
 }
 
+extern "C" int r3d_engine_set_schedule_policy(r3d_engine* eng, int32_t random, int32_t number_of_object, const int32_t* fixed_counts) {
+    if (eng) cudaSetDevice(eng->device);
+    if (!eng || (random && number_of_object < 0) || (!random && !fixed_counts))
+        return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_schedule_policy: bad argument");
+    SchedulePolicy p;
+    memset(&p, 0, sizeof(p));
+    p.random = random ? 1 : 0;
+    p.number_of_object = random ? number_of_object : 0;
+    for (int c = 0; !random && c < eng->dev.n_classes; ++c) {
+        if (fixed_counts[c] < 0) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_schedule_policy: negative class count");
+        p.fixed[c] = fixed_counts[c];
+    }
+    eng->policy = p;
+    eng->policy_set = true;
+    return R3D_OK;
+}
+
+extern "C" int r3d_engine_load_resident(r3d_engine* eng, const r3d_resident_store* s, const int32_t* indices, int32_t n,
+                                        uint64_t seed, uint64_t epoch) {
+    if (eng) cudaSetDevice(eng->device);
+    if (!eng || !s || !indices) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: null argument");
+    if (!eng->objects_set || !eng->yaw_set) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: set objects and yaw tables first");
+    if (!eng->policy_set) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: set the schedule policy first");
+    EngineDev& d = eng->dev;
+    if (n <= 0 || n > d.B) return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_load_resident: n_scans exceeds max_scans");
+    if (s->n_scans <= 0 || !s->xyzi || ((uintptr_t)s->xyzi & 15) || !s->labels || !s->point_offsets || !s->box_offsets ||
+        !s->h_point_offsets || !s->h_box_offsets || (!s->boxes && s->h_box_offsets[s->n_scans] > 0))
+        return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: missing store arrays");
+    if (d.task == 1 && (!s->poses || !d.ss_map)) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: semseg needs poses and the map");
+    if (d.task == 0 && (!s->maps || !s->map_offsets || !s->map_dims)) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: OD needs maps");
+    // the checks of r3d_engine_load_batch, on the host copies of the store's offsets
+    std::vector<int> nb(n);
+    int max_n0 = 0;
+    for (int b = 0; b < n; ++b) {
+        const int i = indices[b];
+        if (i < 0 || i >= s->n_scans) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: index out of range");
+        const int64_t cnt = s->h_point_offsets[i + 1] - s->h_point_offsets[i];
+        if (cnt <= 0 || cnt > d.max_points) return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_load_resident: scan larger than max_points (or empty)");
+        max_n0 = std::max(max_n0, (int)cnt);
+        nb[b] = s->h_box_offsets[i + 1] - s->h_box_offsets[i];
+        if (nb[b] > d.max_boxes) return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_load_resident: too many scene boxes");
+    }
+    long long want = eng->policy.number_of_object;
+    if (!eng->policy.random) { want = 0; for (int c = 0; c < d.n_classes; ++c) want += eng->policy.fixed[c]; }
+    if (want + 1 > d.max_events)
+        return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_load_resident: a scan's schedule asks for more objects than max_events - 1 "
+                                          "(create the engine with max_events = objects per scan + 1)");
+    const size_t nperm = (size_t)d.B * d.max_events * d.n_classes * d.max_tries;
+    if (nperm > eng->perms.n) TRY(eng->perms.alloc(nperm));
+    if (!eng->h_idx) {
+        R3D_CUDA(cudaMallocHost((void**)&eng->h_idx, (size_t)d.B * sizeof(int)));
+        R3D_CUDA(cudaEventCreateWithFlags(&eng->ev_idx, cudaEventDisableTiming));
+        TRY(eng->idx_dev.alloc(d.B));
+    }
+    cudaStream_t st = eng->stream;
+    R3D_CUDA(cudaEventSynchronize(eng->ev_idx));
+    memcpy(eng->h_idx, indices, (size_t)n * sizeof(int));
+    R3D_CUDA(cudaMemcpyAsync(eng->idx_dev.p, eng->h_idx, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, st));
+    R3D_CUDA(cudaEventRecord(eng->ev_idx, st));
+    eng->n_scans = n;
+    eng->max_n0 = max_n0;
+    eng->h_nbox0 = nb;
+    const int* idx = eng->idx_dev.p;
+    const int od = d.task == 0;
+    launch_gather_points(*s, idx, n, max_n0, eng->xyzi.p, d.max_points, eng->label.p, d.P, od, (unsigned)d.road_label, st);
+    launch_gather_meta(*s, idx, n, od, eng->n0_arr.p, eng->nbox0_arr.p, eng->od_map_off.p, eng->od_map_dims.p, eng->poses.p,
+                       eng->boxes.p, eng->boxes0.p, d.max_boxes, st);
+    const int slots = n * d.max_boxes;
+    k_box_tests<<<(slots + 127) / 128, 128, 0, st>>>(eng->boxes.p, eng->box_tests.p, slots);
+    r3d_count_launch();
+    if (od) d.od_maps = s->maps;
+    d.perms = eng->perms.p; d.n_perm_events = d.max_events;
+    launch_draw_schedule(idx, n, d.max_events, d.n_classes, d.max_tries, d.class_list_off, eng->policy, seed, epoch, eng->counts.p,
+                         eng->perms.p, st);
+    TRY(r3d_check_launch("r3d_engine_load_resident"));
+    eng->batch_loaded = true;
+    return arm_batch(eng, true);
+}
+
+extern "C" int r3d_engine_set_ss_map_device(r3d_engine* eng, const uint8_t* map, int32_t size_x, int32_t size_y, int64_t move_x,
+                                            int64_t move_y) {
+    if (eng) cudaSetDevice(eng->device);
+    if (!eng || !map || size_x <= 0 || size_y <= 0) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_ss_map_device: bad argument");
+    eng->dev.ss_map = map; eng->dev.ss_sx = size_x; eng->dev.ss_sy = size_y;
+    eng->dev.ss_move_x = move_x; eng->dev.ss_move_y = move_y;
+    return R3D_OK;
+}
+
+extern "C" int r3d_engine_schedule_read(r3d_engine* eng, int32_t* counts, int32_t* perms, int32_t* n_events) {
+    if (eng) cudaSetDevice(eng->device);
+    if (!eng || !counts || !n_events || !eng->batch_loaded) return r3d_fail(R3D_ERR_ARG, "r3d_engine_schedule_read: bad argument or no batch");
+    const EngineDev& d = eng->dev;
+    R3D_CUDA(engine_wait(eng));
+    const size_t n = (size_t)eng->n_scans;
+    R3D_CUDA(cudaMemcpy(counts, d.counts, n * d.n_classes * sizeof(int), cudaMemcpyDeviceToHost));
+    if (perms) R3D_CUDA(cudaMemcpy(perms, d.perms, n * d.n_perm_events * d.n_classes * d.max_tries * sizeof(int), cudaMemcpyDeviceToHost));
+    *n_events = d.n_perm_events;
+    return R3D_OK;
+}
+
 extern "C" int r3d_engine_reset_batch(r3d_engine* eng) {
     if (eng) cudaSetDevice(eng->device);
     if (!eng || !eng->batch_loaded) return r3d_fail(R3D_ERR_ARG, "r3d_engine_reset_batch: no batch loaded");
@@ -651,8 +763,9 @@ extern "C" int r3d_engine_rearm_batch(r3d_engine* eng, int from_raw_points) {
     if (!eng || !eng->batch_loaded) return r3d_fail(R3D_ERR_ARG, "r3d_engine_rearm_batch: no batch loaded");
     if (!from_raw_points) return arm_batch(eng, false);
     // the whole device path from the resident float4 points again: scene boxes, spherical ingest, spatial indices
-    R3D_CUDA(cudaMemcpyAsync(eng->boxes.p, eng->boxes0.p, eng->h_boxes.size() * sizeof(Box), cudaMemcpyDeviceToDevice, eng->stream));
-    k_box_tests<<<(int)((eng->h_boxes.size() + 127) / 128), 128, 0, eng->stream>>>(eng->boxes.p, eng->box_tests.p, (int)eng->h_boxes.size());
+    const size_t slots = (size_t)eng->n_scans * eng->dev.max_boxes;
+    R3D_CUDA(cudaMemcpyAsync(eng->boxes.p, eng->boxes0.p, slots * sizeof(Box), cudaMemcpyDeviceToDevice, eng->stream));
+    k_box_tests<<<(int)((slots + 127) / 128), 128, 0, eng->stream>>>(eng->boxes.p, eng->box_tests.p, (int)slots);
     r3d_count_launch();
     return arm_batch(eng, true);
 }
@@ -972,6 +1085,20 @@ extern "C" int r3d_engine_output_device(r3d_engine* eng, const float** out_xyzi,
     if (out_offsets_host) memcpy(out_offsets_host, eng->h_offsets, (n + 1) * sizeof(long long));
     if (check_offsets_host) memcpy(check_offsets_host, eng->h_offsets + eng->dev.B + 1, (n + 1) * sizeof(long long));
     return R3D_OK;
+}
+
+extern "C" int r3d_engine_inserted_device(r3d_engine* eng, const int32_t** n_inserted, const int32_t** inserted,
+                                          const double** inserted_box, const float** box7) {
+    if (eng) cudaSetDevice(eng->device);
+    if (!eng || !eng->ran) return r3d_fail(R3D_ERR_ARG, "r3d_engine_inserted_device: run first");
+    const EngineDev& d = eng->dev;
+    if (!eng->n_ins_dev.p) { TRY(eng->n_ins_dev.alloc(d.B)); TRY(eng->box7.alloc((size_t)d.B * d.max_events * 7)); }
+    launch_inserted_targets(eng->st.p, eng->inserted_box.p, eng->n_scans, d.max_events, eng->n_ins_dev.p, eng->box7.p, eng->stream);
+    if (n_inserted) *n_inserted = eng->n_ins_dev.p;
+    if (inserted) *inserted = eng->inserted.p;
+    if (inserted_box) *inserted_box = eng->inserted_box.p;
+    if (box7) *box7 = eng->box7.p;
+    return r3d_check_launch("r3d_engine_inserted_device");
 }
 
 extern "C" int r3d_engine_fetch(r3d_engine* eng, r3d_batch_result* res) {

@@ -71,6 +71,27 @@ def draw_schedule(config, list_lens, tries=MAX_NUM_TRIES):
     return counts, _permutation_heads(int(counts.sum()) + 1, list_lens, tries)
 
 
+def read_kitti_frame(dataset, idx, maps_path):
+    """One KITTI frame as the engine takes it: (xyzi, labels, scene annotation lines, {'Road', 'Sidewalk'} maps)."""
+    xyzi, labels, name = dataset.read_frame(idx)
+    with open(f'{dataset.data_path}/label_2/{name}.txt') as f:
+        box_lines = [line for line in f if len(line.strip()) > 0]                     # od/ins:133-157
+    maps = {}
+    for key, sub in (('Road', 'road_maps'), ('Sidewalk', 'pedestrian_area')):        # od/ins:361-362
+        with np.load(f'{maps_path}/maps/{sub}/npz/{name}.npz', allow_pickle=True) as z:
+            maps[key] = {'map': z['map'], 'min_x': z['min_x'], 'min_y': z['min_y']}
+    return xyzi, labels, box_lines, maps
+
+
+def read_semantic_kitti_frame(dataset, idx):
+    """One SemanticKITTI (or Waymo adapter) frame as the engine takes it: (xyzi, labels, lidar->world pose, scene
+    annotation lines)."""
+    xyzi, labels, pose, anno_path, _ = dataset.read_frame(idx)
+    with open(anno_path) as f:
+        box_lines = [line for line in f if len(line.strip()) > 0]
+    return xyzi, labels, pose, box_lines
+
+
 def _marker(out_dir, name):
     return f'{out_dir}/added_objects/{name}.txt'
 
@@ -244,13 +265,7 @@ def augment_kitti(config, batch_size=64, yaw_steps=360, folder_number=None, engi
                     log(f'{name}: already in progress')
                     continue
                 claimed.add(name)
-                xyzi, labels, _ = dataset.read_frame(idx)
-                with open(f'{dataset.data_path}/label_2/{name}.txt') as f:
-                    box_lines = [line for line in f if len(line.strip()) > 0]                     # od/ins:133-157
-                maps = {}
-                for key, sub in (('Road', 'road_maps'), ('Sidewalk', 'pedestrian_area')):        # od/ins:361-362
-                    with np.load(f'{maps_path}/maps/{sub}/npz/{name}.npz', allow_pickle=True) as z:
-                        maps[key] = {'map': z['map'], 'min_x': z['min_x'], 'min_y': z['min_y']}
+                xyzi, labels, box_lines, maps = read_kitti_frame(dataset, idx, maps_path)
                 counts, perms = draw_schedule(config, list_lens)
                 scans.append(ScanInput(xyzi=xyzi, labels=labels, box_lines=box_lines, counts=counts, perms=perms, maps=maps))
                 names.append(name)
@@ -323,9 +338,7 @@ def augment_semantic_kitti(config, sequence, batch_size=64, yaw_steps=360, folde
                     log(f'{sequence}/{name}: already in progress')
                     continue
                 claimed.add(name)
-                xyzi, labels, pose, anno_path, _ = dataset.read_frame(indices[k])
-                with open(anno_path) as f:
-                    box_lines = [line for line in f if len(line.strip()) > 0]
+                xyzi, labels, pose, box_lines = read_semantic_kitti_frame(dataset, indices[k])
                 counts, perms = draw_schedule(config, list_lens)
                 scans.append(ScanInput(xyzi=xyzi, labels=labels, box_lines=box_lines, counts=counts, perms=perms, pose=pose))
                 names.append(name)

@@ -46,6 +46,20 @@ class ScanResult:
     extra: dict = field(default_factory=dict)
 
 
+def _cuda_tensor(ptr, shape, typestr, dtype):
+    """CUDA tensor that aliases ``prod(shape)`` elements of library-owned device memory at ``ptr`` (no copy)."""
+    import torch
+    dev = torch.device("cuda", torch.cuda.current_device())
+    if shape[0] == 0:
+        return torch.empty(shape, dtype=dtype, device=dev)
+
+    class _View:
+        def __init__(self):
+            self.__cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (int(ptr), False), "version": 3,
+                                             "strides": None}
+    return torch.as_tensor(_View(), device=dev)
+
+
 def _pinned(shape, dtype):
     """numpy array backed by page-locked host memory (owned by a torch tensor kept alive on the array)."""
     import torch
@@ -141,6 +155,7 @@ class Real3DEngine:
                                                       int(mv[1])), "set_ss_map")
         self._keep = []
         self._n_scans = 0
+        self._policy_set = False
         # labels/<frame>.label exists only in the semseg outputs (ss/ds:82-84); OD writes velodyne + check + label_2
         self.fetch_labels = (task == 'ss') if fetch_labels is None else bool(fetch_labels)
 
@@ -349,17 +364,65 @@ class Real3DEngine:
         off, coff = np.zeros(n + 1, dtype=np.int64), np.zeros(n + 1, dtype=np.int64)
         _lib.check(self.lib.r3d_engine_output_device(self.handle, C.byref(px), C.byref(pl), C.byref(pc), off.ctypes.data,
                                                      coff.ctypes.data), "output_device")
-
-        class _View:
-            def __init__(self, ptr, shape, typestr):
-                self.__cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (int(ptr), False), "version": 3,
-                                                 "strides": None}
-        dev = torch.device("cuda", torch.cuda.current_device())
         total, total_c = int(off[n]), int(coff[n])
-        view = lambda ptr, shape, ts, dt: (torch.as_tensor(_View(ptr.value, shape, ts), device=dev) if shape[0] > 0
-                                           else torch.empty(shape, dtype=dt, device=dev))
-        return {"xyzi": view(px, (total, 4), "<f4", torch.float32), "labels": view(pl, (total,), "<i4", torch.int32),
-                "check": view(pc, (total_c, 5), "<f4", torch.float32), "offsets": off, "check_offsets": coff}
+        return {"xyzi": _cuda_tensor(px.value, (total, 4), "<f4", torch.float32),
+                "labels": _cuda_tensor(pl.value, (total,), "<i4", torch.int32),
+                "check": _cuda_tensor(pc.value, (total_c, 5), "<f4", torch.float32), "offsets": off, "check_offsets": coff}
+
+    # ------------------------------------------------------------------------------- resident dataset (online)
+    def set_schedule_policy(self):
+        """``insertion.random`` / ``number_of_object`` / ``number_of_classes`` of the config -> the device-side draw of
+        the class counts (``generate_seed`` od/ins:171-187)."""
+        ins = self.config['insertion']
+        rand = bool(ins.get('random', True))
+        fixed = np.zeros(_lib.R3D_MAX_CLASSES, dtype=np.int32)
+        if not rand:
+            fixed[:len(self.classes)] = np.asarray(ins['number_of_classes'], dtype=np.int32)
+        _lib.check(self.lib.r3d_engine_set_schedule_policy(self.handle, int(rand), int(ins.get('number_of_object', 0)),
+                                                           fixed.ctypes.data), "set_schedule_policy")
+        self._policy_set = True
+
+    def load_resident(self, store, indices, seed, epoch):
+        """Gather the scans ``indices`` (store rows, duplicates allowed) of a device-resident store
+        (``online.ResidentDataset``) as the batch and draw their schedules on the device for (``seed``, ``epoch``).  Only
+        the index list crosses PCIe; a scan's draws depend on (seed, epoch, store index), not on its place in the batch."""
+        if not self._policy_set:
+            self.set_schedule_policy()
+        idx = np.ascontiguousarray(np.asarray(indices, dtype=np.int64).astype(np.int32))
+        self._keep = [store, idx]
+        self._n_scans = len(idx)
+        mask = (1 << 64) - 1
+        _lib.check(self.lib.r3d_engine_load_resident(self.handle, C.byref(store.abi), idx.ctypes.data, len(idx),
+                                                     int(seed) & mask, int(epoch) & mask), "load_resident")
+
+    def set_ss_map_device(self, map_u8, move_x, move_y):
+        """Semseg: read the sequence map from a uint8 CUDA tensor [size_x, size_y] in place (kept alive by the caller)."""
+        _lib.check(self.lib.r3d_engine_set_ss_map_device(self.handle, map_u8.data_ptr(), int(map_u8.shape[0]),
+                                                         int(map_u8.shape[1]), int(move_x), int(move_y)), "set_ss_map_device")
+
+    def schedule_read(self):
+        """(counts int32 [n, classes], perms int32 [n, events, classes, max_tries]) of the loaded batch, on the host."""
+        n, nc = self._n_scans, len(self.classes)
+        counts, ne = np.zeros((n, nc), dtype=np.int32), C.c_int32()
+        _lib.check(self.lib.r3d_engine_schedule_read(self.handle, counts.ctypes.data, None, C.byref(ne)), "schedule_read")
+        perms = np.zeros((n, ne.value, nc, self.max_tries), dtype=np.int32)
+        _lib.check(self.lib.r3d_engine_schedule_read(self.handle, counts.ctypes.data, perms.ctypes.data, C.byref(ne)),
+                   "schedule_read")
+        return counts, perms
+
+    def inserted_device(self):
+        """The inserted objects of the last run as CUDA tensors aliasing the engine's buffers, enqueued on the engine
+        stream: ``n_inserted`` int32 [n], ``inserted`` int32 [n, max_events, 4] (object id, rotation step, class index,
+        visible points) and ``boxes`` float32 [n, max_events, 7] (x, y, z_bottom, length, width, height, yaw); rows
+        past ``n_inserted`` are padding.  Valid until the engine is loaded or run again."""
+        import torch
+        n, e = self._n_scans, self.max_events
+        pn, pi, pb, p7 = C.c_void_p(), C.c_void_p(), C.c_void_p(), C.c_void_p()
+        _lib.check(self.lib.r3d_engine_inserted_device(self.handle, C.byref(pn), C.byref(pi), C.byref(pb), C.byref(p7)),
+                   "inserted_device")
+        return {"n_inserted": _cuda_tensor(pn.value, (n,), "<i4", torch.int32),
+                "inserted": _cuda_tensor(pi.value, (n, e, 4), "<i4", torch.int32),
+                "boxes": _cuda_tensor(p7.value, (n, e, 7), "<f4", torch.float32)}
 
     def unpack(self, buffers, raise_on_error=True):
         """Per-scan output records in the reference's formats."""
