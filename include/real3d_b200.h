@@ -406,6 +406,50 @@ int r3d_engine_schedule_read(r3d_engine* eng, int32_t* counts, int32_t* perms, i
 int r3d_engine_inserted_device(r3d_engine* eng, const int32_t** n_inserted, const int32_t** inserted,
                                const double** inserted_box, const float** box7);
 
+/* World augmentation of resident batches: the random_world_flip / random_world_rotation / random_world_scaling steps
+ * that detection recipes run after GT insertion, applied to the points and boxes of each scan together.  Per scan b
+ * one Philox4x32-10 call (key = the schedule key of (seed, epoch), counter = (0, 0xFFFFFFFF, store index, epoch low
+ * word), a stream the schedule draws never use) gives four 24-bit uniforms u0..u3:
+ *   fx = u0 < flip_x_prob, fy = u1 < flip_y_prob, theta = rot_max * (2 u2 - 1), k = scale_lo + (scale_hi - scale_lo) u3,
+ *   c = cosf(theta), s = sinf(theta).
+ * A point (x, y, z) becomes, in float32 without contraction: x1 = fy ? -x : x, y1 = fx ? -y : y (flip along x negates
+ * y, flip along y negates x), x' = (c x1 - s y1) k, y' = (s x1 + c y1) k, z' = z k.  Intensity and labels are kept.
+ * A box centre follows the same arithmetic, its dimensions are multiplied by k, and its heading h becomes -h (flip x),
+ * then -(h + pi) (flip y), then h + theta, wrapped to [-pi, pi).  A scan's parameters depend on (seed, epoch, store
+ * index) only, like its schedule. */
+typedef struct r3d_world_aug {
+    float flip_x_prob, flip_y_prob;  /* in [0, 1] */
+    float rot_max;                   /* in [0, pi] */
+    float scale_lo, scale_hi;        /* 0 < scale_lo <= scale_hi */
+} r3d_world_aug;
+
+/* The world augmentation of the following r3d_engine_load_resident calls (NULL: off).  While it is on, each resident
+ * load draws world[n][8] = (fx, fy, theta, c, s, k, 0, 0) on the device and the run writes transformed output points
+ * and check rows; with it off a resident load enqueues what it enqueues without this call.  r3d_engine_load_batch
+ * never applies it. */
+int r3d_engine_set_world_aug(r3d_engine* eng, const r3d_world_aug* policy);
+/* DEVICE pointer to the [n][8] world parameters of the loaded batch; fails unless that batch was loaded by
+ * r3d_engine_load_resident with the world augmentation on.  Valid until the next load. */
+int r3d_engine_world_device(r3d_engine* eng, const float** params);
+/* Detection targets of inserted objects (object detection engines): dims3 (HOST, n_objects x 3) is the unpadded KITTI
+ * (l, w, h) of each cut object; class_target (HOST, n_classes) maps an insertion class to its target class id
+ * (1-based, 0 = not a target). */
+int r3d_engine_set_object_targets(r3d_engine* eng, const float* dims3, const int32_t* class_target);
+/* Every ground-truth box of each augmented scan of the last run, as detection targets in DEVICE buffers the caller
+ * owns: out_box7 [n][max_targets][7] float32 (x, y, z_center, dx, dy, dz, heading) in the engine's lidar frame,
+ * out_class [n][max_targets] int32 (0 = padding), out_count [n]; rows past a scan's count are zero.  The scene boxes
+ * come first, in store order, then the inserted objects in insertion order.  scene_box7 / scene_class (DEVICE) hold
+ * one target record and class id per box record of the store (indexed like its boxes through box_offsets); a class
+ * of 0 skips the box.  An inserted object's box is (cx, cy, cz_bottom + h / 2, l, w, h, atan2(m10, m00) - pi / 2 wrapped
+ * to [-pi, pi)) from its inserted_box record and dims3.  With the world augmentation on, the boxes are transformed
+ * as the points are.  Enqueued on the engine stream after the run.  Errors, reported before anything is enqueued: no
+ * run yet, a batch not loaded by r3d_engine_load_resident, a semseg engine, no r3d_engine_set_object_targets, or
+ * max_targets below a scan's kept scene boxes + max_events - 1.  To check the last one the engine reads scene_class
+ * back to the host the first time it sees the array, and assumes its contents do not change afterwards. */
+int r3d_engine_targets_device(r3d_engine* eng, const r3d_resident_store* store, const float* scene_box7,
+                              const int32_t* scene_class, int32_t max_targets, float* out_box7, int32_t* out_class,
+                              int32_t* out_count);
+
 /* debug / parity taps on the resident state of one scan (device -> host), used by the tests */
 int r3d_engine_debug_image(r3d_engine* eng, int scan, double* smooth_out /* rows*cols */);
 int r3d_engine_debug_candidates(r3d_engine* eng, int scan, uint8_t* flags_out /* yaw_steps+1 */,

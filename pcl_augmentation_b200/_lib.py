@@ -64,6 +64,11 @@ class ResidentStore(C.Structure):
                 ("h_box_offsets", C.c_void_p)]
 
 
+class WorldAug(C.Structure):
+    _fields_ = [("flip_x_prob", C.c_float), ("flip_y_prob", C.c_float), ("rot_max", C.c_float), ("scale_lo", C.c_float),
+                ("scale_hi", C.c_float)]
+
+
 # name -> (restype, argtypes); must list every symbol declared in include/real3d_b200.h
 PROTOTYPES = {
     "r3d_version": (C.c_int, []),
@@ -137,6 +142,11 @@ PROTOTYPES = {
     "r3d_engine_schedule_read": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32)]),
     "r3d_engine_inserted_device": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
                                              C.POINTER(C.c_void_p)]),
+    "r3d_engine_set_world_aug": (C.c_int, [C.c_void_p, C.POINTER(WorldAug)]),
+    "r3d_engine_world_device": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
+    "r3d_engine_set_object_targets": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "r3d_engine_targets_device": (C.c_int, [C.c_void_p, C.POINTER(ResidentStore), C.c_void_p, C.c_void_p, C.c_int32,
+                                            C.c_void_p, C.c_void_p, C.c_void_p]),
 }
 
 _lib = None

@@ -42,6 +42,38 @@ def read_label_line_od(line):
                             [width + 0.1, length + 0.1, height + 0.1], [items[0]]])
 
 
+def wrap_pi(h):
+    """Angle(s) wrapped to [-pi, pi), in float64 (the arithmetic of the device's ``wrap_pi``)."""
+    h = np.asarray(h, dtype=np.float64)
+    return h - 2.0 * np.pi * np.floor((h + np.pi) * (1.0 / (2.0 * np.pi)))
+
+
+def scene_targets_od(lines):
+    """Every KITTI ``label_2`` line as a detection target box in the engine's lidar frame (the fixed-offset frame of
+    ``read_label_line_od``), computed in float64: (float64 [n, 7] x, y, z_center, dx, dy, dz, heading; names [n]).
+    ``dx, dy, dz`` are the unpadded KITTI ``l, w, h`` and ``heading = -rotation_y - pi/2``, measured from +x toward +y."""
+    out = np.zeros((len(lines), 7), dtype=np.float64)
+    names = []
+    for i, line in enumerate(lines):
+        items = line.split(' ')
+        height, width, length = float(items[8]), float(items[9]), float(items[10])
+        x, y, z = float(items[11]), float(items[12]), float(items[13])
+        out[i] = (z + 0.27, x * -1, (y * -1 - 0.08) + height / 2, length, width, height, -float(items[14]) - np.pi / 2)
+        names.append(items[0])
+    out[:, 6] = wrap_pi(out[:, 6])
+    return out, names
+
+
+def targets_from_lines_od(lines, target_classes):
+    """KITTI lines -> OpenPCDet-style ``gt_boxes`` (float32 [n, 7]: x, y, z_center, dx, dy, dz, heading) and 1-based
+    class ids into ``target_classes`` (int32 [n]); lines whose name is not in ``target_classes`` (``DontCare``
+    included) are dropped, as OpenPCDet drops them."""
+    boxes, names = scene_targets_od(lines)
+    ids = np.array([list(target_classes).index(n) + 1 if n in target_classes else 0 for n in names], dtype=np.int32)
+    keep = ids > 0
+    return boxes[keep].astype(np.float32), ids[keep]
+
+
 def read_label_line_ss(line):
     """Semseg bbox line ``cls x y z h w l yaw`` -> box dictionary (ss/fs:155-189)."""
     items = line.split(' ')

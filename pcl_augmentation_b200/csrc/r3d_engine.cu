@@ -120,6 +120,18 @@ struct r3d_engine {
     cudaEvent_t ev_idx = nullptr;
     DevBuf<int> idx_dev, n_ins_dev;
     DevBuf<float> box7;
+    bool from_store = false;                     // the batch came from r3d_engine_load_resident (store indices in batch_idx)
+    std::vector<int> batch_idx;
+    // world augmentation (r3d_engine_set_world_aug): the policy, and whether the loaded batch drew its world[n][8]
+    r3d_world_aug world_pol;
+    bool world_on = false, world_loaded = false;
+    DevBuf<float> world;
+    // detection targets (r3d_engine_set_object_targets / r3d_engine_targets_device); kept scene boxes per store scan,
+    // read back once per scene_class array
+    DevBuf<float> obj_dims3;
+    DevBuf<int> class_target;
+    const int* kept_src = nullptr;
+    std::vector<int> kept;
     // profiling
     bool profile = false;
     double prof_ms[KID_COUNT] = {0};
@@ -649,6 +661,9 @@ extern "C" int r3d_engine_load_batch(r3d_engine* eng, const r3d_batch* bt) {
     }
     // the std::vectors above are pageable: the copies from them completed before cudaMemcpyAsync returned
     eng->batch_loaded = true;
+    eng->from_store = false;                         // host batches are never world-augmented
+    eng->world_loaded = false;
+    d.world = nullptr;
     return arm_batch(eng, true);
 }
 
@@ -706,6 +721,7 @@ extern "C" int r3d_engine_load_resident(r3d_engine* eng, const r3d_resident_stor
         R3D_CUDA(cudaEventCreateWithFlags(&eng->ev_idx, cudaEventDisableTiming));
         TRY(eng->idx_dev.alloc(d.B));
     }
+    if (eng->world_on && !eng->world.p) TRY(eng->world.alloc((size_t)d.B * 8));
     cudaStream_t st = eng->stream;
     R3D_CUDA(cudaEventSynchronize(eng->ev_idx));
     memcpy(eng->h_idx, indices, (size_t)n * sizeof(int));
@@ -726,6 +742,11 @@ extern "C" int r3d_engine_load_resident(r3d_engine* eng, const r3d_resident_stor
     d.perms = eng->perms.p; d.n_perm_events = d.max_events;
     launch_draw_schedule(idx, n, d.max_events, d.n_classes, d.max_tries, d.class_list_off, eng->policy, seed, epoch, eng->counts.p,
                          eng->perms.p, st);
+    if (eng->world_on) launch_draw_world(idx, n, eng->world_pol, seed, epoch, eng->world.p, st);
+    d.world = eng->world_on ? eng->world.p : nullptr;
+    eng->world_loaded = eng->world_on;
+    eng->from_store = true;
+    eng->batch_idx.assign(indices, indices + n);
     TRY(r3d_check_launch("r3d_engine_load_resident"));
     eng->batch_loaded = true;
     return arm_batch(eng, true);
@@ -852,7 +873,8 @@ static int run_walker(r3d_engine* eng) {
         Launcher l(eng, KID_OUT);
         k_out_count<<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
         k_out_offsets<<<1, 1024, 0, st>>>(d, n, chunks_all);
-        k_out_write<<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
+        if (d.world) k_out_write<true><<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
+        else k_out_write<false><<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
         r3d_count_launch(2);
     }
     R3D_CUDA(cudaMemcpyAsync(eng->h_offsets, eng->out_off.p, (n + 1) * sizeof(long long), cudaMemcpyDeviceToHost, st));
@@ -1040,7 +1062,8 @@ extern "C" int r3d_engine_run_until(r3d_engine* eng, int stop_at, int* still_run
         Launcher l(eng, KID_OUT);
         k_out_count<<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
         k_out_offsets<<<1, 1024, 0, st>>>(d, n, chunks_all);
-        k_out_write<<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
+        if (d.world) k_out_write<true><<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
+        else k_out_write<false><<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
         r3d_count_launch(2);
     }
     R3D_CUDA(cudaMemcpyAsync(eng->h_offsets, eng->out_off.p, (n + 1) * sizeof(long long), cudaMemcpyDeviceToHost, st));
@@ -1099,6 +1122,79 @@ extern "C" int r3d_engine_inserted_device(r3d_engine* eng, const int32_t** n_ins
     if (inserted_box) *inserted_box = eng->inserted_box.p;
     if (box7) *box7 = eng->box7.p;
     return r3d_check_launch("r3d_engine_inserted_device");
+}
+
+extern "C" int r3d_engine_set_world_aug(r3d_engine* eng, const r3d_world_aug* p) {
+    if (eng) cudaSetDevice(eng->device);
+    if (!eng) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_world_aug: null engine");
+    if (!p) { eng->world_on = false; return R3D_OK; }
+    const float v[5] = {p->flip_x_prob, p->flip_y_prob, p->rot_max, p->scale_lo, p->scale_hi};
+    for (float x : v)
+        if (!std::isfinite(x)) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_world_aug: non-finite value");
+    if (p->flip_x_prob < 0.f || p->flip_x_prob > 1.f || p->flip_y_prob < 0.f || p->flip_y_prob > 1.f)
+        return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_world_aug: flip probabilities must be in [0, 1]");
+    if (p->rot_max < 0.f || p->rot_max > (float)kPi)                // pi as the float32 the caller passes
+        return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_world_aug: rot_max must be in [0, pi]");
+    if (!(p->scale_lo > 0.f) || p->scale_hi < p->scale_lo)
+        return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_world_aug: need 0 < scale_lo <= scale_hi");
+    eng->world_pol = *p;
+    eng->world_on = true;
+    return R3D_OK;
+}
+
+extern "C" int r3d_engine_world_device(r3d_engine* eng, const float** params) {
+    if (eng) cudaSetDevice(eng->device);
+    if (!eng || !params) return r3d_fail(R3D_ERR_ARG, "r3d_engine_world_device: null argument");
+    if (!eng->batch_loaded || !eng->world_loaded)
+        return r3d_fail(R3D_ERR_ARG, "r3d_engine_world_device: the batch was not loaded with a world augmentation");
+    *params = eng->world.p;
+    return R3D_OK;
+}
+
+extern "C" int r3d_engine_set_object_targets(r3d_engine* eng, const float* dims3, const int32_t* class_target) {
+    if (eng) cudaSetDevice(eng->device);
+    if (!eng || !dims3 || !class_target || !eng->objects_set) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_object_targets: bad argument or no objects");
+    const EngineDev& d = eng->dev;
+    for (int c = 0; c < d.n_classes; ++c)
+        if (class_target[c] < 0) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_object_targets: negative class id");
+    TRY(eng->obj_dims3.alloc((size_t)d.n_objects * 3));
+    TRY(eng->class_target.alloc((size_t)d.n_classes));
+    R3D_CUDA(cudaMemcpy(eng->obj_dims3.p, dims3, (size_t)d.n_objects * 3 * sizeof(float), cudaMemcpyHostToDevice));
+    R3D_CUDA(cudaMemcpy(eng->class_target.p, class_target, (size_t)d.n_classes * sizeof(int), cudaMemcpyHostToDevice));
+    return R3D_OK;
+}
+
+extern "C" int r3d_engine_targets_device(r3d_engine* eng, const r3d_resident_store* s, const float* scene_box7,
+                                         const int32_t* scene_class, int32_t max_targets, float* out_box7, int32_t* out_class,
+                                         int32_t* out_count) {
+    if (eng) cudaSetDevice(eng->device);
+    if (!eng || !s || !out_box7 || !out_class || !out_count) return r3d_fail(R3D_ERR_ARG, "r3d_engine_targets_device: null argument");
+    if (!eng->ran) return r3d_fail(R3D_ERR_ARG, "r3d_engine_targets_device: run first");
+    if (!eng->from_store) return r3d_fail(R3D_ERR_ARG, "r3d_engine_targets_device: the batch was not loaded from a resident store");
+    const EngineDev& d = eng->dev;
+    if (d.task != 0) return r3d_fail(R3D_ERR_ARG, "r3d_engine_targets_device: detection targets need an object detection engine");
+    if (!eng->obj_dims3.p) return r3d_fail(R3D_ERR_ARG, "r3d_engine_targets_device: set the object targets first");
+    if (s->n_scans <= 0 || !s->box_offsets || !s->h_box_offsets)
+        return r3d_fail(R3D_ERR_ARG, "r3d_engine_targets_device: missing store arrays");
+    const int total = s->h_box_offsets[s->n_scans];
+    if (total > 0 && (!scene_box7 || !scene_class)) return r3d_fail(R3D_ERR_ARG, "r3d_engine_targets_device: missing scene targets");
+    if (eng->kept_src != scene_class || (int)eng->kept.size() != s->n_scans) {
+        std::vector<int> cls((size_t)total);
+        if (total > 0) R3D_CUDA(cudaMemcpy(cls.data(), scene_class, (size_t)total * sizeof(int), cudaMemcpyDeviceToHost));
+        eng->kept.assign(s->n_scans, 0);
+        for (int i = 0; i < s->n_scans; ++i)
+            for (int j = s->h_box_offsets[i]; j < s->h_box_offsets[i + 1]; ++j) eng->kept[i] += cls[j] != 0;
+        eng->kept_src = scene_class;
+    }
+    for (int i : eng->batch_idx) {
+        if (i < 0 || i >= s->n_scans) return r3d_fail(R3D_ERR_ARG, "r3d_engine_targets_device: batch index outside this store");
+        if ((long long)eng->kept[i] + d.max_events - 1 > max_targets)
+            return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_targets_device: max_targets below a scan's kept scene boxes + max_events - 1");
+    }
+    launch_gt_targets(eng->idx_dev.p, s->box_offsets, scene_box7, scene_class, eng->st.p, eng->inserted.p, eng->inserted_box.p,
+                      d.max_events, eng->obj_dims3.p, eng->class_target.p, eng->world_loaded ? eng->world.p : nullptr, eng->n_scans,
+                      max_targets, out_box7, out_class, out_count, eng->stream);
+    return r3d_check_launch("r3d_engine_targets_device");
 }
 
 extern "C" int r3d_engine_fetch(r3d_engine* eng, r3d_batch_result* res) {

@@ -180,7 +180,21 @@ struct EngineDev {       // passed by value to kernels
     float4* out_xyzi;
     unsigned* out_label;
     float* out_check;
+    const float* world;               // [B][8] world augmentation (fx, fy, theta, c, s, k, 0, 0) of the output; NULL = off
 };
+
+// The world transform of r3d_world_aug (include/real3d_b200.h) on one point: flip, rotate, scale, in float32 without
+// contraction, so that a host restatement reproduces it bit for bit
+struct WorldXf { bool fx, fy; float c, s, k; };
+__device__ __forceinline__ WorldXf world_xf(const float* w) {
+    return WorldXf{w[0] != 0.f, w[1] != 0.f, w[3], w[4], w[5]};
+}
+__device__ __forceinline__ void world_point(const WorldXf& t, float& x, float& y, float& z) {
+    const float x1 = t.fy ? -x : x, y1 = t.fx ? -y : y;
+    x = __fmul_rn(__fsub_rn(__fmul_rn(t.c, x1), __fmul_rn(t.s, y1)), t.k);
+    y = __fmul_rn(__fadd_rn(__fmul_rn(t.s, x1), __fmul_rn(t.c, y1)), t.k);
+    z = __fmul_rn(z, t.k);
+}
 
 #define R3D_N_STATS 40
 #ifndef R3D_OCC_G

@@ -66,6 +66,9 @@ __global__ void __launch_bounds__(1024) k_out_offsets(EngineDev e, int n_scans, 
     }
 }
 
+// WORLD: e.world is set and every output point and check row goes through the scan's world transform on its way out
+// (no extra bytes); the instantiation without it is the plain compaction
+template <bool WORLD>
 __global__ void __launch_bounds__(STREAM_THREADS) k_out_write(EngineDev e, int n_scans) {
     const int b = blockIdx.y;
     if (b >= n_scans) return;
@@ -73,10 +76,22 @@ __global__ void __launch_bounds__(STREAM_THREADS) k_out_write(EngineDev e, int n
     const int n = s.n0 + s.n_tail;
     const int p0 = blockIdx.x * CHUNK;
     const size_t base = (size_t)b * e.P;
+    [[maybe_unused]] WorldXf wx{};
+    if constexpr (WORLD) wx = world_xf(e.world + (size_t)b * 8);
     if (blockIdx.x == 0) {                              // the `check` record of the scan (od/ds:91-93)
         const long long c0 = e.check_off[b];
         const float* ck = e.check + (size_t)b * e.max_inserted * 5;
-        for (int i = threadIdx.x; i < s.n_check * 5; i += blockDim.x) e.out_check[c0 * 5 + i] = ck[i];
+        if constexpr (WORLD) {
+            for (int r = threadIdx.x; r < s.n_check; r += blockDim.x) {
+                const float* in = ck + (size_t)r * 5;
+                float* out = e.out_check + (c0 + r) * 5;
+                float x = in[0], y = in[1], z = in[2];
+                world_point(wx, x, y, z);
+                out[0] = x; out[1] = y; out[2] = z; out[3] = in[3]; out[4] = in[4];
+            }
+        } else {
+            for (int i = threadIdx.x; i < s.n_check * 5; i += blockDim.x) e.out_check[c0 * 5 + i] = ck[i];
+        }
     }
     if (p0 >= n) return;
     long long o0 = e.out_off[b];
@@ -113,6 +128,7 @@ __global__ void __launch_bounds__(STREAM_THREADS) k_out_write(EngineDev e, int n
                 v = make_float4((float)e.tail_x[t], (float)e.tail_y[t], (float)e.tail_z[t], e.tail_i[t]);
             }
             lab = e.label[base + p];
+            if constexpr (WORLD) world_point(wx, v.x, v.y, v.z);
         }
         const unsigned m = __ballot_sync(0xffffffffu, a);
         if (a) {

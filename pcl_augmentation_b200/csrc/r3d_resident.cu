@@ -199,6 +199,101 @@ __global__ void k_inserted_targets(const ScanState* __restrict__ sts, const doub
     o[6] = live ? (float)atan2(q[4], q[3]) : 0.f;
 }
 
+// ------------------------------------------------------------------------------------------ world augmentation
+// One thread per scan: one Philox call on the stream id 0xFFFFFFFF (the schedule streams are 0 and 1 + event * 16 +
+// class < 2^16), so the world parameters of a scan depend on (seed, epoch, store index) only.
+__device__ __forceinline__ float uniform24(unsigned w) { return (float)(w >> 8) * 0x1p-24f; }   // exact, in [0, 1)
+
+__global__ void k_draw_world(const int* __restrict__ idx, int n, r3d_world_aug pol, unsigned long long seed,
+                             unsigned long long epoch, float* world) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= n) return;
+    const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32) ^ (unsigned)(epoch >> 32));
+    const uint4 x = philox4x32_10(make_uint4(0u, 0xFFFFFFFFu, (unsigned)idx[b], (unsigned)epoch), key);
+    const float theta = __fmul_rn(pol.rot_max, __fsub_rn(__fmul_rn(2.f, uniform24(x.z)), 1.f));
+    const float k = __fadd_rn(pol.scale_lo, __fmul_rn(__fsub_rn(pol.scale_hi, pol.scale_lo), uniform24(x.w)));
+    float* w = world + (size_t)b * 8;
+    w[0] = uniform24(x.x) < pol.flip_x_prob ? 1.f : 0.f;
+    w[1] = uniform24(x.y) < pol.flip_y_prob ? 1.f : 0.f;
+    w[2] = theta; w[3] = cosf(theta); w[4] = sinf(theta); w[5] = k; w[6] = 0.f; w[7] = 0.f;
+}
+
+// ------------------------------------------------------------------------------------------ detection targets
+__device__ __forceinline__ double wrap_pi(double h) {        // into [-pi, pi)
+    return __dsub_rn(h, __dmul_rn(2.0 * kPi, floor(__dmul_rn(__dadd_rn(h, kPi), 1.0 / (2.0 * kPi)))));
+}
+// a target box through the scan's world transform (centre as the points, dimensions * k, heading flipped / rotated)
+__device__ __forceinline__ void world_box(const WorldXf& t, float theta, float* o) {
+    world_point(t, o[0], o[1], o[2]);
+    o[3] = __fmul_rn(o[3], t.k); o[4] = __fmul_rn(o[4], t.k); o[5] = __fmul_rn(o[5], t.k);
+    double h = (double)o[6];
+    if (t.fx) h = -h;
+    if (t.fy) h = -__dadd_rn(h, kPi);
+    o[6] = (float)wrap_pi(__dadd_rn(h, (double)theta));
+}
+
+// One warp per scan writes its targets row: the kept scene boxes of its store scan, then its kept inserted objects,
+// compacted with ballots, then zeros up to max_targets.  Inserted box: centre from inserted_box (cx cy cz_bottom m00
+// m10 ...), z to the box centre with the cut object's unpadded height, heading atan2(m10, m00) - pi/2.
+__global__ void k_gt_targets(const int* __restrict__ idx, const int* __restrict__ box_off, const float* __restrict__ scene_box7,
+                             const int* __restrict__ scene_class, const ScanState* __restrict__ sts, const int* __restrict__ inserted,
+                             const double* __restrict__ ibox, int E, const float* __restrict__ dims3,
+                             const int* __restrict__ class_target, const float* __restrict__ world, int n, int max_targets,
+                             float* out_box7, int* out_class, int* out_count) {
+    const int b = (int)((blockIdx.x * (size_t)blockDim.x + threadIdx.x) >> 5);
+    const int lane = threadIdx.x & 31;
+    if (b >= n) return;                                       // whole warps: n * 32 threads of whole CTAs
+    const int i = idx[b];
+    const int first = box_off[i], nb = box_off[i + 1] - first;
+    const int ni = sts[b].n_inserted;
+    float* ob = out_box7 + (size_t)b * max_targets * 7;
+    int* oc = out_class + (size_t)b * max_targets;
+    WorldXf wx{};
+    float theta = 0.f;
+    if (world) { wx = world_xf(world + (size_t)b * 8); theta = world[(size_t)b * 8 + 2]; }
+    const unsigned below = (1u << lane) - 1u;
+    int m = 0;
+    for (int j0 = 0; j0 < nb; j0 += 32) {
+        const int j = j0 + lane;
+        const int cls = j < nb ? scene_class[first + j] : 0;
+        const unsigned keep = __ballot_sync(0xffffffffu, cls != 0);
+        if (cls != 0) {
+            const int pos = m + __popc(keep & below);
+            float o[7];
+            for (int q = 0; q < 7; ++q) o[q] = scene_box7[(size_t)(first + j) * 7 + q];
+            if (world) world_box(wx, theta, o);
+            for (int q = 0; q < 7; ++q) ob[(size_t)pos * 7 + q] = o[q];
+            oc[pos] = cls;
+        }
+        m += __popc(keep);
+    }
+    for (int j0 = 0; j0 < ni; j0 += 32) {
+        const int j = j0 + lane;
+        const size_t t = (size_t)b * E + j;
+        const int cls = j < ni ? class_target[inserted[t * 4 + 2]] : 0;
+        const unsigned keep = __ballot_sync(0xffffffffu, cls != 0);
+        if (cls != 0) {
+            const int pos = m + __popc(keep & below);
+            const double* q = ibox + t * 8;
+            const float* dm = dims3 + (size_t)inserted[t * 4] * 3;
+            float o[7];
+            o[0] = (float)q[0]; o[1] = (float)q[1];
+            o[2] = (float)__dadd_rn(q[2], __dmul_rn((double)dm[2], 0.5));
+            o[3] = dm[0]; o[4] = dm[1]; o[5] = dm[2];
+            o[6] = (float)wrap_pi(__dsub_rn(atan2(q[4], q[3]), 0.5 * kPi));
+            if (world) world_box(wx, theta, o);
+            for (int r = 0; r < 7; ++r) ob[(size_t)pos * 7 + r] = o[r];
+            oc[pos] = cls;
+        }
+        m += __popc(keep);
+    }
+    for (int p = m + lane; p < max_targets; p += 32) {
+        for (int q = 0; q < 7; ++q) ob[(size_t)p * 7 + q] = 0.f;
+        oc[p] = 0;
+    }
+    if (lane == 0) out_count[b] = m;
+}
+
 // ------------------------------------------------------------------------------------------------ launchers
 void launch_gather_points(const r3d_resident_store& s, const int* idx, int n, int max_n0, float4* xyzi, int max_points,
                           unsigned* label, int P, int od, unsigned road_label, cudaStream_t st) {
@@ -231,6 +326,23 @@ void launch_draw_schedule(const int* idx, int n, int E, int C, int T, const int*
 void launch_inserted_targets(const ScanState* sts, const double* inserted_box, int n, int E, int* n_inserted, float* box7,
                              cudaStream_t st) {
     k_inserted_targets<<<(n * E + 127) / 128, 128, 0, st>>>(sts, inserted_box, n, E, n_inserted, box7);
+    r3d_count_launch();
+}
+
+void launch_draw_world(const int* idx, int n, const r3d_world_aug& pol, unsigned long long seed, unsigned long long epoch,
+                       float* world, cudaStream_t st) {
+    k_draw_world<<<(n + 127) / 128, 128, 0, st>>>(idx, n, pol, seed, epoch, world);
+    r3d_count_launch();
+}
+
+void launch_gt_targets(const int* idx, const int* box_off, const float* scene_box7, const int* scene_class, const ScanState* sts,
+                       const int* inserted, const double* inserted_box, int E, const float* dims3, const int* class_target,
+                       const float* world, int n, int max_targets, float* out_box7, int* out_class, int* out_count,
+                       cudaStream_t st) {
+    constexpr int WARPS = 4;
+    k_gt_targets<<<(n + WARPS - 1) / WARPS, WARPS * 32, 0, st>>>(idx, box_off, scene_box7, scene_class, sts, inserted, inserted_box,
+                                                                  E, dims3, class_target, world, n, max_targets, out_box7,
+                                                                  out_class, out_count);
     r3d_count_launch();
 }
 

@@ -24,5 +24,13 @@ void launch_draw_schedule(const int* idx, int n, int E, int C, int T, const int*
 // n_inserted [n] and the float32 boxes [n][E][7] of the last run
 void launch_inserted_targets(const ScanState* sts, const double* inserted_box, int n, int E, int* n_inserted, float* box7,
                              cudaStream_t st);
+// world [n][8] = (fx, fy, theta, c, s, k, 0, 0) of the scans idx[0 .. n) for (seed, epoch) (r3d_world_aug)
+void launch_draw_world(const int* idx, int n, const r3d_world_aug& pol, unsigned long long seed, unsigned long long epoch,
+                       float* world, cudaStream_t st);
+// detection targets of the last run (r3d_engine_targets_device); world may be NULL
+void launch_gt_targets(const int* idx, const int* box_off, const float* scene_box7, const int* scene_class, const ScanState* sts,
+                       const int* inserted, const double* inserted_box, int E, const float* dims3, const int* class_target,
+                       const float* world, int n, int max_targets, float* out_box7, int* out_class, int* out_count,
+                       cudaStream_t st);
 
 }  // namespace r3d

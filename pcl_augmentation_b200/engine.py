@@ -424,6 +424,59 @@ class Real3DEngine:
                 "inserted": _cuda_tensor(pi.value, (n, e, 4), "<i4", torch.int32),
                 "boxes": _cuda_tensor(p7.value, (n, e, 7), "<f4", torch.float32)}
 
+    def set_world_aug(self, policy):
+        """World flip / rotation / scaling of the following ``load_resident`` batches (``online.WorldAug`` or any object
+        with its five fields; None turns it off).  ``load`` batches are never transformed."""
+        if policy is None:
+            _lib.check(self.lib.r3d_engine_set_world_aug(self.handle, None), "set_world_aug")
+            return
+        w = _lib.WorldAug(float(policy.flip_x_prob), float(policy.flip_y_prob), float(policy.rot_max),
+                          float(policy.scale_lo), float(policy.scale_hi))
+        _lib.check(self.lib.r3d_engine_set_world_aug(self.handle, C.byref(w)), "set_world_aug")
+
+    def world_device(self):
+        """float32 CUDA tensor [n, 8] (fx, fy, theta, c, s, k, 0, 0) of the loaded batch, aliasing the engine's buffer;
+        raises unless the batch was loaded by ``load_resident`` with a world augmentation."""
+        import torch
+        p = C.c_void_p()
+        _lib.check(self.lib.r3d_engine_world_device(self.handle, C.byref(p)), "world_device")
+        return _cuda_tensor(p.value, (self._n_scans, 8), "<f4", torch.float32)
+
+    def set_target_classes(self, target_classes):
+        """Object detection: the target classes of ``targets_device`` (class id = 1 + position in the list).  The
+        dimensions of a cut object's target box are the unpadded ``l, w, h`` of its own KITTI string."""
+        if self.task != 'od':
+            raise _lib.Real3DError("detection targets need an object detection engine")
+        target_classes = list(target_classes)
+        missing = [c for c in self.classes if c not in target_classes]
+        if missing:
+            raise _lib.Real3DError(f"insertion classes {missing} are not in target_classes {target_classes}")
+        dims = np.zeros((max(len(self.obj_strings), 1), 3), dtype=np.float32)
+        for i, s in enumerate(self.obj_strings):
+            items = (s.item() if hasattr(s, 'item') else str(s)).split(' ')
+            dims[i] = (float(items[10]), float(items[9]), float(items[8]))
+        class_target = np.array([target_classes.index(c) + 1 for c in self.classes], dtype=np.int32)
+        _lib.check(self.lib.r3d_engine_set_object_targets(self.handle, dims.ctypes.data, class_target.ctypes.data),
+                   "set_object_targets")
+        self.target_classes = target_classes
+
+    def targets_device(self, store, out):
+        """Enqueue the detection targets of the last run (a ``load_resident`` batch of ``store``) on the engine stream
+        into ``out`` = {'gt_boxes': float32 [>= n, max_targets, 7], 'gt_classes': int32 [>= n, max_targets], 'n_gt':
+        int32 [>= n]} (contiguous CUDA tensors): the scan's scene boxes, then its inserted objects, then zeros."""
+        if self.task != 'od':
+            raise _lib.Real3DError("targets_device: detection targets need an object detection engine")
+        if getattr(self, 'target_classes', None) is None:
+            raise _lib.Real3DError("targets_device: call set_target_classes first")
+        box7, cls = store.scene_targets(self.target_classes)
+        gb, gc, ng = out['gt_boxes'], out['gt_classes'], out['n_gt']
+        n, m = self._n_scans, int(gb.shape[1])
+        assert gb.is_contiguous() and gc.is_contiguous() and ng.is_contiguous()
+        assert gb.shape[0] >= n and gb.shape[2] == 7 and tuple(gc.shape[1:]) == (m,) and gc.shape[0] >= n and ng.shape[0] >= n
+        ptr = lambda t: t.data_ptr() if t.numel() else None
+        _lib.check(self.lib.r3d_engine_targets_device(self.handle, C.byref(store.abi), ptr(box7), ptr(cls), m,
+                                                      gb.data_ptr(), gc.data_ptr(), ng.data_ptr()), "targets_device")
+
     def unpack(self, buffers, raise_on_error=True):
         """Per-scan output records in the reference's formats."""
         out = []

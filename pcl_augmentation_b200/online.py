@@ -11,6 +11,7 @@ the batch it lands in or on the rank that owns it; they are their own random str
 from __future__ import annotations
 
 import collections
+import math
 import os
 from dataclasses import dataclass
 
@@ -85,6 +86,15 @@ class ResidentDataset:
         # the same per batch)
         recs = bx.box_records_from_lines(lines, ss=task == 'ss') if lines else np.zeros((0, 16))
         self.boxes = torch.from_numpy(np.ascontiguousarray(recs, dtype=np.float64).reshape(-1, 16)).to(dev)
+        # OD: every scene box as a detection target record (bx.scene_targets_od) and the id of its name in box_names,
+        # 1:1 with the box records; the class ids of a target_classes list are derived from them on the device
+        self.box_names, self._scene_targets = [], {}
+        if task == 'od':
+            t7, names = bx.scene_targets_od(lines)
+            self.box_names = sorted(set(names))
+            self.h_box_name_ids = np.array([self.box_names.index(n) for n in names], dtype=np.int32)
+            self.scene_box7 = torch.from_numpy(np.ascontiguousarray(t7.astype(np.float32)).reshape(-1, 7)).to(dev)
+            self.box_name_ids = torch.from_numpy(self.h_box_name_ids).to(dev)
         self.point_offsets = torch.from_numpy(self.h_point_offsets).to(dev)
         self.box_offsets = torch.from_numpy(self.h_box_offsets).to(dev)
         self.max_points = int(np.diff(self.h_point_offsets).max())
@@ -116,6 +126,27 @@ class ResidentDataset:
 
     def __len__(self):
         return self.n_scans
+
+    def scene_targets(self, target_classes):
+        """(scene_box7 float32 [boxes, 7], class ids int32 [boxes]) on the device for ``target_classes``: 1-based
+        position of the box's name in the list, 0 for a box that is not a target.  Mapped once per list."""
+        if self.task != 'od':
+            raise _lib.Real3DError("detection targets need an object detection store")
+        key = tuple(target_classes)
+        if key not in self._scene_targets:
+            torch = _lib.require_cuda()
+            lut = np.array([key.index(n) + 1 if n in key else 0 for n in self.box_names] or [0], dtype=np.int32)
+            ids = torch.from_numpy(lut).to(self.box_name_ids.device)[self.box_name_ids.long()].to(torch.int32).contiguous()
+            torch.cuda.current_stream().synchronize()        # the engine reads the ids back once, outside this stream
+            is_target = (lut[self.h_box_name_ids] > 0).astype(np.int64)
+            kept = np.cumsum(np.concatenate([[0], is_target]))[self.h_box_offsets]
+            self._scene_targets[key] = (self.scene_box7, ids, int(np.diff(kept).max()))
+        return self._scene_targets[key][:2]
+
+    def max_kept_boxes(self, target_classes):
+        """The most scene boxes of one scan that are ``target_classes`` targets."""
+        self.scene_targets(target_classes)
+        return self._scene_targets[tuple(target_classes)][2]
 
     @classmethod
     def from_scans(cls, task, scans, map_data=None):
@@ -159,6 +190,31 @@ class ResidentDataset:
 
 
 @dataclass
+class WorldAug:
+    """Per-scan world augmentation after the insertion (OpenPCDet's ``random_world_flip`` / ``random_world_rotation`` /
+    ``random_world_scaling``; defaults of its KITTI configs): flip along x (y -> -y) with ``flip_x_prob``, along y
+    (x -> -x) with ``flip_y_prob``, rotate about z by a uniform angle in [-rot_max, rot_max], scale by a uniform factor
+    in [scale_lo, scale_hi], in that order, to the points and the boxes together.  The exact arithmetic is that of
+    ``r3d_world_aug`` in include/real3d_b200.h."""
+    flip_x_prob: float = 0.5
+    flip_y_prob: float = 0.0
+    rot_max: float = math.pi / 4
+    scale_lo: float = 0.95
+    scale_hi: float = 1.05
+
+    def __post_init__(self):
+        vals = (self.flip_x_prob, self.flip_y_prob, self.rot_max, self.scale_lo, self.scale_hi)
+        if not all(math.isfinite(float(v)) for v in vals):
+            raise ValueError(f"WorldAug: non-finite value in {self}")
+        if not (0.0 <= self.flip_x_prob <= 1.0 and 0.0 <= self.flip_y_prob <= 1.0):
+            raise ValueError("WorldAug: flip probabilities must be in [0, 1]")
+        if not 0.0 <= self.rot_max <= math.pi:
+            raise ValueError("WorldAug: rot_max must be in [0, pi]")
+        if not 0.0 < self.scale_lo <= self.scale_hi:
+            raise ValueError("WorldAug: need 0 < scale_lo <= scale_hi")
+
+
+@dataclass
 class AugmentedBatch:
     """One augmented batch as CUDA tensors that alias the engine's buffers (valid until the engine that made it is
     loaded again, ``depth`` batches later).  Scan s owns rows ``offsets[s]:offsets[s + 1]`` of xyzi / labels and
@@ -173,8 +229,15 @@ class AugmentedBatch:
     class_index: object       # int32 [n, max_events]
     rotation: object          # int32 [n, max_events]: yaw step of the placement
     visible: object           # int32 [n, max_events]: visible points of the inserted object
-    boxes: object             # float32 [n, max_events, 7]: x, y, z_bottom, length, width, height, yaw (lidar frame)
+    boxes: object             # float32 [n, max_events, 7]: x, y, z_bottom, length, width, height, yaw (lidar frame):
+                              # the inserted objects in the engine's collision-box convention, before the world transform
     indices: np.ndarray       # int64 [n], host: the store scans of the batch
+    # with target_classes: every ground-truth box of the augmented scan (scene boxes in file order, then the inserted
+    # objects), OpenPCDet gt_boxes layout x, y, z_center, dx, dy, dz, heading, after the world transform
+    gt_boxes: object = None   # float32 [n, max_targets, 7]; rows past n_gt are zero
+    gt_classes: object = None # int32 [n, max_targets]: 1-based into target_classes, 0 = padding
+    n_gt: object = None       # int32 [n]
+    world: object = None      # float32 [n, 8]: with world_aug, (fx, fy, theta, c, s, k, 0, 0) of each scan
 
 
 class OnlineAugmenter:
@@ -182,7 +245,9 @@ class OnlineAugmenter:
     batch k + 1 is augmented while the consumer still works on batch k."""
 
     def __init__(self, task, config, db, dataset, *, batch_size, seed, yaw_steps=360, depth=2, rank=0, world=1,
-                 **engine_kwargs):
+                 target_classes=None, world_aug=None, **engine_kwargs):
+        """``target_classes`` (object detection): the class names of ``gt_boxes`` / ``gt_classes``; every insertion
+        class must be one of them.  ``world_aug``: a ``WorldAug`` applied to every batch (None: off)."""
         torch = _lib.require_cuda()
         from .dataset_driver import _objects_per_frame
         assert dataset.task == task and depth >= 1
@@ -201,6 +266,21 @@ class OnlineAugmenter:
         self._next = 0
         self._pending = collections.deque()
         self._torch = torch
+        self.world_aug = world_aug
+        for e in self.engines:
+            e.set_world_aug(world_aug)
+        self.target_classes = None if target_classes is None else list(target_classes)
+        self._targets = []
+        if self.target_classes is not None:
+            if task != 'od':
+                raise _lib.Real3DError("detection targets need an object detection dataset")
+            self.max_targets = dataset.max_kept_boxes(self.target_classes) + self.max_events - 1
+            dev = dataset.xyzi.device
+            for e in self.engines:             # each slot owns the buffers of the batch its engine holds
+                e.set_target_classes(self.target_classes)
+                self._targets.append({'gt_boxes': torch.zeros((self.batch_size, self.max_targets, 7), dtype=torch.float32, device=dev),
+                                      'gt_classes': torch.zeros((self.batch_size, self.max_targets), dtype=torch.int32, device=dev),
+                                      'n_gt': torch.zeros(self.batch_size, dtype=torch.int32, device=dev)})
 
     def _submit(self, indices, epoch):
         torch = self._torch
@@ -231,13 +311,22 @@ class OnlineAugmenter:
         eng = self.engines[slot]
         out = eng.outputs_on_device()                # waits for the run: the one host synchronisation of a batch
         ins = eng.inserted_device()
+        extra = {}
+        if self.target_classes is not None:
+            tg = self._targets[slot]
+            eng.targets_device(self.dataset, tg)
+            n = len(idx)
+            extra.update(gt_boxes=tg['gt_boxes'][:n], gt_classes=tg['gt_classes'][:n], n_gt=tg['n_gt'][:n])
+        if self.world_aug is not None:
+            extra['world'] = eng.world_device()
         ready = torch.cuda.Event()
         ready.record(self._streams[slot])
         torch.cuda.current_stream().wait_event(ready)
         t = ins['inserted']
         return AugmentedBatch(xyzi=out['xyzi'], labels=out['labels'], offsets=out['offsets'], check=out['check'],
                               check_offsets=out['check_offsets'], n_inserted=ins['n_inserted'], object_id=t[..., 0],
-                              rotation=t[..., 1], class_index=t[..., 2], visible=t[..., 3], boxes=ins['boxes'], indices=idx)
+                              rotation=t[..., 1], class_index=t[..., 2], visible=t[..., 3], boxes=ins['boxes'], indices=idx,
+                              **extra)
 
     def augment(self, indices, epoch):
         """Augment the store scans ``indices`` (at most ``batch_size``; duplicates allowed) with the draws of

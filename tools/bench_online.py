@@ -6,6 +6,7 @@ intensities are redrawn (2.2 GB of points + labels: larger than L2, so the gathe
 
     python tools/bench_online.py [--batches 20] [--warmup 2] [--depth 3] [--out DIR]            rates
     python tools/bench_online.py --profile [--out DIR]                                           kernel times + copies
+    python tools/bench_online.py --targets [--world-aug] [--rounds 3] [--out DIR]                 variants A/B
 
 Rates (scans/s, host clock around work that ends in a device synchronise):
   * online     OnlineAugmenter.epochs over the store, a new epoch each pass (gather + device schedule draw + run), and
@@ -14,6 +15,9 @@ Rates (scans/s, host clock around work that ends in a device synchronise):
   * host       load + run of a batch staged in pinned host buffers (Real3DEngine.stage, outside the timed loop).
 --profile: torch.profiler over a few online batches: device time of k_gather_points and k_draw_schedule, the gather's
 bytes per second against a device-to-device copy measured in the same run, and every host-to-device copy of a batch.
+--targets / --world-aug: the online rate of plain batches, of batches with detection targets (targets_device) and, with
+--world-aug, of batches with targets and world augmentation, alternating the variants round by round on the same
+engines; with --profile, the kernel times of a plain epoch and of an epoch with the variant's options, in one process.
 """
 from __future__ import annotations
 
@@ -41,7 +45,10 @@ def card():
     return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else "unknown"
 
 
-def setup(depth):
+TARGETS = ["Car", "Pedestrian", "Cyclist"]
+
+
+def setup(depth, targets=False, world_aug=None):
     import bench
     from pcl_augmentation_b200.engine import scan_input_from_case
     from pcl_augmentation_b200.online import OnlineAugmenter, ResidentDataset
@@ -58,8 +65,54 @@ def setup(depth):
     kw = bench.engine_kwargs("c3", base)
     kw.pop("max_scans"), kw.pop("map_data")
     c0 = base[0]
-    aug = OnlineAugmenter("od", c0.config, c0.db, store, batch_size=BATCH, seed=2024, depth=depth, **kw)
+    aug = OnlineAugmenter("od", c0.config, c0.db, store, batch_size=BATCH, seed=2024, depth=depth,
+                          target_classes=TARGETS if targets else None, world_aug=world_aug, **kw)
     return aug, store, scans
+
+
+def set_variant(aug, targets, world_aug):
+    """Switch an augmenter built with targets between the variants (its target buffers stay allocated)."""
+    aug.target_classes = TARGETS if targets else None
+    aug.world_aug = world_aug
+    for e in aug.engines:
+        e.set_world_aug(world_aug)
+
+
+def variants(args):
+    import torch
+    from pcl_augmentation_b200.online import WorldAug
+    aug, store, _ = setup(args.depth, targets=True)
+    names = {"online": (False, None), "online_targets": (True, None)}
+    if args.world_aug:
+        names["online_targets_world"] = (True, WorldAug())
+    per_epoch = N_STORE // BATCH
+    n_epochs = -(-args.batches // per_epoch)
+    out = {"card": card(), "store_scans": N_STORE, "batch": BATCH, "rounds": args.rounds}
+    for name, (t, w) in names.items():                  # warm every variant
+        set_variant(aug, t, w)
+        for _ in aug.epochs(range(10_000, 10_000 + -(-args.warmup // per_epoch))):
+            pass
+    torch.cuda.synchronize()
+    rates_by = {k: [] for k in names}
+    epoch = 0
+    for _ in range(args.rounds):
+        for name, (t, w) in names.items():
+            set_variant(aug, t, w)
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            n = 0
+            for _, b in aug.epochs(range(epoch, epoch + n_epochs)):
+                n += len(b.indices)
+            torch.cuda.synchronize()
+            rates_by[name].append(n / (time.perf_counter() - t0))
+            epoch += n_epochs
+    for name, r in rates_by.items():
+        out[name + "_scans_per_s"] = r
+        out[name + "_median"] = float(np.median(r))
+    for name in names:
+        out[name + "_over_online"] = out[name + "_median"] / out["online_median"]
+    aug.close()
+    return out
 
 
 def rates(args):
@@ -118,7 +171,9 @@ def rates(args):
 def profile(args):
     import torch
     from torch.profiler import ProfilerActivity, profile as tprofile
-    aug, store, _ = setup(args.depth)
+    from pcl_augmentation_b200.online import WorldAug
+    aug, store, _ = setup(args.depth, targets=args.targets)
+    set_variant(aug, False, None)
     for _ in aug.epoch(99):
         pass
     torch.cuda.synchronize()
@@ -148,7 +203,7 @@ def profile(args):
     for ev in events:
         name, cat = ev.get("name", ""), ev.get("cat", "")
         if cat == "kernel":
-            for k in ("k_gather_points", "k_draw_schedule", "k_gather_boxes", "k_gather_scan_meta", "k_inserted_targets"):
+            for k in KERNELS:
                 if k in name:
                     kern.setdefault(k, []).append(float(ev.get("dur", 0.0)))
         elif cat == "gpu_memcpy" and "HtoD" in name:
@@ -161,8 +216,42 @@ def profile(args):
            "gather_bytes_per_s": pts * 38 / (gather_us * 1e-6), "copy_peak_bytes_per_s": copy_bps,
            "h2d_copies_per_batch": len(h2d) / max(n_batches, 1), "h2d_copies": h2d[:16]}
     out["gather_over_copy_peak"] = out["gather_bytes_per_s"] / copy_bps
+    if args.targets or args.world_aug:                 # the same epoch with the variant's options, same process
+        set_variant(aug, args.targets, WorldAug() if args.world_aug else None)
+        for _ in aug.epoch(98):
+            pass
+        torch.cuda.synchronize()
+        kern_on, _ = kernel_times(aug, 0)
+        out["variant"] = {"targets": args.targets, "world_aug": args.world_aug}
+        out["variant_kernels_us_per_launch"] = {k: {"mean": float(np.mean(v)), "launches": len(v)} for k, v in kern_on.items()}
     aug.close()
     return out
+
+
+KERNELS = ("k_gather_points", "k_draw_schedule", "k_gather_boxes", "k_gather_scan_meta", "k_inserted_targets", "k_draw_world",
+           "k_gt_targets", "k_out_write")
+
+
+def kernel_times(aug, epoch):
+    """Device time per launch of KERNELS over one online epoch (torch.profiler), and the host-to-device copies."""
+    import torch
+    from torch.profiler import ProfilerActivity, profile as tprofile
+    n_batches = 0
+    with tprofile(activities=[ProfilerActivity.CUDA, ProfilerActivity.CPU]) as prof:
+        for _ in aug.epoch(epoch):
+            n_batches += 1
+        torch.cuda.synchronize()
+    trace = os.path.join(tempfile.mkdtemp(), "online.pt.trace.json")
+    prof.export_chrome_trace(trace)
+    with open(trace) as f:
+        events = json.load(f)["traceEvents"]
+    kern = {}
+    for ev in events:
+        if ev.get("cat", "") == "kernel":
+            for k in KERNELS:
+                if k in ev.get("name", ""):
+                    kern.setdefault(k, []).append(float(ev.get("dur", 0.0)))
+    return kern, n_batches
 
 
 def main():
@@ -171,17 +260,25 @@ def main():
     ap.add_argument("--warmup", type=int, default=4)
     ap.add_argument("--depth", type=int, default=3)
     ap.add_argument("--profile", action="store_true")
+    ap.add_argument("--targets", action="store_true", help="detection targets for every batch (see the module doc)")
+    ap.add_argument("--world-aug", action="store_true", help="world flip / rotation / scaling (WorldAug defaults)")
+    ap.add_argument("--rounds", type=int, default=3, help="--targets: alternations of the variants")
     ap.add_argument("--out", default=None, help="directory for the JSON result (printed either way)")
     args = ap.parse_args()
     import __graft_entry__  # noqa: F401  (puts the repository on sys.path)
     from pcl_augmentation_b200 import _lib
     _lib.require_cuda()
-    res = profile(args) if args.profile else rates(args)
+    if args.world_aug and not args.targets and not args.profile:
+        ap.error("--world-aug is measured as online + targets + world aug: pass --targets too")
+    res = profile(args) if args.profile else variants(args) if args.targets else rates(args)
     line = json.dumps(res)
     print(line)
     if args.out:
         os.makedirs(args.out, exist_ok=True)
-        with open(os.path.join(args.out, "bench_online_profile.json" if args.profile else "bench_online.json"), "w") as f:
+        name = "bench_online_profile" if args.profile else "bench_online"
+        name += "_targets" if args.targets else ""
+        name += "_world" if args.world_aug else ""
+        with open(os.path.join(args.out, name + ".json"), "w") as f:
             f.write(line + "\n")
 
 
