@@ -10,12 +10,16 @@
 #include <thread>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <string>
 #include <vector>
 
 using namespace r3d;
 
 #define R3D_MAX_SUB 16
+// the three full re-projection kernels and close/fill walk the work lists k_update wrote (all scans in round 0, a
+// handful later): grids sized for "some scans", not for every (chunk, scan) / (tile, scan) pair
+#define R3D_FULL_Y 32
 
 namespace {
 
@@ -81,33 +85,26 @@ struct r3d_engine {
     int run_nsub = 0, run_done = 0, run_rounds = 0;
     bool objects_set = false, yaw_set = false, batch_loaded = false, ran = false;
     int last_rounds = 0;
-    // device buffers
-    DevBuf<float4> xyzi, out_xyzi, gpts, apts;
-    DevBuf<unsigned long long> sel_keys;
-    DevBuf<double> sel_r, tail_x, tail_y, tail_z, r, el, smooth, poses, obj_x, obj_y, obj_z, cos_k, sin_k, radii_sq, cand_level,
-        inserted_box;
-    DevBuf<float> tail_i, obj_i, check, out_check;
-    DevBuf<unsigned> label, dmask, vmask, occ_win, unplaceable, obj_label, out_label, tickets;
-    DevBuf<unsigned short> col, cand_list, label16, out_label16;
-    DevBuf<unsigned char> label1;
-    DevBuf<long long> pt_off;
-    DevBuf<int> chunk_cnt, pix, gate_update, gate_try, gate_apply, gate_full, gate_patch, cf_rect, col_off, col_idx, acell, active_count, far_arr, od_map_dims, counts, perms, class_list_off,
-        class_list, radii_ok, cand_v, gcell, n_list, feas, occ_pix, sel_pix, inserted, n0_arr, nbox0_arr, work_cnt, full_list, cf_tasks, need2, occ_far;
-    DevBuf<unsigned> occ_cnt;
-    DevBuf<unsigned> round_ctl;
-    DevBuf<unsigned char> alive, od_maps, ss_map, cand_flags, gnear, gscratch;
-    DevBuf<unsigned long long> zraw, obj_raw, stats;
-    DevBuf<long long> od_map_off, out_count, out_off, check_off;
-    DevBuf<ScanState> st;
-    DevBuf<Box> boxes, boxes0;                   // boxes0: the scene boxes as loaded (re-arm drops the inserted ones, device to device)
-    DevBuf<BoxTest> box_tests;
-    DevBuf<ObjBox> obj, try_obj;
+    // the per-scan arrays of `dev` ([B][extent], allocated by per_scan()): device memory owned by the engine, and the
+    // field's byte offset in EngineDev and per-scan byte stride, by which sub_view() moves it to a sub-batch
+    struct PerScan { size_t field, stride; void* p; };
+    std::vector<PerScan> scan_arrays;
+    // batch-wide device buffers, and buffers the kernels do not see through EngineDev
+    DevBuf<float4> out_xyzi;
+    DevBuf<double> obj_x, obj_y, obj_z, cos_k, sin_k, radii_sq;
+    DevBuf<float> obj_i, out_check;
+    DevBuf<unsigned> obj_label, out_label, round_ctl;
+    DevBuf<unsigned short> label16, out_label16;
+    DevBuf<unsigned char> label1, od_maps, ss_map;
+    DevBuf<int> active_count, perms, class_list_off, class_list, radii_ok, n0_arr, nbox0_arr;
+    DevBuf<unsigned long long> stats;
+    DevBuf<long long> pt_off, od_map_off, out_off, check_off;
+    DevBuf<Box> boxes0;                          // the scene boxes as loaded (re-arm drops the inserted ones, device to device)
+    DevBuf<ObjBox> obj;
     DevBuf<ClassCfg> classes;
     CUtensorMap zraw_tmap;            // [B][H][W] u64 z-buffer as a 3-D tiled tensor, box = one staged close/fill tile
     bool zraw_tmap_ok = false;
-    // host copies needed for re-arming
-    std::vector<Box> h_boxes;
-    std::vector<int> h_nbox0;
+    std::vector<int> h_nbox0;                    // scene boxes per scan of the loaded batch
     unsigned long long* h_words = nullptr;   // mapped pinned: one word per round slot, written by k_ctrl
     unsigned long long* d_words = nullptr;   // device alias of h_words
     unsigned seq = 0;
@@ -138,6 +135,24 @@ struct r3d_engine {
     int64_t prof_launches[KID_COUNT] = {0};
     std::vector<std::pair<int, std::pair<cudaEvent_t, cudaEvent_t>>> pending_events;
     std::vector<cudaEvent_t> event_pool;
+
+    // releases everything, also of an engine whose creation failed part way (null handles are skipped); the DevBuf
+    // members are freed after this body, once the sub-batch streams are idle
+    ~r3d_engine() {
+        for (int i = 0; i < R3D_MAX_SUB; ++i) {
+            if (sub_stream[i]) { cudaStreamSynchronize(sub_stream[i]); cudaStreamDestroy(sub_stream[i]); }
+            if (sub_done[i]) cudaEventDestroy(sub_done[i]);
+            if (round_graph[i].exec) cudaGraphExecDestroy(round_graph[i].exec);
+        }
+        for (const PerScan& a : scan_arrays) cudaFree(a.p);
+        for (cudaEvent_t ev : event_pool) cudaEventDestroy(ev);
+        for (cudaEvent_t ev : {ev_armed, ev_wait, ev_idx})
+            if (ev) cudaEventDestroy(ev);
+        if (h_words) cudaFreeHost(h_words);
+        if (h_offsets) cudaFreeHost(h_offsets);
+        if (h_idx) cudaFreeHost(h_idx);
+        if (stream) cudaStreamDestroy(stream);
+    }
 };
 
 namespace {
@@ -224,6 +239,37 @@ size_t select_smem_bytes(int max_pts) {
            2 * (size_t)(SEL_TILE_PX / 32) * 4 + 16;
 }
 
+// Allocates the per-scan array `field` of eng->dev: B x `extent` elements, owned by the engine.  This is the only place
+// that states a per-scan array's extent: sub_view() offsets every array allocated here by the same stride.  A field
+// allocated again (a new object DB) frees its previous array.
+template <class T>
+int per_scan(r3d_engine* eng, T*& field, size_t extent) {
+    const size_t at = (size_t)(reinterpret_cast<char*>(&field) - reinterpret_cast<char*>(&eng->dev));
+    for (size_t i = 0; i < eng->scan_arrays.size(); ++i)
+        if (eng->scan_arrays[i].field == at) {
+            cudaFree(eng->scan_arrays[i].p);
+            eng->scan_arrays.erase(eng->scan_arrays.begin() + i);
+            break;
+        }
+    field = nullptr;
+    void* p = nullptr;
+    const cudaError_t err = cudaMalloc(&p, (size_t)eng->dev.B * extent * sizeof(T));
+    if (err != cudaSuccess) return r3d_fail_cuda(err, "cudaMalloc");
+    eng->scan_arrays.push_back({at, extent * sizeof(T), p});
+    field = static_cast<T*>(p);
+    return R3D_OK;
+}
+
+// the host fills some arrays the kernels only read (EngineDev declares them const)
+template <class T> T* mut(const T* p) { return const_cast<T*>(p); }
+
+// every API call first binds the calling thread to the engine's device; false for a null engine
+bool bind(r3d_engine* eng) {
+    if (!eng) return false;
+    cudaSetDevice(eng->device);
+    return true;
+}
+
 }  // namespace
 
 #define TRY(x) do { int _rc = (x); if (_rc != R3D_OK) return _rc; } while (0)
@@ -273,27 +319,9 @@ extern "C" int r3d_engine_create(const r3d_engine_cfg* cfg, r3d_engine** out) {
     int count = 0;
     if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0)
         return r3d_fail(R3D_ERR_CUDA, "r3d_engine_create: no CUDA device (this library has no CPU fallback)");
-    r3d_engine* eng = new r3d_engine();
+    std::unique_ptr<r3d_engine> owner(new r3d_engine());           // frees whatever was created if a step below fails
+    r3d_engine* eng = owner.get();
     eng->cfg = *cfg;
-    R3D_CUDA(cudaGetDevice(&eng->device));
-    // the round kernels (short, latency bound) run on high-priority streams; uploads, the one-off spherical ingest /
-    // index builds and the output compaction of OTHER engines on the same GPU (ScanPipeline) must not sit in front of them
-    int prio_least = 0, prio_greatest = 0;
-    R3D_CUDA(cudaDeviceGetStreamPriorityRange(&prio_least, &prio_greatest));
-    R3D_CUDA(cudaStreamCreateWithPriority(&eng->stream, cudaStreamNonBlocking, prio_least));
-    eng->n_sub = (cfg->flags >> 8) & 31;
-    eng->use_graphs = !(cfg->flags & 2);
-    eng->staged = (cfg->flags & 8) != 0;
-    if (const char* env = getenv("R3D_STAGED")) eng->staged = atoi(env) != 0;
-    if (const char* env = getenv("R3D_GRAPHS")) eng->use_graphs = atoi(env) != 0;
-    if (const char* env = getenv("R3D_SUBBATCHES")) eng->n_sub = atoi(env);
-    if (eng->n_sub <= 0) eng->n_sub = 4;
-    eng->n_sub = std::min(eng->n_sub, R3D_MAX_SUB);
-    for (int i = 0; i < R3D_MAX_SUB; ++i) {
-        R3D_CUDA(cudaStreamCreateWithPriority(&eng->sub_stream[i], cudaStreamNonBlocking, prio_greatest));
-        R3D_CUDA(cudaEventCreateWithFlags(&eng->sub_done[i], cudaEventDisableTiming));
-    }
-    R3D_CUDA(cudaEventCreateWithFlags(&eng->ev_armed, cudaEventDisableTiming));
     EngineDev& d = eng->dev;
     memset(&d, 0, sizeof(d));
     d.task = cfg->task; d.rows = cfg->rows; d.cols = cfg->cols; d.hw = cfg->rows * cfg->cols; d.K = cfg->yaw_steps;
@@ -308,54 +336,12 @@ extern "C" int r3d_engine_create(const r3d_engine_cfg* cfg, r3d_engine** out) {
     d.grid_inv_cell = (float)(1.0 / d.grid_cell);
     d.G = 2 * (cfg->grid_half > 0 ? cfg->grid_half : 200);
     d.force_full = (cfg->flags & 1) ? 1 : 0;
-    const size_t B = d.B, P = d.P, K1 = d.K + 1, HW = d.hw;
-    TRY(eng->xyzi.alloc(B * d.max_points)); TRY(eng->tail_x.alloc(B * d.max_inserted)); TRY(eng->tail_y.alloc(B * d.max_inserted));
-    TRY(eng->tail_z.alloc(B * d.max_inserted)); TRY(eng->tail_i.alloc(B * d.max_inserted)); TRY(eng->label.alloc(B * P));
-    TRY(eng->r.alloc(B * P)); TRY(eng->el.alloc(B * P)); TRY(eng->col.alloc(B * P)); TRY(eng->pix.alloc(B * P));
-    TRY(eng->alive.alloc(B * P)); TRY(eng->zraw.alloc(B * HW)); TRY(eng->obj_raw.alloc(B * HW)); TRY(eng->smooth.alloc(B * HW));
-    eng->zraw_tmap_ok = make_zraw_tensor_map(&eng->zraw_tmap, eng->zraw.p, d.cols, d.rows, (int)B);
-    TRY(eng->dmask.alloc(B * d.dwords)); TRY(eng->vmask.alloc(B * d.dwords)); TRY(eng->st.alloc(B));
-    TRY(eng->gate_update.alloc(B)); TRY(eng->gate_try.alloc(B)); TRY(eng->gate_apply.alloc(B)); TRY(eng->gate_full.alloc(B));
-    TRY(eng->gate_patch.alloc(B)); TRY(eng->cf_rect.alloc(B * 4)); TRY(eng->active_count.alloc(R3D_MAX_SUB * 64 * 2));
-    TRY(eng->round_ctl.alloc(R3D_MAX_SUB * 32));
     d.cf_tiles_x = (d.cols + CF_TW - 1) / CF_TW;
     d.cf_tiles = d.cf_tiles_x * ((d.rows + CF_TH - 1) / CF_TH);
-    TRY(eng->work_cnt.alloc(B * 4)); TRY(eng->full_list.alloc(B)); TRY(eng->cf_tasks.alloc(B * (size_t)d.cf_tiles));
-    R3D_CUDA(cudaMemset(eng->work_cnt.p, 0, B * 4 * sizeof(int)));
-    TRY(eng->need2.alloc(B));
-    R3D_CUDA(cudaMemset(eng->need2.p, 0, B * sizeof(int)));
     d.cand_window = (cfg->flags & 4) ? 0 : 48;
-    if (const char* env = getenv("R3D_WINDOW")) d.cand_window = std::max(0, atoi(env));
     if (d.task != 0) d.cand_window = 0;          // semseg walks the yaws with a carried z shift (ss/fs:146-147): no window
-    TRY(eng->far_arr.alloc(B)); TRY(eng->boxes.alloc(B * d.max_boxes)); TRY(eng->box_tests.alloc(B * d.max_boxes));
-    TRY(eng->boxes0.alloc(B * d.max_boxes));
-    TRY(eng->poses.alloc(B * 16)); TRY(eng->occ_win.alloc(B * ((size_t)d.map_window * d.map_window / 32)));
-    TRY(eng->counts.alloc(B * d.n_classes)); TRY(eng->cos_k.alloc(K1)); TRY(eng->sin_k.alloc(K1));
-    TRY(eng->radii_sq.alloc(R3D_NUM_RADII)); TRY(eng->radii_ok.alloc(R3D_NUM_RADII)); TRY(eng->classes.alloc(R3D_MAX_CLASSES));
-    TRY(eng->cand_flags.alloc(B * K1)); TRY(eng->cand_level.alloc(B * K1)); TRY(eng->cand_v.alloc(B * K1));
-    TRY(eng->cand_list.alloc(B * K1)); TRY(eng->n_list.alloc(B)); TRY(eng->tickets.alloc(B * 4));
-    R3D_CUDA(cudaMemset(eng->tickets.p, 0, B * 4 * sizeof(unsigned)));
-    TRY(eng->feas.alloc(B * d.K)); TRY(eng->inserted.alloc(B * d.max_events * 4)); TRY(eng->inserted_box.alloc(B * d.max_events * 8));
-    TRY(eng->check.alloc(B * d.max_inserted * 5)); TRY(eng->out_count.alloc(B)); TRY(eng->out_off.alloc(B + 1));
-    TRY(eng->check_off.alloc(B + 1)); TRY(eng->out_xyzi.alloc(B * P)); TRY(eng->out_label.alloc(B * P));
-    TRY(eng->out_check.alloc(B * d.max_inserted * 5)); TRY(eng->n0_arr.alloc(B)); TRY(eng->nbox0_arr.alloc(B));
-    TRY(eng->gcell.alloc(B * (size_t)d.G * d.G)); TRY(eng->gpts.alloc(B * d.max_points));
-    TRY(eng->gnear.alloc(B * (size_t)d.G * d.G)); TRY(eng->gscratch.alloc(B * (size_t)d.G * d.G));
-    TRY(eng->col_off.alloc(B * (size_t)(d.cols + 1))); TRY(eng->col_idx.alloc(B * d.max_points));
-    TRY(eng->acell.alloc(B * (size_t)d.G * d.G)); TRY(eng->apts.alloc(B * d.max_points));
-    TRY(eng->try_obj.alloc(B));
     d.max_chunks = (d.P + CHUNK - 1) / CHUNK;
-    TRY(eng->chunk_cnt.alloc(B * (size_t)d.max_chunks));
-    { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&eng->n_sms, cudaDevAttrMultiProcessorCount, dev); }
-    TRY(eng->od_map_off.alloc(B * 2 + 1)); TRY(eng->od_map_dims.alloc(B * 8)); TRY(eng->stats.alloc(R3D_N_STATS));
-    R3D_CUDA(cudaMemset(eng->stats.p, 0, R3D_N_STATS * sizeof(unsigned long long)));
-    TRY(eng->occ_far.alloc(B * (OCC_FAR_CAP + 1)));
-    if (cfg->task == 1) TRY(eng->occ_cnt.alloc(B * (size_t)d.map_window * d.map_window));
-    R3D_CUDA(cudaMemset(eng->occ_far.p, 0xFF, B * (OCC_FAR_CAP + 1) * sizeof(int)));
-    R3D_CUDA(cudaHostAlloc((void**)&eng->h_words, R3D_MAX_SUB * 64 * sizeof(unsigned long long), cudaHostAllocMapped));
-    memset(eng->h_words, 0, R3D_MAX_SUB * 64 * sizeof(unsigned long long));
-    R3D_CUDA(cudaHostGetDevicePointer((void**)&eng->d_words, eng->h_words, 0));
-    R3D_CUDA(cudaMallocHost((void**)&eng->h_offsets, (2 * (B + 1) + 1) * sizeof(long long)));
+    if (d.max_points + d.max_inserted > (1 << APT_IDX_BITS)) return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_create: more than 2^27 points per scan");
     std::vector<ClassCfg> cls(R3D_MAX_CLASSES);
     for (int c = 0; c < R3D_MAX_CLASSES; ++c) {
         const r3d_class_cfg& s = cfg->classes[c];
@@ -375,60 +361,84 @@ extern "C" int r3d_engine_create(const r3d_engine_cfg* cfg, r3d_engine** out) {
             }
             cls[c].ok_slots |= 1u << slot;
         }
-    if (d.max_points + d.max_inserted > (1 << APT_IDX_BITS)) return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_create: more than 2^27 points per scan");
+    eng->n_sub = (cfg->flags >> 8) & 31;
+    if (eng->n_sub <= 0) eng->n_sub = 4;
+    eng->n_sub = std::min(eng->n_sub, R3D_MAX_SUB);
+    eng->use_graphs = !(cfg->flags & 2);
+    eng->staged = (cfg->flags & 8) != 0;
+    R3D_CUDA(cudaGetDevice(&eng->device));
+    R3D_CUDA(cudaDeviceGetAttribute(&eng->n_sms, cudaDevAttrMultiProcessorCount, eng->device));
+    // the round kernels (short, latency bound) run on high-priority streams; uploads, the one-off spherical ingest /
+    // index builds and the output compaction of OTHER engines on the same GPU (ScanPipeline) must not sit in front of them
+    int prio_least = 0, prio_greatest = 0;
+    R3D_CUDA(cudaDeviceGetStreamPriorityRange(&prio_least, &prio_greatest));
+    R3D_CUDA(cudaStreamCreateWithPriority(&eng->stream, cudaStreamNonBlocking, prio_least));
+    for (int i = 0; i < R3D_MAX_SUB; ++i) {
+        R3D_CUDA(cudaStreamCreateWithPriority(&eng->sub_stream[i], cudaStreamNonBlocking, prio_greatest));
+        R3D_CUDA(cudaEventCreateWithFlags(&eng->sub_done[i], cudaEventDisableTiming));
+    }
+    R3D_CUDA(cudaEventCreateWithFlags(&eng->ev_armed, cudaEventDisableTiming));
+    const size_t B = d.B, P = d.P, K1 = d.K + 1, GG = (size_t)d.G * d.G, MW2 = (size_t)d.map_window * d.map_window;
+    TRY(per_scan(eng, d.xyzi, d.max_points)); TRY(per_scan(eng, d.tail_x, d.max_inserted)); TRY(per_scan(eng, d.tail_y, d.max_inserted));
+    TRY(per_scan(eng, d.tail_z, d.max_inserted)); TRY(per_scan(eng, d.tail_i, d.max_inserted)); TRY(per_scan(eng, d.label, P));
+    TRY(per_scan(eng, d.r, P)); TRY(per_scan(eng, d.el, P)); TRY(per_scan(eng, d.col, P)); TRY(per_scan(eng, d.pix, P));
+    TRY(per_scan(eng, d.alive, P)); TRY(per_scan(eng, d.zraw, d.hw)); TRY(per_scan(eng, d.obj_raw, d.hw)); TRY(per_scan(eng, d.smooth, d.hw));
+    eng->zraw_tmap_ok = make_zraw_tensor_map(&eng->zraw_tmap, d.zraw, d.cols, d.rows, (int)B);
+    TRY(per_scan(eng, d.dmask, d.dwords)); TRY(per_scan(eng, d.vmask, d.dwords)); TRY(per_scan(eng, d.st, 1));
+    TRY(per_scan(eng, d.gate_update, 1)); TRY(per_scan(eng, d.gate_try, 1)); TRY(per_scan(eng, d.gate_apply, 1));
+    TRY(per_scan(eng, d.gate_full, 1)); TRY(per_scan(eng, d.gate_patch, 1)); TRY(per_scan(eng, d.cf_rect, 4));
+    TRY(per_scan(eng, d.work_cnt, 4)); TRY(per_scan(eng, d.full_list, 1)); TRY(per_scan(eng, d.cf_tasks, d.cf_tiles));
+    TRY(per_scan(eng, d.need2, 1)); TRY(per_scan(eng, d.far_arr, 1)); TRY(per_scan(eng, d.boxes, d.max_boxes));
+    TRY(per_scan(eng, d.box_tests, d.max_boxes)); TRY(per_scan(eng, d.poses, 16)); TRY(per_scan(eng, d.occ_win, MW2 / 32));
+    TRY(per_scan(eng, d.counts, d.n_classes)); TRY(per_scan(eng, d.cand_flags, K1)); TRY(per_scan(eng, d.cand_level, K1));
+    TRY(per_scan(eng, d.cand_v, K1)); TRY(per_scan(eng, d.cand_list, K1)); TRY(per_scan(eng, d.n_list, 1));
+    TRY(per_scan(eng, d.tickets, 4)); TRY(per_scan(eng, d.feas, d.K)); TRY(per_scan(eng, d.inserted, (size_t)d.max_events * 4));
+    TRY(per_scan(eng, d.inserted_box, (size_t)d.max_events * 8)); TRY(per_scan(eng, d.check, (size_t)d.max_inserted * 5));
+    TRY(per_scan(eng, d.out_count, 1)); TRY(per_scan(eng, d.gcell, GG)); TRY(per_scan(eng, d.gpts, d.max_points));
+    TRY(per_scan(eng, d.gnear, GG)); TRY(per_scan(eng, d.gscratch, GG)); TRY(per_scan(eng, d.col_off, d.cols + 1));
+    TRY(per_scan(eng, d.col_idx, d.max_points)); TRY(per_scan(eng, d.acell, GG)); TRY(per_scan(eng, d.apts, d.max_points));
+    TRY(per_scan(eng, d.try_obj, 1)); TRY(per_scan(eng, d.chunk_cnt, d.max_chunks)); TRY(per_scan(eng, d.od_map_dims, 8));
+    TRY(per_scan(eng, d.occ_far, OCC_FAR_CAP + 1));
+    if (cfg->task == 1) TRY(per_scan(eng, d.occ_cnt, MW2));
+    TRY(eng->active_count.alloc(R3D_MAX_SUB * 64 * 2)); TRY(eng->round_ctl.alloc(R3D_MAX_SUB * 32));
+    TRY(eng->out_off.alloc(B + 1)); TRY(eng->check_off.alloc(B + 1)); TRY(eng->out_xyzi.alloc(B * P)); TRY(eng->out_label.alloc(B * P));
+    TRY(eng->out_check.alloc(B * d.max_inserted * 5)); TRY(eng->n0_arr.alloc(B)); TRY(eng->nbox0_arr.alloc(B));
+    TRY(eng->boxes0.alloc(B * d.max_boxes)); TRY(eng->cos_k.alloc(K1)); TRY(eng->sin_k.alloc(K1));
+    TRY(eng->radii_sq.alloc(R3D_NUM_RADII)); TRY(eng->radii_ok.alloc(R3D_NUM_RADII)); TRY(eng->classes.alloc(R3D_MAX_CLASSES));
+    TRY(eng->od_map_off.alloc(B * 2 + 1)); TRY(eng->stats.alloc(R3D_N_STATS));
+    d.active_count = eng->active_count.p; d.out_off = eng->out_off.p; d.check_off = eng->check_off.p;
+    d.out_xyzi = eng->out_xyzi.p; d.out_label = eng->out_label.p; d.out_check = eng->out_check.p;
+    d.cos_k = eng->cos_k.p; d.sin_k = eng->sin_k.p; d.radii_sq = eng->radii_sq.p; d.radii_ok = eng->radii_ok.p;
+    d.classes = eng->classes.p; d.od_map_off = eng->od_map_off.p; d.stats = eng->stats.p;
+    R3D_CUDA(cudaMemset(d.work_cnt, 0, B * 4 * sizeof(int)));
+    R3D_CUDA(cudaMemset(d.need2, 0, B * sizeof(int)));
+    R3D_CUDA(cudaMemset(d.tickets, 0, B * 4 * sizeof(unsigned)));
+    R3D_CUDA(cudaMemset(d.stats, 0, R3D_N_STATS * sizeof(unsigned long long)));
+    R3D_CUDA(cudaMemset(d.occ_far, 0xFF, B * (OCC_FAR_CAP + 1) * sizeof(int)));
+    R3D_CUDA(cudaHostAlloc((void**)&eng->h_words, R3D_MAX_SUB * 64 * sizeof(unsigned long long), cudaHostAllocMapped));
+    memset(eng->h_words, 0, R3D_MAX_SUB * 64 * sizeof(unsigned long long));
+    R3D_CUDA(cudaHostGetDevicePointer((void**)&eng->d_words, eng->h_words, 0));
+    R3D_CUDA(cudaMallocHost((void**)&eng->h_offsets, (2 * (B + 1) + 1) * sizeof(long long)));
     R3D_CUDA(cudaMemcpy(eng->classes.p, cls.data(), cls.size() * sizeof(ClassCfg), cudaMemcpyHostToDevice));
     R3D_CUDA(cudaMemcpy(eng->radii_sq.p, cfg->radii_sq, sizeof(cfg->radii_sq), cudaMemcpyHostToDevice));
     R3D_CUDA(cudaMemcpy(eng->radii_ok.p, cfg->radii_ok, sizeof(cfg->radii_ok), cudaMemcpyHostToDevice));
-    k_fill_u64<<<148 * 4, 256, 0, eng->stream>>>(eng->obj_raw.p, B * HW, R3D_EMPTY_U64); r3d_count_launch();
-    R3D_CUDA(cudaMemsetAsync(eng->dmask.p, 0, B * d.dwords * sizeof(unsigned), eng->stream));
+    k_fill_u64<<<148 * 4, 256, 0, eng->stream>>>(d.obj_raw, B * d.hw, R3D_EMPTY_U64); r3d_count_launch();
+    R3D_CUDA(cudaMemsetAsync(d.dmask, 0, B * d.dwords * sizeof(unsigned), eng->stream));
     R3D_CUDA(cudaStreamSynchronize(eng->stream));
-    // wire the device view
-    d.xyzi = eng->xyzi.p; d.tail_x = eng->tail_x.p; d.tail_y = eng->tail_y.p; d.tail_z = eng->tail_z.p; d.tail_i = eng->tail_i.p;
-    d.label = eng->label.p; d.r = eng->r.p; d.el = eng->el.p; d.col = eng->col.p; d.pix = eng->pix.p; d.alive = eng->alive.p;
-    d.zraw = eng->zraw.p; d.obj_raw = eng->obj_raw.p; d.smooth = eng->smooth.p; d.dmask = eng->dmask.p; d.vmask = eng->vmask.p;
-    d.st = eng->st.p; d.gate_update = eng->gate_update.p; d.gate_try = eng->gate_try.p; d.gate_apply = eng->gate_apply.p;
-    d.gate_full = eng->gate_full.p; d.gate_patch = eng->gate_patch.p; d.cf_rect = eng->cf_rect.p;
-    d.work_cnt = eng->work_cnt.p; d.full_list = eng->full_list.p; d.cf_tasks = eng->cf_tasks.p; d.need2 = eng->need2.p;
-    d.active_count = eng->active_count.p; d.far_arr = eng->far_arr.p; d.boxes = eng->boxes.p; d.box_tests = eng->box_tests.p;
-    d.poses = eng->poses.p; d.occ_win = eng->occ_win.p; d.counts = eng->counts.p; d.cos_k = eng->cos_k.p; d.sin_k = eng->sin_k.p;
-    d.radii_sq = eng->radii_sq.p; d.radii_ok = eng->radii_ok.p; d.classes = eng->classes.p; d.cand_flags = eng->cand_flags.p;
-    d.cand_level = eng->cand_level.p; d.cand_list = eng->cand_list.p; d.n_list = eng->n_list.p; d.tickets = eng->tickets.p;
-    d.cand_v = eng->cand_v.p; d.feas = eng->feas.p; d.inserted = eng->inserted.p; d.inserted_box = eng->inserted_box.p;
-    d.check = eng->check.p; d.out_count = eng->out_count.p; d.out_off = eng->out_off.p; d.check_off = eng->check_off.p;
-    d.out_xyzi = eng->out_xyzi.p; d.out_label = eng->out_label.p; d.out_check = eng->out_check.p;
-    d.gcell = eng->gcell.p; d.gpts = eng->gpts.p; d.gnear = eng->gnear.p; d.gscratch = eng->gscratch.p;
-    d.col_off = eng->col_off.p; d.col_idx = eng->col_idx.p; d.acell = eng->acell.p; d.apts = eng->apts.p;
-    d.try_obj = eng->try_obj.p; d.chunk_cnt = eng->chunk_cnt.p;
-    d.od_map_off = eng->od_map_off.p; d.od_map_dims = eng->od_map_dims.p; d.stats = eng->stats.p; d.occ_far = eng->occ_far.p; d.occ_cnt = eng->occ_cnt.p;
-    *out = eng;
+    *out = owner.release();
     return R3D_OK;
 }
 
 extern "C" int r3d_engine_destroy(r3d_engine* eng) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng) return R3D_OK;
+    if (!bind(eng)) return R3D_OK;
     cudaStreamSynchronize(eng->stream);
     drain_events(eng);
-    for (cudaEvent_t ev : eng->event_pool) cudaEventDestroy(ev);
-    if (eng->h_words) cudaFreeHost(eng->h_words);
-    if (eng->h_offsets) cudaFreeHost(eng->h_offsets);
-    for (int i = 0; i < R3D_MAX_SUB; ++i) {
-        if (eng->sub_stream[i]) { cudaStreamSynchronize(eng->sub_stream[i]); cudaStreamDestroy(eng->sub_stream[i]); }
-        if (eng->sub_done[i]) cudaEventDestroy(eng->sub_done[i]);
-    }
-    if (eng->ev_armed) cudaEventDestroy(eng->ev_armed);
-    if (eng->ev_wait) cudaEventDestroy(eng->ev_wait);
-    if (eng->ev_idx) cudaEventDestroy(eng->ev_idx);
-    if (eng->h_idx) cudaFreeHost(eng->h_idx);
-    for (int i = 0; i < R3D_MAX_SUB; ++i) if (eng->round_graph[i].exec) cudaGraphExecDestroy(eng->round_graph[i].exec);
-    cudaStreamDestroy(eng->stream);
     delete eng;
     return R3D_OK;
 }
 
 extern "C" int r3d_engine_set_yaw_tables(r3d_engine* eng, const double* cos_k, const double* sin_k) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !cos_k || !sin_k) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_yaw_tables: null argument");
+    if (!bind(eng) || !cos_k || !sin_k) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_yaw_tables: null argument");
     const size_t n = (size_t)eng->dev.K + 1;
     R3D_CUDA(cudaMemcpy(eng->cos_k.p, cos_k, n * sizeof(double), cudaMemcpyHostToDevice));
     R3D_CUDA(cudaMemcpy(eng->sin_k.p, sin_k, n * sizeof(double), cudaMemcpyHostToDevice));
@@ -437,8 +447,7 @@ extern "C" int r3d_engine_set_yaw_tables(r3d_engine* eng, const double* cos_k, c
 }
 
 extern "C" int r3d_engine_set_objects(r3d_engine* eng, const r3d_object_db* db) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !db || db->n_objects <= 0) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_objects: bad argument");
+    if (!bind(eng) || !db || db->n_objects <= 0) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_objects: bad argument");
     EngineDev& d = eng->dev;
     const int n = db->n_objects;
     const int64_t total = db->point_offsets[n];
@@ -478,8 +487,8 @@ extern "C" int r3d_engine_set_objects(r3d_engine* eng, const r3d_object_db* db) 
     TRY(eng->obj_label.alloc(total)); TRY(eng->obj.alloc(n)); TRY(eng->class_list_off.alloc(d.n_classes + 1));
     const int nl = db->class_list_offsets[d.n_classes];
     TRY(eng->class_list.alloc(std::max(nl, 1)));
-    TRY(eng->unplaceable.alloc((size_t)d.B * ((n + 31) / 32)));
-    TRY(eng->occ_pix.alloc((size_t)d.B * OCC_G * max_pts)); TRY(eng->sel_pix.alloc((size_t)d.B * max_pts));
+    TRY(per_scan(eng, d.unplaceable, (n + 31) / 32));
+    TRY(per_scan(eng, d.occ_pix, (size_t)OCC_G * max_pts)); TRY(per_scan(eng, d.sel_pix, max_pts));
     R3D_CUDA(cudaMemcpy(eng->obj_x.p, x.data(), total * sizeof(double), cudaMemcpyHostToDevice));
     R3D_CUDA(cudaMemcpy(eng->obj_y.p, y.data(), total * sizeof(double), cudaMemcpyHostToDevice));
     R3D_CUDA(cudaMemcpy(eng->obj_z.p, z.data(), total * sizeof(double), cudaMemcpyHostToDevice));
@@ -490,13 +499,11 @@ extern "C" int r3d_engine_set_objects(r3d_engine* eng, const r3d_object_db* db) 
     R3D_CUDA(cudaMemcpy(eng->class_list.p, db->class_list, nl * sizeof(int), cudaMemcpyHostToDevice));
     d.obj_x = eng->obj_x.p; d.obj_y = eng->obj_y.p; d.obj_z = eng->obj_z.p; d.obj_i = eng->obj_i.p; d.obj_label = eng->obj_label.p;
     d.obj = eng->obj.p; d.class_list_off = eng->class_list_off.p; d.class_list = eng->class_list.p;
-    d.unplaceable = eng->unplaceable.p; d.occ_pix = eng->occ_pix.p; d.sel_pix = eng->sel_pix.p;
     const size_t sel_smem = select_smem_bytes(std::min(max_pts, SEL_SMEM_PTS));
     d.sel_key_cap = next_pow2(max_pts);
     if (max_pts > std::min(SEL_SMEM_PTS, walk_od::WALK_SEL_PTS)) {        // objects the selection cannot keep in shared memory
-        TRY(eng->sel_keys.alloc((size_t)d.B * d.sel_key_cap)); TRY(eng->sel_r.alloc((size_t)d.B * max_pts));
+        TRY(per_scan(eng, d.sel_keys, d.sel_key_cap)); TRY(per_scan(eng, d.sel_r, max_pts));
     }
-    d.sel_keys = eng->sel_keys.p; d.sel_r = eng->sel_r.p;
     R3D_CUDA(cudaFuncSetAttribute(k_select_emit, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sel_smem));
     R3D_CUDA(cudaFuncSetAttribute(k_occl_count, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)occl_smem_bytes(d)));
     if (onmap_smem_bytes(d.K) > 100 * 1024) return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_set_objects: too many yaw steps for the placement kernel's shared memory");
@@ -513,12 +520,26 @@ extern "C" int r3d_engine_set_objects(r3d_engine* eng, const r3d_object_db* db) 
 
 extern "C" int r3d_engine_set_ss_map(r3d_engine* eng, const uint8_t* map, int32_t size_x, int32_t size_y, int64_t move_x,
                                      int64_t move_y) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !map || size_x <= 0 || size_y <= 0) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_ss_map: bad argument");
+    if (!bind(eng) || !map || size_x <= 0 || size_y <= 0) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_ss_map: bad argument");
     TRY(eng->ss_map.alloc((size_t)size_x * size_y));
     R3D_CUDA(cudaMemcpy(eng->ss_map.p, map, (size_t)size_x * size_y, cudaMemcpyHostToDevice));
     eng->dev.ss_map = eng->ss_map.p; eng->dev.ss_sx = size_x; eng->dev.ss_sy = size_y;
     eng->dev.ss_move_x = move_x; eng->dev.ss_move_y = move_y;
+    return R3D_OK;
+}
+
+// per-box collision tests of the loaded batch's scene boxes
+static void launch_box_tests(r3d_engine* eng) {
+    const int slots = eng->n_scans * eng->dev.max_boxes;
+    k_box_tests<<<(slots + 127) / 128, 128, 0, eng->stream>>>(eng->dev.boxes, eng->dev.box_tests, slots);
+    r3d_count_launch();
+}
+
+// the scene boxes as loaded: drops the boxes appended by the previous run (device to device)
+static int restore_scene_boxes(r3d_engine* eng) {
+    const size_t slots = (size_t)eng->n_scans * eng->dev.max_boxes;
+    R3D_CUDA(cudaMemcpyAsync(eng->dev.boxes, eng->boxes0.p, slots * sizeof(Box), cudaMemcpyDeviceToDevice, eng->stream));
+    launch_box_tests(eng);
     return R3D_OK;
 }
 
@@ -528,12 +549,12 @@ static int arm_batch(r3d_engine* eng, bool ingest) {
     const int n = eng->n_scans;
     cudaStream_t st = eng->stream;
     k_reset_state<<<(n + 127) / 128, 128, 0, st>>>(d, n, eng->n0_arr.p, eng->nbox0_arr.p); r3d_count_launch();
-    R3D_CUDA(cudaMemsetAsync(eng->dmask.p, 0, (size_t)n * d.dwords * sizeof(unsigned), st));   // vis_px masks: cleared lazily afterwards
+    R3D_CUDA(cudaMemsetAsync(d.dmask, 0, (size_t)n * d.dwords * sizeof(unsigned), st));   // vis_px masks: cleared lazily afterwards
     const int chunks = (eng->max_n0 + CHUNK - 1) / CHUNK;
     if (ingest) {
-        R3D_CUDA(cudaMemsetAsync(eng->gcell.p, 0, (size_t)n * d.G * d.G * sizeof(int), st));
-        R3D_CUDA(cudaMemsetAsync(eng->col_off.p, 0, (size_t)n * (d.cols + 1) * sizeof(int), st));
-        R3D_CUDA(cudaMemsetAsync(eng->acell.p, 0, (size_t)n * d.G * d.G * sizeof(int), st));
+        R3D_CUDA(cudaMemsetAsync(d.gcell, 0, (size_t)n * d.G * d.G * sizeof(int), st));
+        R3D_CUDA(cudaMemsetAsync(d.col_off, 0, (size_t)n * (d.cols + 1) * sizeof(int), st));
+        R3D_CUDA(cudaMemsetAsync(d.acell, 0, (size_t)n * d.G * d.G * sizeof(int), st));
         { Launcher l(eng, KID_INGEST); k_ingest_count<<<dim3(chunks, n), STREAM_THREADS, 0, st>>>(d, n); }
         {
             Launcher l(eng, KID_GRID);
@@ -548,19 +569,36 @@ static int arm_batch(r3d_engine* eng, bool ingest) {
     } else {
         eng->fresh = false;
         k_reset_alive<<<dim3(std::max(chunks, 1), n), 256, 0, st>>>(d, n); r3d_count_launch();
-        // scene boxes: drop the boxes appended by the previous run
-        const size_t slots = (size_t)n * d.max_boxes;
-        R3D_CUDA(cudaMemcpyAsync(eng->boxes.p, eng->boxes0.p, slots * sizeof(Box), cudaMemcpyDeviceToDevice, st));
-        k_box_tests<<<(int)((slots + 127) / 128), 128, 0, st>>>(eng->boxes.p, eng->box_tests.p, (int)slots);
-        r3d_count_launch();
+        TRY(restore_scene_boxes(eng));
     }
     eng->ran = false;
     return r3d_check_launch("arm_batch");
 }
 
+// Checks that a batch fits the engine before anything of it is enqueued, and makes it the loaded shape: points[s]
+// points and boxes[s] scene boxes in scan s, at most `objects` objects in any scan's schedule.  The errors name the
+// entry point `fn`.
+static int set_batch_shape(r3d_engine* eng, const char* fn, const std::vector<int64_t>& points, const std::vector<int>& boxes,
+                           long long objects) {
+    const EngineDev& d = eng->dev;
+    auto fail = [fn](const char* what) { return r3d_fail(R3D_ERR_CAPACITY, (std::string(fn) + ": " + what).c_str()); };
+    int max_n0 = 0;
+    for (size_t s = 0; s < points.size(); ++s) {
+        if (points[s] <= 0 || points[s] > d.max_points) return fail("scan larger than max_points (or empty)");
+        if (boxes[s] > d.max_boxes) return fail("too many scene boxes");
+        max_n0 = std::max(max_n0, (int)points[s]);
+    }
+    if (objects + 1 > d.max_events)                 // a schedule must fit the per-scan event / insertion records
+        return fail("a scan's schedule asks for more objects than max_events - 1 "
+                    "(create the engine with max_events = objects per scan + 1)");
+    eng->n_scans = (int)points.size();
+    eng->max_n0 = max_n0;
+    eng->h_nbox0 = boxes;
+    return R3D_OK;
+}
+
 extern "C" int r3d_engine_load_batch(r3d_engine* eng, const r3d_batch* bt) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !bt) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_batch: null argument");
+    if (!bind(eng) || !bt) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_batch: null argument");
     if (!eng->objects_set || !eng->yaw_set) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_batch: set objects and yaw tables first");
     EngineDev& d = eng->dev;
     const int n = bt->n_scans;
@@ -570,31 +608,31 @@ extern "C" int r3d_engine_load_batch(r3d_engine* eng, const r3d_batch* bt) {
     if (d.task == 1 && (!bt->poses || !d.ss_map)) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_batch: semseg needs poses and the map");
     if (d.task == 0 && (!bt->maps || !bt->map_offsets || !bt->map_dims)) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_batch: OD needs maps");
     cudaStream_t st = eng->stream;
-    std::vector<int> n0(n), nb(n);
-    eng->max_n0 = 0;
+    std::vector<int64_t> points(n);
+    std::vector<int> nb(n, 0);
+    long long objects = 0;
     for (int s = 0; s < n; ++s) {
-        const int64_t cnt = bt->point_offsets[s + 1] - bt->point_offsets[s];
-        if (cnt <= 0 || cnt > d.max_points) return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_load_batch: scan larger than max_points (or empty)");
-        n0[s] = (int)cnt; eng->max_n0 = std::max(eng->max_n0, (int)cnt);
-        nb[s] = bt->box_offsets ? bt->box_offsets[s + 1] - bt->box_offsets[s] : 0;
-        if (nb[s] > d.max_boxes) return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_load_batch: too many scene boxes");
+        points[s] = bt->point_offsets[s + 1] - bt->point_offsets[s];
+        if (bt->box_offsets) nb[s] = bt->box_offsets[s + 1] - bt->box_offsets[s];
+        long long want = 0;
+        for (int c = 0; c < d.n_classes; ++c) want += std::max(bt->counts[(size_t)s * d.n_classes + c], 0);
+        objects = std::max(objects, want);
     }
-    eng->n_scans = n;
+    TRY(set_batch_shape(eng, "r3d_engine_load_batch", points, nb, objects));
+    const std::vector<int> n0(points.begin(), points.end());
     // scene boxes
-    eng->h_boxes.assign((size_t)n * d.max_boxes, Box());
+    std::vector<Box> h_boxes((size_t)n * d.max_boxes);
     for (int s = 0; s < n; ++s)
         for (int j = 0; j < nb[s]; ++j) {
             const double* src = bt->boxes + ((size_t)bt->box_offsets[s] + j) * R3D_BOX_DOUBLES;
-            Box& b = eng->h_boxes[(size_t)s * d.max_boxes + j];
+            Box& b = h_boxes[(size_t)s * d.max_boxes + j];
             b.cx = src[0]; b.cy = src[1]; b.cz = src[2];
             for (int i = 0; i < 9; ++i) b.m[i] = src[3 + i];
             b.length = src[12]; b.width = src[13]; b.height = src[14]; b.reach = src[15];
         }
-    eng->h_nbox0 = nb;
-    R3D_CUDA(cudaMemcpyAsync(eng->boxes.p, eng->h_boxes.data(), eng->h_boxes.size() * sizeof(Box), cudaMemcpyHostToDevice, st));
-    R3D_CUDA(cudaMemcpyAsync(eng->boxes0.p, eng->boxes.p, eng->h_boxes.size() * sizeof(Box), cudaMemcpyDeviceToDevice, st));
-    k_box_tests<<<(int)((eng->h_boxes.size() + 127) / 128), 128, 0, st>>>(eng->boxes.p, eng->box_tests.p, (int)eng->h_boxes.size());
-    r3d_count_launch();
+    R3D_CUDA(cudaMemcpyAsync(d.boxes, h_boxes.data(), h_boxes.size() * sizeof(Box), cudaMemcpyHostToDevice, st));
+    R3D_CUDA(cudaMemcpyAsync(eng->boxes0.p, d.boxes, h_boxes.size() * sizeof(Box), cudaMemcpyDeviceToDevice, st));
+    launch_box_tests(eng);
     R3D_CUDA(cudaMemcpyAsync(eng->n0_arr.p, n0.data(), n * sizeof(int), cudaMemcpyHostToDevice, st));
     R3D_CUDA(cudaMemcpyAsync(eng->nbox0_arr.p, nb.data(), n * sizeof(int), cudaMemcpyHostToDevice, st));
     if (d.task == 0) {
@@ -602,19 +640,12 @@ extern "C" int r3d_engine_load_batch(r3d_engine* eng, const r3d_batch* bt) {
         if ((size_t)bytes > eng->od_maps.n) TRY(eng->od_maps.alloc((size_t)bytes));
         R3D_CUDA(cudaMemcpyAsync(eng->od_maps.p, bt->maps, (size_t)bytes, cudaMemcpyHostToDevice, st));
         R3D_CUDA(cudaMemcpyAsync(eng->od_map_off.p, bt->map_offsets, ((size_t)n * 2 + 1) * sizeof(long long), cudaMemcpyHostToDevice, st));
-        R3D_CUDA(cudaMemcpyAsync(eng->od_map_dims.p, bt->map_dims, (size_t)n * 8 * sizeof(int), cudaMemcpyHostToDevice, st));
+        R3D_CUDA(cudaMemcpyAsync(mut(d.od_map_dims), bt->map_dims, (size_t)n * 8 * sizeof(int), cudaMemcpyHostToDevice, st));
         d.od_maps = eng->od_maps.p;
     } else {
-        R3D_CUDA(cudaMemcpyAsync(eng->poses.p, bt->poses, (size_t)n * 16 * sizeof(double), cudaMemcpyHostToDevice, st));
+        R3D_CUDA(cudaMemcpyAsync(mut(d.poses), bt->poses, (size_t)n * 16 * sizeof(double), cudaMemcpyHostToDevice, st));
     }
-    for (int sc = 0; sc < n; ++sc) {                  // a schedule must fit the per-scan event / insertion records
-        long long want = 0;
-        for (int c = 0; c < d.n_classes; ++c) want += std::max(bt->counts[(size_t)sc * d.n_classes + c], 0);
-        if (want + 1 > d.max_events)
-            return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_load_batch: a scan's schedule asks for more objects than max_events - 1 "
-                                              "(create the engine with max_events = objects per scan + 1)");
-    }
-    R3D_CUDA(cudaMemcpyAsync(eng->counts.p, bt->counts, (size_t)n * d.n_classes * sizeof(int), cudaMemcpyHostToDevice, st));
+    R3D_CUDA(cudaMemcpyAsync(mut(d.counts), bt->counts, (size_t)n * d.n_classes * sizeof(int), cudaMemcpyHostToDevice, st));
     const size_t nperm = (size_t)n * bt->n_events * d.n_classes * d.max_tries;
     if (nperm > eng->perms.n) TRY(eng->perms.alloc(nperm));
     R3D_CUDA(cudaMemcpyAsync(eng->perms.p, bt->perms, nperm * sizeof(int), cudaMemcpyHostToDevice, st));
@@ -640,23 +671,23 @@ extern "C" int r3d_engine_load_batch(r3d_engine* eng, const r3d_batch* bt) {
         R3D_CUDA(cudaMemcpyAsync(eng->pt_off.p, bt->point_offsets, ((size_t)n + 1) * sizeof(long long), cudaMemcpyHostToDevice, st));
     }
     if (uniform) {
-        R3D_CUDA(cudaMemcpy2DAsync(eng->xyzi.p, (size_t)d.max_points * sizeof(float4), bt->xyzi + bt->point_offsets[0] * 4,
+        R3D_CUDA(cudaMemcpy2DAsync(mut(d.xyzi), (size_t)d.max_points * sizeof(float4), bt->xyzi + bt->point_offsets[0] * 4,
                                    (size_t)n0[0] * sizeof(float4), (size_t)n0[0] * sizeof(float4), n, cudaMemcpyHostToDevice, st));
         if (!packed)
-            R3D_CUDA(cudaMemcpy2DAsync(eng->label.p, (size_t)d.P * sizeof(unsigned), bt->labels + bt->point_offsets[0],
+            R3D_CUDA(cudaMemcpy2DAsync(d.label, (size_t)d.P * sizeof(unsigned), bt->labels + bt->point_offsets[0],
                                        (size_t)n0[0] * sizeof(unsigned), (size_t)n0[0] * sizeof(unsigned), n, cudaMemcpyHostToDevice, st));
     } else {
         for (int s = 0; s < n; ++s) {
             const int64_t o = bt->point_offsets[s];
-            R3D_CUDA(cudaMemcpyAsync(eng->xyzi.p + (size_t)s * d.max_points, bt->xyzi + o * 4, (size_t)n0[s] * sizeof(float4), cudaMemcpyHostToDevice, st));
+            R3D_CUDA(cudaMemcpyAsync(mut(d.xyzi) + (size_t)s * d.max_points, bt->xyzi + o * 4, (size_t)n0[s] * sizeof(float4), cudaMemcpyHostToDevice, st));
             if (!packed)
-                R3D_CUDA(cudaMemcpyAsync(eng->label.p + (size_t)s * d.P, bt->labels + o, (size_t)n0[s] * sizeof(unsigned), cudaMemcpyHostToDevice, st));
+                R3D_CUDA(cudaMemcpyAsync(d.label + (size_t)s * d.P, bt->labels + o, (size_t)n0[s] * sizeof(unsigned), cudaMemcpyHostToDevice, st));
         }
     }
     if (packed) {
         const int chunks = (eng->max_n0 + CHUNK - 1) / CHUNK;
-        if (bits) k_expand_label_bits<<<dim3(chunks, n), STREAM_THREADS, 0, st>>>(eng->label1.p, eng->pt_off.p, eng->label.p, d.P, n, (unsigned)d.road_label);
-        else k_widen_labels<<<dim3(chunks, n), STREAM_THREADS, 0, st>>>(eng->label16.p, eng->pt_off.p, eng->label.p, d.P, n);
+        if (bits) k_expand_label_bits<<<dim3(chunks, n), STREAM_THREADS, 0, st>>>(eng->label1.p, eng->pt_off.p, d.label, d.P, n, (unsigned)d.road_label);
+        else k_widen_labels<<<dim3(chunks, n), STREAM_THREADS, 0, st>>>(eng->label16.p, eng->pt_off.p, d.label, d.P, n);
         r3d_count_launch();
     }
     // the std::vectors above are pageable: the copies from them completed before cudaMemcpyAsync returned
@@ -668,8 +699,7 @@ extern "C" int r3d_engine_load_batch(r3d_engine* eng, const r3d_batch* bt) {
 }
 
 extern "C" int r3d_engine_set_schedule_policy(r3d_engine* eng, int32_t random, int32_t number_of_object, const int32_t* fixed_counts) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || (random && number_of_object < 0) || (!random && !fixed_counts))
+    if (!bind(eng) || (random && number_of_object < 0) || (!random && !fixed_counts))
         return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_schedule_policy: bad argument");
     SchedulePolicy p;
     memset(&p, 0, sizeof(p));
@@ -686,8 +716,7 @@ extern "C" int r3d_engine_set_schedule_policy(r3d_engine* eng, int32_t random, i
 
 extern "C" int r3d_engine_load_resident(r3d_engine* eng, const r3d_resident_store* s, const int32_t* indices, int32_t n,
                                         uint64_t seed, uint64_t epoch) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !s || !indices) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: null argument");
+    if (!bind(eng) || !s || !indices) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: null argument");
     if (!eng->objects_set || !eng->yaw_set) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: set objects and yaw tables first");
     if (!eng->policy_set) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: set the schedule policy first");
     EngineDev& d = eng->dev;
@@ -698,22 +727,17 @@ extern "C" int r3d_engine_load_resident(r3d_engine* eng, const r3d_resident_stor
     if (d.task == 1 && (!s->poses || !d.ss_map)) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: semseg needs poses and the map");
     if (d.task == 0 && (!s->maps || !s->map_offsets || !s->map_dims)) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: OD needs maps");
     // the checks of r3d_engine_load_batch, on the host copies of the store's offsets
+    std::vector<int64_t> points(n);
     std::vector<int> nb(n);
-    int max_n0 = 0;
     for (int b = 0; b < n; ++b) {
         const int i = indices[b];
         if (i < 0 || i >= s->n_scans) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: index out of range");
-        const int64_t cnt = s->h_point_offsets[i + 1] - s->h_point_offsets[i];
-        if (cnt <= 0 || cnt > d.max_points) return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_load_resident: scan larger than max_points (or empty)");
-        max_n0 = std::max(max_n0, (int)cnt);
+        points[b] = s->h_point_offsets[i + 1] - s->h_point_offsets[i];
         nb[b] = s->h_box_offsets[i + 1] - s->h_box_offsets[i];
-        if (nb[b] > d.max_boxes) return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_load_resident: too many scene boxes");
     }
-    long long want = eng->policy.number_of_object;
-    if (!eng->policy.random) { want = 0; for (int c = 0; c < d.n_classes; ++c) want += eng->policy.fixed[c]; }
-    if (want + 1 > d.max_events)
-        return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_load_resident: a scan's schedule asks for more objects than max_events - 1 "
-                                          "(create the engine with max_events = objects per scan + 1)");
+    long long objects = eng->policy.number_of_object;
+    if (!eng->policy.random) { objects = 0; for (int c = 0; c < d.n_classes; ++c) objects += eng->policy.fixed[c]; }
+    TRY(set_batch_shape(eng, "r3d_engine_load_resident", points, nb, objects));
     const size_t nperm = (size_t)d.B * d.max_events * d.n_classes * d.max_tries;
     if (nperm > eng->perms.n) TRY(eng->perms.alloc(nperm));
     if (!eng->h_idx) {
@@ -727,20 +751,15 @@ extern "C" int r3d_engine_load_resident(r3d_engine* eng, const r3d_resident_stor
     memcpy(eng->h_idx, indices, (size_t)n * sizeof(int));
     R3D_CUDA(cudaMemcpyAsync(eng->idx_dev.p, eng->h_idx, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, st));
     R3D_CUDA(cudaEventRecord(eng->ev_idx, st));
-    eng->n_scans = n;
-    eng->max_n0 = max_n0;
-    eng->h_nbox0 = nb;
     const int* idx = eng->idx_dev.p;
     const int od = d.task == 0;
-    launch_gather_points(*s, idx, n, max_n0, eng->xyzi.p, d.max_points, eng->label.p, d.P, od, (unsigned)d.road_label, st);
-    launch_gather_meta(*s, idx, n, od, eng->n0_arr.p, eng->nbox0_arr.p, eng->od_map_off.p, eng->od_map_dims.p, eng->poses.p,
-                       eng->boxes.p, eng->boxes0.p, d.max_boxes, st);
-    const int slots = n * d.max_boxes;
-    k_box_tests<<<(slots + 127) / 128, 128, 0, st>>>(eng->boxes.p, eng->box_tests.p, slots);
-    r3d_count_launch();
+    launch_gather_points(*s, idx, n, eng->max_n0, mut(d.xyzi), d.max_points, d.label, d.P, od, (unsigned)d.road_label, st);
+    launch_gather_meta(*s, idx, n, od, eng->n0_arr.p, eng->nbox0_arr.p, eng->od_map_off.p, mut(d.od_map_dims), mut(d.poses),
+                       d.boxes, eng->boxes0.p, d.max_boxes, st);
+    launch_box_tests(eng);
     if (od) d.od_maps = s->maps;
     d.perms = eng->perms.p; d.n_perm_events = d.max_events;
-    launch_draw_schedule(idx, n, d.max_events, d.n_classes, d.max_tries, d.class_list_off, eng->policy, seed, epoch, eng->counts.p,
+    launch_draw_schedule(idx, n, d.max_events, d.n_classes, d.max_tries, d.class_list_off, eng->policy, seed, epoch, mut(d.counts),
                          eng->perms.p, st);
     if (eng->world_on) launch_draw_world(idx, n, eng->world_pol, seed, epoch, eng->world.p, st);
     d.world = eng->world_on ? eng->world.p : nullptr;
@@ -754,16 +773,14 @@ extern "C" int r3d_engine_load_resident(r3d_engine* eng, const r3d_resident_stor
 
 extern "C" int r3d_engine_set_ss_map_device(r3d_engine* eng, const uint8_t* map, int32_t size_x, int32_t size_y, int64_t move_x,
                                             int64_t move_y) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !map || size_x <= 0 || size_y <= 0) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_ss_map_device: bad argument");
+    if (!bind(eng) || !map || size_x <= 0 || size_y <= 0) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_ss_map_device: bad argument");
     eng->dev.ss_map = map; eng->dev.ss_sx = size_x; eng->dev.ss_sy = size_y;
     eng->dev.ss_move_x = move_x; eng->dev.ss_move_y = move_y;
     return R3D_OK;
 }
 
 extern "C" int r3d_engine_schedule_read(r3d_engine* eng, int32_t* counts, int32_t* perms, int32_t* n_events) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !counts || !n_events || !eng->batch_loaded) return r3d_fail(R3D_ERR_ARG, "r3d_engine_schedule_read: bad argument or no batch");
+    if (!bind(eng) || !counts || !n_events || !eng->batch_loaded) return r3d_fail(R3D_ERR_ARG, "r3d_engine_schedule_read: bad argument or no batch");
     const EngineDev& d = eng->dev;
     R3D_CUDA(engine_wait(eng));
     const size_t n = (size_t)eng->n_scans;
@@ -774,54 +791,58 @@ extern "C" int r3d_engine_schedule_read(r3d_engine* eng, int32_t* counts, int32_
 }
 
 extern "C" int r3d_engine_reset_batch(r3d_engine* eng) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !eng->batch_loaded) return r3d_fail(R3D_ERR_ARG, "r3d_engine_reset_batch: no batch loaded");
+    if (!bind(eng) || !eng->batch_loaded) return r3d_fail(R3D_ERR_ARG, "r3d_engine_reset_batch: no batch loaded");
     return arm_batch(eng, false);
 }
 
 extern "C" int r3d_engine_rearm_batch(r3d_engine* eng, int from_raw_points) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !eng->batch_loaded) return r3d_fail(R3D_ERR_ARG, "r3d_engine_rearm_batch: no batch loaded");
+    if (!bind(eng) || !eng->batch_loaded) return r3d_fail(R3D_ERR_ARG, "r3d_engine_rearm_batch: no batch loaded");
     if (!from_raw_points) return arm_batch(eng, false);
     // the whole device path from the resident float4 points again: scene boxes, spherical ingest, spatial indices
-    const size_t slots = (size_t)eng->n_scans * eng->dev.max_boxes;
-    R3D_CUDA(cudaMemcpyAsync(eng->boxes.p, eng->boxes0.p, slots * sizeof(Box), cudaMemcpyDeviceToDevice, eng->stream));
-    k_box_tests<<<(int)((slots + 127) / 128), 128, 0, eng->stream>>>(eng->boxes.p, eng->box_tests.p, (int)slots);
-    r3d_count_launch();
+    TRY(restore_scene_boxes(eng));
     return arm_batch(eng, true);
 }
 
 // view of the device data model that starts at scan b0: every per-scan array is [scan][...], so offsetting the base
 // pointers lets the kernels run unchanged on a contiguous sub-batch
-static EngineDev sub_view(const EngineDev& d, int b0) {
-    if (b0 == 0) return d;
-    EngineDev v = d;
-    const size_t b = (size_t)b0;
-    const size_t gg = (size_t)d.G * d.G, k1 = (size_t)d.K + 1, ww = (size_t)d.map_window * d.map_window / 32;
-#define R3D_OFF(field, stride) if (d.field) v.field = d.field + b * (size_t)(stride)
-    R3D_OFF(gcell, gg); R3D_OFF(gpts, d.max_points); R3D_OFF(gnear, gg); R3D_OFF(gscratch, gg); R3D_OFF(acell, gg); R3D_OFF(apts, d.max_points);
-    R3D_OFF(xyzi, d.max_points); R3D_OFF(tail_x, d.max_inserted); R3D_OFF(tail_y, d.max_inserted);
-    R3D_OFF(tail_z, d.max_inserted); R3D_OFF(tail_i, d.max_inserted); R3D_OFF(label, d.P); R3D_OFF(r, d.P); R3D_OFF(el, d.P);
-    R3D_OFF(col, d.P); R3D_OFF(pix, d.P); R3D_OFF(alive, d.P); R3D_OFF(zraw, d.hw); R3D_OFF(obj_raw, d.hw);
-    R3D_OFF(smooth, d.hw); R3D_OFF(dmask, d.dwords); R3D_OFF(vmask, d.dwords); R3D_OFF(st, 1); R3D_OFF(gate_update, 1);
-    R3D_OFF(gate_try, 1); R3D_OFF(gate_apply, 1); R3D_OFF(gate_full, 1); R3D_OFF(gate_patch, 1); R3D_OFF(cf_rect, 4);
-    R3D_OFF(work_cnt, 4); R3D_OFF(full_list, 1); R3D_OFF(cf_tasks, d.cf_tiles); R3D_OFF(need2, 1);
-    R3D_OFF(col_off, d.cols + 1); R3D_OFF(col_idx, d.max_points); R3D_OFF(far_arr, 1); R3D_OFF(boxes, d.max_boxes);
-    R3D_OFF(box_tests, d.max_boxes); R3D_OFF(od_map_off, 2); R3D_OFF(od_map_dims, 8); R3D_OFF(poses, 16); R3D_OFF(occ_win, ww);
-    R3D_OFF(counts, d.n_classes); R3D_OFF(perms, (size_t)d.n_perm_events * d.n_classes * d.max_tries);
-    R3D_OFF(unplaceable, (d.n_objects + 31) / 32); R3D_OFF(try_obj, 1); R3D_OFF(cand_flags, k1); R3D_OFF(cand_level, k1);
-    R3D_OFF(cand_v, k1); R3D_OFF(cand_list, k1); R3D_OFF(n_list, 1); R3D_OFF(tickets, 4); R3D_OFF(feas, d.K);
-    R3D_OFF(occ_pix, (size_t)OCC_G * d.max_obj_points); R3D_OFF(sel_pix, d.max_obj_points);
-    R3D_OFF(sel_keys, d.sel_key_cap); R3D_OFF(sel_r, d.max_obj_points); R3D_OFF(inserted, (size_t)d.max_events * 4);
-    R3D_OFF(inserted_box, (size_t)d.max_events * 8); R3D_OFF(check, (size_t)d.max_inserted * 5); R3D_OFF(chunk_cnt, d.max_chunks);
-    R3D_OFF(out_count, 1); R3D_OFF(occ_far, OCC_FAR_CAP + 1); R3D_OFF(occ_cnt, (size_t)d.map_window * d.map_window);
-#undef R3D_OFF
+static EngineDev sub_view(const r3d_engine* eng, int b0) {
+    EngineDev v = eng->dev;
+    if (b0 == 0) return v;
+    char* base = reinterpret_cast<char*>(&v);
+    for (const r3d_engine::PerScan& a : eng->scan_arrays) {
+        char* p;
+        memcpy(&p, base + a.field, sizeof(p));
+        p += (size_t)b0 * a.stride;
+        memcpy(base + a.field, &p, sizeof(p));
+    }
+    // perms: [n][n_perm_events][C][tries] of the loaded schedule, not of its allocation; od_map_off: [B][2] + an end slot
+    if (v.perms) v.perms += (size_t)b0 * v.n_perm_events * v.n_classes * v.max_tries;
+    if (v.od_map_off) v.od_map_off += (size_t)b0 * 2;
     return v;
 }
 
 extern "C" int r3d_engine_run_until(r3d_engine* eng, int stop_at, int* still_running);
 
 extern "C" int r3d_engine_run(r3d_engine* eng) { return r3d_engine_run_until(eng, 0, nullptr); }
+
+// output compaction of the batch after its last round, and the read-back of the point / check row offsets
+static int launch_output(r3d_engine* eng, int chunks_all) {
+    const EngineDev& d = eng->dev;
+    const int n = eng->n_scans;
+    cudaStream_t st = eng->stream;
+    {
+        Launcher l(eng, KID_OUT);
+        k_out_count<<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
+        k_out_offsets<<<1, 1024, 0, st>>>(d, n, chunks_all);
+        if (d.world) k_out_write<true><<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
+        else k_out_write<false><<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
+        r3d_count_launch(2);
+    }
+    R3D_CUDA(cudaMemcpyAsync(eng->h_offsets, eng->out_off.p, (n + 1) * sizeof(long long), cudaMemcpyDeviceToHost, st));
+    R3D_CUDA(cudaMemcpyAsync(eng->h_offsets + (d.B + 1), eng->check_off.p, (n + 1) * sizeof(long long), cudaMemcpyDeviceToHost, st));
+    eng->ran = true;
+    return R3D_OK;
+}
 
 // The default execution model: batch-wide streaming kernels for the first range image of every scan, then ONE launch
 // of the per-scan walker (r3d_k_walk.cuh) that takes every scan through all its slots and tries, then the output
@@ -832,9 +853,6 @@ static int run_walker(r3d_engine* eng) {
     cudaStream_t st = eng->stream;
     const int chunks0 = (eng->max_n0 + CHUNK - 1) / CHUNK;
     const int chunks_all = (eng->max_n0 + d.max_inserted + CHUNK - 1) / CHUNK;
-#ifndef R3D_FULL_Y
-#define R3D_FULL_Y 32
-#endif
     const int full_y = std::min(n, R3D_FULL_Y);
     const bool fresh = eng->fresh;
     eng->fresh = false;
@@ -860,8 +878,8 @@ static int run_walker(r3d_engine* eng) {
         }
     }
     if (d.task == 1) {
-        R3D_CUDA(cudaMemsetAsync(eng->occ_win.p, 0, (size_t)n * ((size_t)d.map_window * d.map_window / 32) * sizeof(unsigned), st));
-        R3D_CUDA(cudaMemsetAsync(eng->occ_cnt.p, 0, (size_t)n * (size_t)d.map_window * d.map_window * sizeof(unsigned), st));
+        R3D_CUDA(cudaMemsetAsync(d.occ_win, 0, (size_t)n * ((size_t)d.map_window * d.map_window / 32) * sizeof(unsigned), st));
+        R3D_CUDA(cudaMemsetAsync(d.occ_cnt, 0, (size_t)n * (size_t)d.map_window * d.map_window * sizeof(unsigned), st));
         Launcher l(eng, KID_ADJUST); k_adjust_map<<<dim3(chunks0, n), STREAM_THREADS, 0, st>>>(d, n, 1);
     }
     {
@@ -869,24 +887,14 @@ static int run_walker(r3d_engine* eng) {
         if (d.task == 1) walk_ss::k_scan_walk<<<n, walk_ss::WALK_THREADS, walk_ss::walk_smem_layout(d.K, d.dwords).total, st>>>(d, n);
         else walk_od::k_scan_walk<<<n, walk_od::WALK_THREADS, walk_od::walk_smem_layout(d.K, d.dwords).total, st>>>(d, n);
     }
-    {
-        Launcher l(eng, KID_OUT);
-        k_out_count<<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
-        k_out_offsets<<<1, 1024, 0, st>>>(d, n, chunks_all);
-        if (d.world) k_out_write<true><<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
-        else k_out_write<false><<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
-        r3d_count_launch(2);
-    }
-    R3D_CUDA(cudaMemcpyAsync(eng->h_offsets, eng->out_off.p, (n + 1) * sizeof(long long), cudaMemcpyDeviceToHost, st));
-    R3D_CUDA(cudaMemcpyAsync(eng->h_offsets + (d.B + 1), eng->check_off.p, (n + 1) * sizeof(long long), cudaMemcpyDeviceToHost, st));
+    TRY(launch_output(eng, chunks_all));
     R3D_CUDA(cudaMemcpyAsync(eng->h_offsets + 2 * (d.B + 1), eng->stats.p + 8, sizeof(long long), cudaMemcpyDeviceToHost, st));
-    eng->ran = true; eng->walked = true;
+    eng->walked = true;
     return r3d_check_launch("r3d_engine_run");
 }
 
 extern "C" int r3d_engine_run_until(r3d_engine* eng, int stop_at, int* still_running) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !eng->batch_loaded) return r3d_fail(R3D_ERR_ARG, "r3d_engine_run: no batch loaded");
+    if (!bind(eng) || !eng->batch_loaded) return r3d_fail(R3D_ERR_ARG, "r3d_engine_run: no batch loaded");
     if (still_running) *still_running = 0;
     if (!eng->staged) return run_walker(eng);
     eng->walked = false;
@@ -912,7 +920,7 @@ extern "C" int r3d_engine_run_until(r3d_engine* eng, int stop_at, int* still_run
         for (int i = 0; i < eng->run_nsub; ++i) {
             Sub& s = sub[i];
             s.b0 = (int)((long long)n * i / eng->run_nsub); s.n = (int)((long long)n * (i + 1) / eng->run_nsub) - s.b0;
-            s.round = 0; s.done = false; s.left = s.n; s.d = sub_view(d0, s.b0); s.st = eng->sub_stream[i];
+            s.round = 0; s.done = false; s.left = s.n; s.d = sub_view(eng, s.b0); s.st = eng->sub_stream[i];
             s.d.active_count = eng->active_count.p + (size_t)i * 128;
             s.d.host_word = eng->d_words + (size_t)i * 64;
             s.d.round_ctl = eng->round_ctl.p + (size_t)i * 32;
@@ -942,11 +950,6 @@ extern "C" int r3d_engine_run_until(r3d_engine* eng, int stop_at, int* still_run
     // the launch sequence of one round; also what a round graph is captured from
     auto launch_round = [&](const EngineDev& d, int ns, cudaStream_t ss, bool r0) {
         const size_t pref_smem = (size_t)(ns + 1) * sizeof(int);
-        // the three full re-projection kernels and close/fill walk the work lists k_update wrote (all scans in round
-        // 0, a handful later): grids sized for "some scans", not for every (chunk, scan) / (tile, scan) pair
-#ifndef R3D_FULL_Y
-#define R3D_FULL_Y 32
-#endif
         const int full_y = std::min(ns, R3D_FULL_Y);
         const int cf_grid = std::min(ns * d.cf_tiles, eng->n_sms * 8);
         { Launcher l(eng, KID_CTRL, ss); k_ctrl<<<ns, 32, 0, ss>>>(d, ns); }
@@ -1057,39 +1060,25 @@ extern "C" int r3d_engine_run_until(r3d_engine* eng, int stop_at, int* still_run
         R3D_CUDA(cudaEventRecord(eng->sub_done[i], sub[i].st));
         R3D_CUDA(cudaStreamWaitEvent(st, eng->sub_done[i], 0));
     }
-    {
-        const EngineDev& d = d0;
-        Launcher l(eng, KID_OUT);
-        k_out_count<<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
-        k_out_offsets<<<1, 1024, 0, st>>>(d, n, chunks_all);
-        if (d.world) k_out_write<true><<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
-        else k_out_write<false><<<dim3(chunks_all, n), STREAM_THREADS, 0, st>>>(d, n);
-        r3d_count_launch(2);
-    }
-    R3D_CUDA(cudaMemcpyAsync(eng->h_offsets, eng->out_off.p, (n + 1) * sizeof(long long), cudaMemcpyDeviceToHost, st));
-    R3D_CUDA(cudaMemcpyAsync(eng->h_offsets + (d0.B + 1), eng->check_off.p, (n + 1) * sizeof(long long), cudaMemcpyDeviceToHost, st));
-    eng->ran = true;
+    TRY(launch_output(eng, chunks_all));
     return r3d_check_launch("r3d_engine_run");
 }
 
 extern "C" int r3d_engine_set_sub_batches(r3d_engine* eng, int n_sub) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || n_sub < 1 || n_sub > R3D_MAX_SUB) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_sub_batches: 1..16");
+    if (!bind(eng) || n_sub < 1 || n_sub > R3D_MAX_SUB) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_sub_batches: 1..16");
     eng->n_sub = n_sub;
     return R3D_OK;
 }
 
 extern "C" int r3d_engine_sync(r3d_engine* eng) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng) return r3d_fail(R3D_ERR_ARG, "r3d_engine_sync: null engine");
+    if (!bind(eng)) return r3d_fail(R3D_ERR_ARG, "r3d_engine_sync: null engine");
     R3D_CUDA(engine_wait(eng));
     drain_events(eng);
     return R3D_OK;
 }
 
 extern "C" int r3d_engine_output_rows(r3d_engine* eng, int64_t* total_points, int64_t* total_check) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !eng->ran) return r3d_fail(R3D_ERR_ARG, "r3d_engine_output_rows: run first");
+    if (!bind(eng) || !eng->ran) return r3d_fail(R3D_ERR_ARG, "r3d_engine_output_rows: run first");
     R3D_CUDA(engine_wait(eng));
     if (total_points) *total_points = eng->h_offsets[eng->n_scans];
     if (total_check) *total_check = eng->h_offsets[eng->dev.B + 1 + eng->n_scans];
@@ -1098,8 +1087,7 @@ extern "C" int r3d_engine_output_rows(r3d_engine* eng, int64_t* total_points, in
 
 extern "C" int r3d_engine_output_device(r3d_engine* eng, const float** out_xyzi, const uint32_t** out_labels, const float** check,
                                         int64_t* out_offsets_host, int64_t* check_offsets_host) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !eng->ran) return r3d_fail(R3D_ERR_ARG, "r3d_engine_output_device: run first");
+    if (!bind(eng) || !eng->ran) return r3d_fail(R3D_ERR_ARG, "r3d_engine_output_device: run first");
     R3D_CUDA(engine_wait(eng));
     const int n = eng->n_scans;
     if (out_xyzi) *out_xyzi = reinterpret_cast<const float*>(eng->out_xyzi.p);
@@ -1112,21 +1100,19 @@ extern "C" int r3d_engine_output_device(r3d_engine* eng, const float** out_xyzi,
 
 extern "C" int r3d_engine_inserted_device(r3d_engine* eng, const int32_t** n_inserted, const int32_t** inserted,
                                           const double** inserted_box, const float** box7) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !eng->ran) return r3d_fail(R3D_ERR_ARG, "r3d_engine_inserted_device: run first");
+    if (!bind(eng) || !eng->ran) return r3d_fail(R3D_ERR_ARG, "r3d_engine_inserted_device: run first");
     const EngineDev& d = eng->dev;
     if (!eng->n_ins_dev.p) { TRY(eng->n_ins_dev.alloc(d.B)); TRY(eng->box7.alloc((size_t)d.B * d.max_events * 7)); }
-    launch_inserted_targets(eng->st.p, eng->inserted_box.p, eng->n_scans, d.max_events, eng->n_ins_dev.p, eng->box7.p, eng->stream);
+    launch_inserted_targets(eng->dev.st, eng->dev.inserted_box, eng->n_scans, d.max_events, eng->n_ins_dev.p, eng->box7.p, eng->stream);
     if (n_inserted) *n_inserted = eng->n_ins_dev.p;
-    if (inserted) *inserted = eng->inserted.p;
-    if (inserted_box) *inserted_box = eng->inserted_box.p;
+    if (inserted) *inserted = eng->dev.inserted;
+    if (inserted_box) *inserted_box = eng->dev.inserted_box;
     if (box7) *box7 = eng->box7.p;
     return r3d_check_launch("r3d_engine_inserted_device");
 }
 
 extern "C" int r3d_engine_set_world_aug(r3d_engine* eng, const r3d_world_aug* p) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_world_aug: null engine");
+    if (!bind(eng)) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_world_aug: null engine");
     if (!p) { eng->world_on = false; return R3D_OK; }
     const float v[5] = {p->flip_x_prob, p->flip_y_prob, p->rot_max, p->scale_lo, p->scale_hi};
     for (float x : v)
@@ -1143,8 +1129,7 @@ extern "C" int r3d_engine_set_world_aug(r3d_engine* eng, const r3d_world_aug* p)
 }
 
 extern "C" int r3d_engine_world_device(r3d_engine* eng, const float** params) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !params) return r3d_fail(R3D_ERR_ARG, "r3d_engine_world_device: null argument");
+    if (!bind(eng) || !params) return r3d_fail(R3D_ERR_ARG, "r3d_engine_world_device: null argument");
     if (!eng->batch_loaded || !eng->world_loaded)
         return r3d_fail(R3D_ERR_ARG, "r3d_engine_world_device: the batch was not loaded with a world augmentation");
     *params = eng->world.p;
@@ -1152,8 +1137,7 @@ extern "C" int r3d_engine_world_device(r3d_engine* eng, const float** params) {
 }
 
 extern "C" int r3d_engine_set_object_targets(r3d_engine* eng, const float* dims3, const int32_t* class_target) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !dims3 || !class_target || !eng->objects_set) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_object_targets: bad argument or no objects");
+    if (!bind(eng) || !dims3 || !class_target || !eng->objects_set) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_object_targets: bad argument or no objects");
     const EngineDev& d = eng->dev;
     for (int c = 0; c < d.n_classes; ++c)
         if (class_target[c] < 0) return r3d_fail(R3D_ERR_ARG, "r3d_engine_set_object_targets: negative class id");
@@ -1167,8 +1151,7 @@ extern "C" int r3d_engine_set_object_targets(r3d_engine* eng, const float* dims3
 extern "C" int r3d_engine_targets_device(r3d_engine* eng, const r3d_resident_store* s, const float* scene_box7,
                                          const int32_t* scene_class, int32_t max_targets, float* out_box7, int32_t* out_class,
                                          int32_t* out_count) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !s || !out_box7 || !out_class || !out_count) return r3d_fail(R3D_ERR_ARG, "r3d_engine_targets_device: null argument");
+    if (!bind(eng) || !s || !out_box7 || !out_class || !out_count) return r3d_fail(R3D_ERR_ARG, "r3d_engine_targets_device: null argument");
     if (!eng->ran) return r3d_fail(R3D_ERR_ARG, "r3d_engine_targets_device: run first");
     if (!eng->from_store) return r3d_fail(R3D_ERR_ARG, "r3d_engine_targets_device: the batch was not loaded from a resident store");
     const EngineDev& d = eng->dev;
@@ -1191,15 +1174,14 @@ extern "C" int r3d_engine_targets_device(r3d_engine* eng, const r3d_resident_sto
         if ((long long)eng->kept[i] + d.max_events - 1 > max_targets)
             return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_targets_device: max_targets below a scan's kept scene boxes + max_events - 1");
     }
-    launch_gt_targets(eng->idx_dev.p, s->box_offsets, scene_box7, scene_class, eng->st.p, eng->inserted.p, eng->inserted_box.p,
+    launch_gt_targets(eng->idx_dev.p, s->box_offsets, scene_box7, scene_class, eng->dev.st, eng->dev.inserted, eng->dev.inserted_box,
                       d.max_events, eng->obj_dims3.p, eng->class_target.p, eng->world_loaded ? eng->world.p : nullptr, eng->n_scans,
                       max_targets, out_box7, out_class, out_count, eng->stream);
     return r3d_check_launch("r3d_engine_targets_device");
 }
 
 extern "C" int r3d_engine_fetch(r3d_engine* eng, r3d_batch_result* res) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !res || !eng->ran) return r3d_fail(R3D_ERR_ARG, "r3d_engine_fetch: run first");
+    if (!bind(eng) || !res || !eng->ran) return r3d_fail(R3D_ERR_ARG, "r3d_engine_fetch: run first");
     EngineDev& d = eng->dev;
     const int n = eng->n_scans;
     cudaStream_t st = eng->stream;
@@ -1217,10 +1199,10 @@ extern "C" int r3d_engine_fetch(r3d_engine* eng, r3d_batch_result* res) {
         R3D_CUDA(cudaMemcpyAsync(res->out_labels16, eng->out_label16.p, (size_t)total * sizeof(unsigned short), cudaMemcpyDeviceToHost, st));
     }
     if (res->check_xyzil && total_check) R3D_CUDA(cudaMemcpyAsync(res->check_xyzil, eng->out_check.p, (size_t)total_check * 5 * sizeof(float), cudaMemcpyDeviceToHost, st));
-    if (res->inserted) R3D_CUDA(cudaMemcpyAsync(res->inserted, eng->inserted.p, (size_t)n * d.max_events * 4 * sizeof(int), cudaMemcpyDeviceToHost, st));
-    if (res->inserted_box) R3D_CUDA(cudaMemcpyAsync(res->inserted_box, eng->inserted_box.p, (size_t)n * d.max_events * 8 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (res->inserted) R3D_CUDA(cudaMemcpyAsync(res->inserted, eng->dev.inserted, (size_t)n * d.max_events * 4 * sizeof(int), cudaMemcpyDeviceToHost, st));
+    if (res->inserted_box) R3D_CUDA(cudaMemcpyAsync(res->inserted_box, eng->dev.inserted_box, (size_t)n * d.max_events * 8 * sizeof(double), cudaMemcpyDeviceToHost, st));
     std::vector<ScanState> hs(n);
-    R3D_CUDA(cudaMemcpyAsync(hs.data(), eng->st.p, n * sizeof(ScanState), cudaMemcpyDeviceToHost, st));
+    R3D_CUDA(cudaMemcpyAsync(hs.data(), eng->dev.st, n * sizeof(ScanState), cudaMemcpyDeviceToHost, st));
     R3D_CUDA(engine_wait(eng));
     for (int s = 0; s < n; ++s) {
         if (res->n_inserted) res->n_inserted[s] = hs[s].n_inserted;
@@ -1231,8 +1213,7 @@ extern "C" int r3d_engine_fetch(r3d_engine* eng, r3d_batch_result* res) {
 }
 
 extern "C" int r3d_engine_profile_enable(r3d_engine* eng, int on) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng) return r3d_fail(R3D_ERR_ARG, "r3d_engine_profile_enable: null engine");
+    if (!bind(eng)) return r3d_fail(R3D_ERR_ARG, "r3d_engine_profile_enable: null engine");
     cudaStreamSynchronize(eng->stream);
     drain_events(eng);
     eng->profile = on != 0;
@@ -1242,16 +1223,14 @@ extern "C" int r3d_engine_profile_enable(r3d_engine* eng, int on) {
 }
 
 extern "C" int r3d_engine_stats_ex(r3d_engine* eng, uint64_t* out, int n) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !out || n < 0 || n > R3D_N_STATS) return r3d_fail(R3D_ERR_ARG, "r3d_engine_stats_ex: bad argument");
+    if (!bind(eng) || !out || n < 0 || n > R3D_N_STATS) return r3d_fail(R3D_ERR_ARG, "r3d_engine_stats_ex: bad argument");
     R3D_CUDA(cudaStreamSynchronize(eng->stream));
     R3D_CUDA(cudaMemcpy(out, eng->stats.p, (size_t)n * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
     return R3D_OK;
 }
 
 extern "C" int r3d_engine_walk_profile(r3d_engine* eng, int64_t* cycles, int32_t* tries, int n) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !cycles || !tries || n < 0 || n > eng->dev.B) return r3d_fail(R3D_ERR_ARG, "r3d_engine_walk_profile: bad argument");
+    if (!bind(eng) || !cycles || !tries || n < 0 || n > eng->dev.B) return r3d_fail(R3D_ERR_ARG, "r3d_engine_walk_profile: bad argument");
     R3D_CUDA(cudaStreamSynchronize(eng->stream));
     std::vector<ScanState> st((size_t)n);
     R3D_CUDA(cudaMemcpy(st.data(), eng->dev.st, (size_t)n * sizeof(ScanState), cudaMemcpyDeviceToHost));
@@ -1260,20 +1239,17 @@ extern "C" int r3d_engine_walk_profile(r3d_engine* eng, int64_t* cycles, int32_t
 }
 
 extern "C" int r3d_engine_stats(r3d_engine* eng, uint64_t* out8) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !out8) return r3d_fail(R3D_ERR_ARG, "r3d_engine_stats: null argument");
+    if (!bind(eng) || !out8) return r3d_fail(R3D_ERR_ARG, "r3d_engine_stats: null argument");
     R3D_CUDA(cudaStreamSynchronize(eng->stream));
     R3D_CUDA(cudaMemcpy(out8, eng->stats.p, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
     return R3D_OK;
 }
 
-extern "C" void* r3d_engine_stream(r3d_engine* eng) {
-    if (eng) cudaSetDevice(eng->device); return eng ? (void*)eng->stream : nullptr; }
+extern "C" void* r3d_engine_stream(r3d_engine* eng) { return bind(eng) ? (void*)eng->stream : nullptr; }
 
 extern "C" int r3d_engine_profile_read(r3d_engine* eng, char* names_out, int names_cap, double* ms_out,
                                        int64_t* launches_out, int max_kernels, int* n_kernels_out) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng) return r3d_fail(R3D_ERR_ARG, "r3d_engine_profile_read: null engine");
+    if (!bind(eng)) return r3d_fail(R3D_ERR_ARG, "r3d_engine_profile_read: null engine");
     cudaStreamSynchronize(eng->stream);
     drain_events(eng);
     std::string names;
@@ -1289,21 +1265,19 @@ extern "C" int r3d_engine_profile_read(r3d_engine* eng, char* names_out, int nam
 }
 
 extern "C" int r3d_engine_debug_image(r3d_engine* eng, int scan, double* smooth_out) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || scan < 0 || scan >= eng->n_scans || !smooth_out) return r3d_fail(R3D_ERR_ARG, "r3d_engine_debug_image: bad argument");
+    if (!bind(eng) || scan < 0 || scan >= eng->n_scans || !smooth_out) return r3d_fail(R3D_ERR_ARG, "r3d_engine_debug_image: bad argument");
     R3D_CUDA(cudaStreamSynchronize(eng->stream));
-    R3D_CUDA(cudaMemcpy(smooth_out, eng->smooth.p + (size_t)scan * eng->dev.hw, (size_t)eng->dev.hw * sizeof(double), cudaMemcpyDeviceToHost));
+    R3D_CUDA(cudaMemcpy(smooth_out, eng->dev.smooth + (size_t)scan * eng->dev.hw, (size_t)eng->dev.hw * sizeof(double), cudaMemcpyDeviceToHost));
     return R3D_OK;
 }
 
 extern "C" int r3d_engine_debug_candidates(r3d_engine* eng, int scan, uint8_t* flags_out, double* level_out, int32_t* visible_out) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || scan < 0 || scan >= eng->n_scans) return r3d_fail(R3D_ERR_ARG, "r3d_engine_debug_candidates: bad argument");
+    if (!bind(eng) || scan < 0 || scan >= eng->n_scans) return r3d_fail(R3D_ERR_ARG, "r3d_engine_debug_candidates: bad argument");
     const size_t K1 = eng->dev.K + 1;
     R3D_CUDA(cudaStreamSynchronize(eng->stream));
-    if (flags_out) R3D_CUDA(cudaMemcpy(flags_out, eng->cand_flags.p + scan * K1, K1, cudaMemcpyDeviceToHost));
-    if (level_out) R3D_CUDA(cudaMemcpy(level_out, eng->cand_level.p + scan * K1, K1 * sizeof(double), cudaMemcpyDeviceToHost));
-    if (visible_out) R3D_CUDA(cudaMemcpy(visible_out, eng->cand_v.p + scan * K1, K1 * sizeof(int), cudaMemcpyDeviceToHost));
+    if (flags_out) R3D_CUDA(cudaMemcpy(flags_out, eng->dev.cand_flags + scan * K1, K1, cudaMemcpyDeviceToHost));
+    if (level_out) R3D_CUDA(cudaMemcpy(level_out, eng->dev.cand_level + scan * K1, K1 * sizeof(double), cudaMemcpyDeviceToHost));
+    if (visible_out) R3D_CUDA(cudaMemcpy(visible_out, eng->dev.cand_v + scan * K1, K1 * sizeof(int), cudaMemcpyDeviceToHost));
     return R3D_OK;
 }
 
@@ -1368,8 +1342,7 @@ __global__ void k_probe_points(EngineDev e, int scan, int obj, int n_feasible, d
 extern "C" int r3d_engine_probe_places(r3d_engine* eng, int scan, int object_id, const double* scene_rows9, int64_t n_rows,
                                        uint8_t* flags_out, double* box_out, double* xyz_out, int xyz_capacity,
                                        int32_t* n_feasible_out) {
-    if (eng) cudaSetDevice(eng->device);
-    if (!eng || !eng->batch_loaded || scan < 0 || scan >= eng->n_scans || object_id < 0 || object_id >= eng->dev.n_objects ||
+    if (!bind(eng) || !eng->batch_loaded || scan < 0 || scan >= eng->n_scans || object_id < 0 || object_id >= eng->dev.n_objects ||
         n_rows < 0 || (n_rows > 0 && !scene_rows9) || !flags_out || !box_out || !n_feasible_out)
         return r3d_fail(R3D_ERR_ARG, "r3d_engine_probe_places: bad argument");
     EngineDev d = eng->dev;
@@ -1391,14 +1364,14 @@ extern "C" int r3d_engine_probe_places(r3d_engine* eng, int scan, int object_id,
     R3D_CUDA(cudaMemcpy(n0v.data(), eng->n0_arr.p, n * sizeof(int), cudaMemcpyDeviceToHost));
     const int n0 = n0v[scan];
     const size_t tb = (size_t)scan * d.max_inserted, pb = (size_t)scan * d.P;
-    R3D_CUDA(cudaMemsetAsync(eng->alive.p + pb, 0, n0, st));
+    R3D_CUDA(cudaMemsetAsync(eng->dev.alive + pb, 0, n0, st));
     if (n_rows) {
-        R3D_CUDA(cudaMemcpyAsync(eng->tail_x.p + tb, x.data(), n_rows * sizeof(double), cudaMemcpyHostToDevice, st));
-        R3D_CUDA(cudaMemcpyAsync(eng->tail_y.p + tb, y.data(), n_rows * sizeof(double), cudaMemcpyHostToDevice, st));
-        R3D_CUDA(cudaMemcpyAsync(eng->tail_z.p + tb, z.data(), n_rows * sizeof(double), cudaMemcpyHostToDevice, st));
-        R3D_CUDA(cudaMemcpyAsync(eng->tail_i.p + tb, in.data(), n_rows * sizeof(float), cudaMemcpyHostToDevice, st));
-        R3D_CUDA(cudaMemcpyAsync(eng->label.p + pb + n0, lab.data(), n_rows * sizeof(unsigned), cudaMemcpyHostToDevice, st));
-        R3D_CUDA(cudaMemsetAsync(eng->alive.p + pb + n0, 1, n_rows, st));
+        R3D_CUDA(cudaMemcpyAsync(eng->dev.tail_x + tb, x.data(), n_rows * sizeof(double), cudaMemcpyHostToDevice, st));
+        R3D_CUDA(cudaMemcpyAsync(eng->dev.tail_y + tb, y.data(), n_rows * sizeof(double), cudaMemcpyHostToDevice, st));
+        R3D_CUDA(cudaMemcpyAsync(eng->dev.tail_z + tb, z.data(), n_rows * sizeof(double), cudaMemcpyHostToDevice, st));
+        R3D_CUDA(cudaMemcpyAsync(eng->dev.tail_i + tb, in.data(), n_rows * sizeof(float), cudaMemcpyHostToDevice, st));
+        R3D_CUDA(cudaMemcpyAsync(eng->dev.label + pb + n0, lab.data(), n_rows * sizeof(unsigned), cudaMemcpyHostToDevice, st));
+        R3D_CUDA(cudaMemsetAsync(eng->dev.alive + pb + n0, 1, n_rows, st));
     }
     k_probe_setup<<<n, 128, 0, st>>>(d, n, scan, object_id, (int)n_rows); r3d_count_launch();
     const int chunks_all = (n0 + (int)n_rows + CHUNK - 1) / CHUNK;
@@ -1412,7 +1385,7 @@ extern "C" int r3d_engine_probe_places(r3d_engine* eng, int scan, int object_id,
     k_collide<<<task_ctas, TASK_THREADS, pref_smem, st>>>(d, n, 0); r3d_count_launch();
     k_feasible_list<<<n, 128, 0, st>>>(d, n); r3d_count_launch();
     std::vector<ScanState> hs(1);
-    R3D_CUDA(cudaMemcpyAsync(hs.data(), eng->st.p + scan, sizeof(ScanState), cudaMemcpyDeviceToHost, st));
+    R3D_CUDA(cudaMemcpyAsync(hs.data(), eng->dev.st + scan, sizeof(ScanState), cudaMemcpyDeviceToHost, st));
     R3D_CUDA(cudaStreamSynchronize(st));
     const int nf = hs[0].n_feasible;
     *n_feasible_out = nf;
@@ -1426,7 +1399,7 @@ extern "C" int r3d_engine_probe_places(r3d_engine* eng, int scan, int object_id,
     const size_t nxyz = xyz_out ? (size_t)nf * hob[0].count * 3 : 0;
     if (nxyz) TRY(dxyz.alloc(nxyz));
     k_probe_points<<<148, 256, 0, st>>>(d, scan, object_id, nf, nxyz ? dxyz.p : nullptr, dbox.p); r3d_count_launch();
-    R3D_CUDA(cudaMemcpyAsync(flags_out, eng->cand_flags.p + scan * K1, K1, cudaMemcpyDeviceToHost, st));
+    R3D_CUDA(cudaMemcpyAsync(flags_out, eng->dev.cand_flags + scan * K1, K1, cudaMemcpyDeviceToHost, st));
     R3D_CUDA(cudaMemcpyAsync(box_out, dbox.p, K1 * 5 * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (nxyz) R3D_CUDA(cudaMemcpyAsync(xyz_out, dxyz.p, nxyz * sizeof(double), cudaMemcpyDeviceToHost, st));
     R3D_CUDA(cudaStreamSynchronize(st));
