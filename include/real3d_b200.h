@@ -388,7 +388,10 @@ int r3d_engine_set_schedule_policy(r3d_engine* eng, int32_t random, int32_t numb
  * on the device: class counts and, per (event, class), a uniformly random ordered head of min(max_tries, list length)
  * distinct sample indices followed by -1 (random.shuffle od/ins:400), from Philox4x32-10 keyed by (seed, epoch, store
  * index, event, class) — never by the position in the batch, so a scan's draws do not depend on how scans are batched
- * or sharded.  Input errors are reported before anything is enqueued.  The only host -> device copy is the index list;
+ * or sharded.  The draws are integer arithmetic on Philox words (and float32 steps with one rounding each for the world
+ * parameters), pinned bit for bit by the numpy restatement oracle/online_draws.py.  The device draw takes max_tries <=
+ * 4266 (its shared memory, 48 bytes per try, within 200 KiB); a larger max_tries is R3D_ERR_CAPACITY here and works on
+ * the host path.  Input errors are reported before anything is enqueued.  The only host -> device copy is the index list;
  * everything else is enqueued on the engine stream.  The OD maps are read from the store in place (keep it alive while
  * the batch is in use). */
 int r3d_engine_load_resident(r3d_engine* eng, const r3d_resident_store* store, const int32_t* indices, int32_t n,

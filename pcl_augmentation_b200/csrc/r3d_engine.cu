@@ -514,6 +514,8 @@ extern "C" int r3d_engine_set_objects(r3d_engine* eng, const r3d_object_db* db) 
         return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_set_objects: range image / yaw steps too large for the walker's shared memory");
     R3D_CUDA(cudaFuncSetAttribute(walk_od::k_scan_walk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)walk_od::walk_smem_layout(d.K, d.dwords).total));
     R3D_CUDA(cudaFuncSetAttribute(walk_ss::k_scan_walk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)walk_ss::walk_smem_layout(d.K, d.dwords).total));
+    // the device schedule draw of r3d_engine_load_resident, which refuses a larger max_tries (the host path takes any)
+    if (d.max_tries <= DRAW_MAX_TRIES) R3D_CUDA(allow_draw_schedule_smem(d.max_tries));
     eng->objects_set = true;
     return R3D_OK;
 }
@@ -720,6 +722,8 @@ extern "C" int r3d_engine_load_resident(r3d_engine* eng, const r3d_resident_stor
     if (!eng->objects_set || !eng->yaw_set) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: set objects and yaw tables first");
     if (!eng->policy_set) return r3d_fail(R3D_ERR_ARG, "r3d_engine_load_resident: set the schedule policy first");
     EngineDev& d = eng->dev;
+    if (d.max_tries > DRAW_MAX_TRIES)
+        return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_load_resident: max_tries above 4266, the most the device schedule draw takes");
     if (n <= 0 || n > d.B) return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_load_resident: n_scans exceeds max_scans");
     if (s->n_scans <= 0 || !s->xyzi || ((uintptr_t)s->xyzi & 15) || !s->labels || !s->point_offsets || !s->box_offsets ||
         !s->h_point_offsets || !s->h_box_offsets || (!s->boxes && s->h_box_offsets[s->n_scans] > 0))

@@ -314,12 +314,23 @@ void launch_gather_meta(const r3d_resident_store& s, const int* idx, int n, int 
     r3d_count_launch(2);
 }
 
+size_t draw_schedule_smem(int T) { return (size_t)DRAW_WARPS * 3 * T * sizeof(int); }
+static_assert(DRAW_WARPS * 3 * DRAW_MAX_TRIES * sizeof(int) <= 200 * 1024 && DRAW_MAX_TRIES < (1 << 16),
+              "DRAW_MAX_TRIES: the schedule draw's shared memory and its step counter word");
+
+cudaError_t allow_draw_schedule_smem(int T) {
+    cudaFuncAttributes a;
+    cudaError_t err = cudaFuncGetAttributes(&a, k_draw_schedule);
+    if (err != cudaSuccess || (size_t)a.maxDynamicSharedSizeBytes >= draw_schedule_smem(T)) return err;
+    return cudaFuncSetAttribute(k_draw_schedule, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)draw_schedule_smem(T));
+}
+
 void launch_draw_schedule(const int* idx, int n, int E, int C, int T, const int* class_list_off, const SchedulePolicy& pol,
                           unsigned long long seed, unsigned long long epoch, int* counts, int* perms, cudaStream_t st) {
     const long long warps = (long long)n * (E * C + 1);
     const int blocks = (int)((warps + DRAW_WARPS - 1) / DRAW_WARPS);
-    k_draw_schedule<<<blocks, DRAW_WARPS * 32, (size_t)DRAW_WARPS * 3 * T * sizeof(int), st>>>(idx, n, E, C, T, class_list_off, pol,
-                                                                                       seed, epoch, counts, perms);
+    k_draw_schedule<<<blocks, DRAW_WARPS * 32, draw_schedule_smem(T), st>>>(idx, n, E, C, T, class_list_off, pol, seed, epoch,
+                                                                            counts, perms);
     r3d_count_launch();
 }
 

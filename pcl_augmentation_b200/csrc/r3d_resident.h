@@ -18,6 +18,14 @@ void launch_gather_points(const r3d_resident_store& s, const int* idx, int n, in
 // max_boxes) into boxes and boxes0
 void launch_gather_meta(const r3d_resident_store& s, const int* idx, int n, int od, int* n0, int* nbox0, long long* map_off,
                         int* map_dims, double* poses, Box* boxes, Box* boxes0, int max_boxes, cudaStream_t st);
+// Dynamic shared memory of k_draw_schedule for max_tries T (three int arrays of T per warp), and the largest T the
+// device draw takes: 48 * T within 200 KiB, T <= 4266.  The bound also keeps the step j below 2^16, which the
+// (j | attempt << 16) counter word of a head draw needs.
+size_t draw_schedule_smem(int T);
+constexpr int DRAW_MAX_TRIES = 4266;
+// raises k_draw_schedule's dynamic shared memory limit on the current device to draw_schedule_smem(T) (never lowers
+// it, so engines with different max_tries can share the device); T <= DRAW_MAX_TRIES
+cudaError_t allow_draw_schedule_smem(int T);
 // counts [n][C] and perms [n][E][C][T] of the scans idx[0 .. n) for (seed, epoch)
 void launch_draw_schedule(const int* idx, int n, int E, int C, int T, const int* class_list_off, const SchedulePolicy& pol,
                           unsigned long long seed, unsigned long long epoch, int* counts, int* perms, cudaStream_t st);

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 from scipy import stats
 
+from oracle.online_draws import world_boxes, world_points
 from pcl_augmentation_b200 import _lib
 from pcl_augmentation_b200 import boxes as bx
 from pcl_augmentation_b200.engine import Real3DEngine, ScanInput, scan_input_from_case
@@ -57,28 +58,6 @@ def host_path(cases, idx, counts, perms, **kw):
 
 
 # ------------------------------------------------------------------ host restatements
-def world_points(w, xyz):
-    """r3d_world_aug on points in float32: flip, rotate, scale (numpy rounds every float32 operation)."""
-    fx, fy, _, c, s, k = (np.float32(v) for v in w[:6])
-    x, y, z = (np.asarray(xyz[:, i], dtype=np.float32) for i in range(3))
-    x1 = -x if fy else x
-    y1 = -y if fx else y
-    return np.stack([(c * x1 - s * y1) * k, (s * x1 + c * y1) * k, z * k], axis=1)
-
-
-def world_boxes(w, b7):
-    out = np.array(b7, dtype=np.float32, copy=True)
-    out[:, :3] = world_points(w, out[:, :3])
-    out[:, 3:6] *= np.float32(w[5])
-    h = out[:, 6].astype(np.float64)
-    if w[0]:
-        h = -h
-    if w[1]:
-        h = -(h + np.pi)
-    out[:, 6] = bx.wrap_pi(h + np.float64(np.float32(w[2]))).astype(np.float32)
-    return out
-
-
 def angle_diff(a, b):
     return np.abs(bx.wrap_pi(np.asarray(a, np.float64) - np.asarray(b, np.float64)))
 
