@@ -457,6 +457,12 @@ int r3d_engine_targets_device(r3d_engine* eng, const r3d_resident_store* store, 
 int r3d_engine_debug_image(r3d_engine* eng, int scan, double* smooth_out /* rows*cols */);
 int r3d_engine_debug_candidates(r3d_engine* eng, int scan, uint8_t* flags_out /* yaw_steps+1 */,
                                 double* level_out /* yaw_steps+1 */, int32_t* visible_out /* yaw_steps+1 */);
+/* The column index of one scan's original points (built by the streaming prepass): *group_out = image columns per
+ * bucket; off_out (ceil(cols / group) + 1 entries, may be NULL) = exclusive END of each bucket in idx_out; idx_out
+ * (max_points entries, may be NULL) = point indices bucket by bucket; col_out (max_points entries, may be NULL) = the
+ * azimuth bin of every point. */
+int r3d_engine_debug_col_index(r3d_engine* eng, int scan, int32_t* group_out, int32_t* off_out, int32_t* idx_out,
+                               uint16_t* col_out);
 
 #ifdef __cplusplus
 }

@@ -136,6 +136,7 @@ PROTOTYPES = {
     "r3d_engine_stream": (C.c_void_p, [C.c_void_p]),
     "r3d_engine_debug_image": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "r3d_engine_debug_candidates": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "r3d_engine_debug_col_index": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "r3d_engine_set_schedule_policy": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
     "r3d_engine_load_resident": (C.c_int, [C.c_void_p, C.POINTER(ResidentStore), C.c_void_p, C.c_int32, C.c_uint64, C.c_uint64]),
     "r3d_engine_set_ss_map_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_int64]),

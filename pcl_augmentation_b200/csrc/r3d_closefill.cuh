@@ -101,7 +101,7 @@ __device__ __forceinline__ void close_fill_tile(const In& in, int H, int W, int6
                 if (m & 2u) { neighbors += 1; sum = r3d::add(sum, s_val[sr + dr][sc]); }
                 if (m & 4u) { neighbors += 1; sum = r3d::add(sum, s_val[sr + dr][sc + 1]); }
             }
-            if (neighbors > 0) t = __ddiv_rn(sum, (double)neighbors);        // cl:57
+            if (neighbors > 0) t = r3d::mean_div(sum, neighbors);        // cl:57
             filled = true;                                                   // cl:55,58: label = 1
         }
         const int64_t idx = base + (int64_t)r * W + c;
@@ -230,7 +230,7 @@ static __device__ __forceinline__ void cf_pipelined_tiles(CfPipeSmem& sm, const 
                     if (m & 2u) { neighbors += 1; sum = r3d::add(sum, r3d::bits_dbl(sm.raw[buf][sr + dr][sc])); }
                     if (m & 4u) { neighbors += 1; sum = r3d::add(sum, r3d::bits_dbl(sm.raw[buf][sr + dr][sc + 1])); }
                 }
-                if (neighbors > 0) tv = __ddiv_rn(sum, (double)neighbors);       // cl:57
+                if (neighbors > 0) tv = r3d::mean_div(sum, neighbors);       // cl:57
             }
             out_train[base + (int64_t)r * W + c] = tv;
             far |= tv > r3d::kEmptyRange;
@@ -368,7 +368,7 @@ static __global__ void __launch_bounds__(CF_THREADS, 4) k_close_fill_tma(const _
                         if (m & 2u) { neighbors += 1; sum = r3d::add(sum, r3d::bits_dbl(s_raw[buf][sr + dr][sc + u])); }
                         if (m & 4u) { neighbors += 1; sum = r3d::add(sum, r3d::bits_dbl(s_raw[buf][sr + dr][sc + u + 1])); }
                     }
-                    if (neighbors > 0) tv[u] = __ddiv_rn(sum, (double)neighbors);    // cl:57
+                    if (neighbors > 0) tv[u] = r3d::mean_div(sum, neighbors);    // cl:57
                 }
                 far |= tv[u] > r3d::kEmptyRange;
             }

@@ -63,6 +63,24 @@ __device__ __forceinline__ int bin_col(const ImageGeom& g, double az) {
     return trunc_to_int(__ddiv_rn(az_mod(az), g.d_az));
 }
 
+// ---- mean of n = 1 .. 15 ranges (the close / fill neighbour mean, cl:57), correctly rounded like sum / n but without
+// the fp64 division: y = RN(1/n) from a table, q = RN(sum * y) is within an ulp of the quotient, the remainder
+// sum - q * n is exact in one fma, and by Markstein's theorem q + r * y rounded once is RN(sum / n).
+// (tests/test_mean_div_host.py checks it against sum / n in exact rational arithmetic.)  The table is read through the
+// L1 (__ldg) rather than the constant cache, whose reads serialise when the lanes of a warp index different entries.
+static __device__ const double kRecipSmall[16] = {0.0, 1.0, 1.0 / 2, 1.0 / 3, 1.0 / 4, 1.0 / 5, 1.0 / 6, 1.0 / 7, 1.0 / 8,
+                                                  1.0 / 9, 1.0 / 10, 1.0 / 11, 1.0 / 12, 1.0 / 13, 1.0 / 14, 1.0 / 15};
+__device__ __forceinline__ double mean_div(double sum, int n) {
+#ifdef R3D_MEAN_DDIV                                     // A/B builds only: the plain division
+    return __ddiv_rn(sum, (double)n);
+#else
+    const double y = __ldg(&kRecipSmall[n]);
+    const double q = __dmul_rn(sum, y);
+    const double r = __fma_rn(-q, (double)n, sum);
+    return __fma_rn(r, y, q);
+#endif
+}
+
 // ---- fast binning.  A bin index only needs the transcendental to ~1e-6 rad unless the point sits next to a bin edge:
 // float atan2f / acosf (CUDA: <= 3 / 2 ulp) give the position in bin units with a known error bound; if that position
 // is at least the bound away from both edges of its bin (and from both ends of the image), floor() of it IS the index

@@ -395,7 +395,7 @@ extern "C" int r3d_engine_create(const r3d_engine_cfg* cfg, r3d_engine** out) {
     TRY(per_scan(eng, d.tickets, 4)); TRY(per_scan(eng, d.feas, d.K)); TRY(per_scan(eng, d.inserted, (size_t)d.max_events * 4));
     TRY(per_scan(eng, d.inserted_box, (size_t)d.max_events * 8)); TRY(per_scan(eng, d.check, (size_t)d.max_inserted * 5));
     TRY(per_scan(eng, d.out_count, 1)); TRY(per_scan(eng, d.gcell, GG)); TRY(per_scan(eng, d.gpts, d.max_points));
-    TRY(per_scan(eng, d.gnear, GG)); TRY(per_scan(eng, d.gscratch, GG)); TRY(per_scan(eng, d.col_off, d.cols + 1));
+    TRY(per_scan(eng, d.gnear, GG)); TRY(per_scan(eng, d.gscratch, GG)); TRY(per_scan(eng, d.col_off, col_groups(d.cols) + 1));
     TRY(per_scan(eng, d.col_idx, d.max_points)); TRY(per_scan(eng, d.acell, GG)); TRY(per_scan(eng, d.apts, d.max_points));
     TRY(per_scan(eng, d.try_obj, 1)); TRY(per_scan(eng, d.chunk_cnt, d.max_chunks)); TRY(per_scan(eng, d.od_map_dims, 8));
     TRY(per_scan(eng, d.occ_far, OCC_FAR_CAP + 1));
@@ -555,7 +555,7 @@ static int arm_batch(r3d_engine* eng, bool ingest) {
     const int chunks = (eng->max_n0 + CHUNK - 1) / CHUNK;
     if (ingest) {
         R3D_CUDA(cudaMemsetAsync(d.gcell, 0, (size_t)n * d.G * d.G * sizeof(int), st));
-        R3D_CUDA(cudaMemsetAsync(d.col_off, 0, (size_t)n * (d.cols + 1) * sizeof(int), st));
+        R3D_CUDA(cudaMemsetAsync(d.col_off, 0, (size_t)n * (col_groups(d.cols) + 1) * sizeof(int), st));
         R3D_CUDA(cudaMemsetAsync(d.acell, 0, (size_t)n * d.G * d.G * sizeof(int), st));
         { Launcher l(eng, KID_INGEST); k_ingest_count<<<dim3(chunks, n), STREAM_THREADS, 0, st>>>(d, n); }
         {
@@ -1282,6 +1282,19 @@ extern "C" int r3d_engine_debug_candidates(r3d_engine* eng, int scan, uint8_t* f
     if (flags_out) R3D_CUDA(cudaMemcpy(flags_out, eng->dev.cand_flags + scan * K1, K1, cudaMemcpyDeviceToHost));
     if (level_out) R3D_CUDA(cudaMemcpy(level_out, eng->dev.cand_level + scan * K1, K1 * sizeof(double), cudaMemcpyDeviceToHost));
     if (visible_out) R3D_CUDA(cudaMemcpy(visible_out, eng->dev.cand_v + scan * K1, K1 * sizeof(int), cudaMemcpyDeviceToHost));
+    return R3D_OK;
+}
+
+extern "C" int r3d_engine_debug_col_index(r3d_engine* eng, int scan, int32_t* group_out, int32_t* off_out, int32_t* idx_out,
+                                          uint16_t* col_out) {
+    if (!bind(eng) || scan < 0 || scan >= eng->n_scans || !group_out) return r3d_fail(R3D_ERR_ARG, "r3d_engine_debug_col_index: bad argument");
+    const EngineDev& d = eng->dev;
+    const size_t ng1 = (size_t)col_groups(d.cols) + 1;
+    *group_out = COL_GROUP;
+    R3D_CUDA(cudaStreamSynchronize(eng->stream));
+    if (off_out) R3D_CUDA(cudaMemcpy(off_out, d.col_off + scan * ng1, ng1 * sizeof(int), cudaMemcpyDeviceToHost));
+    if (idx_out) R3D_CUDA(cudaMemcpy(idx_out, d.col_idx + (size_t)scan * d.max_points, (size_t)d.max_points * sizeof(int), cudaMemcpyDeviceToHost));
+    if (col_out) R3D_CUDA(cudaMemcpy(col_out, d.col + (size_t)scan * d.P, (size_t)d.max_points * sizeof(uint16_t), cudaMemcpyDeviceToHost));
     return R3D_OK;
 }
 

@@ -114,7 +114,8 @@ struct EngineDev {       // passed by value to kernels
     int* cf_tasks;                    // [B][cf_tiles]: scan * cf_tiles + tile
     int cf_tiles, cf_tiles_x;         // close/fill tiles per image, per image row of tiles
     int force_full;                   // debug / test: always take the full re-projection path
-    int *col_off, *col_idx;           // [B][cols+1], [B][max_points]: original points bucketed by azimuth bin
+    int *col_off, *col_idx;           // [B][col_groups(cols)+1], [B][max_points]: original points bucketed by groups of
+                                      // COL_GROUP adjacent azimuth bins
     // round control of ONE sub-batch.  The round number lives on the device (round_ctl[0], advanced by the last k_ctrl
     // CTA) so that the launch sequence of a round has constant arguments and can be replayed as a CUDA graph.
     int* active_count;                // [64][2] per round slot: unfinished scans, finished k_ctrl CTAs
@@ -197,6 +198,16 @@ __device__ __forceinline__ void world_point(const WorldXf& t, float& x, float& y
 }
 
 #define R3D_N_STATS 40
+#ifndef R3D_COL_GROUP
+#define R3D_COL_GROUP 8
+#endif
+// Adjacent image columns per bucket of the column index (col_off / col_idx); 1 = one bucket per column.  A warp's 32
+// consecutive points of a ring span ~25 columns but only ~4 groups of 8: fewer aggregated atomics in the two streaming
+// passes, and the index is written in runs instead of one sector per point.  The slot update visits whole groups; the
+// extra points at the two ends lie outside the masked rectangle and are never removed.
+constexpr int COL_GROUP = R3D_COL_GROUP;
+static_assert(COL_GROUP >= 1, "R3D_COL_GROUP must be positive");
+__host__ __device__ __forceinline__ int col_groups(int cols) { return (cols + COL_GROUP - 1) / COL_GROUP; }
 #ifndef R3D_OCC_G
 #define R3D_OCC_G 8
 #endif

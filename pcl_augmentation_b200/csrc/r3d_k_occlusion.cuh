@@ -132,7 +132,7 @@ __device__ bool obj_pixel_value(const unsigned long long* raw, const unsigned* d
             if (v != R3D_EMPTY_U64) { neighbors += 1; sum = add(sum, bits_dbl(v)); }
         }
     if (neighbors == 0) return false;
-    val = __ddiv_rn(sum, (double)neighbors);
+    val = mean_div(sum, neighbors);
     return true;
 }
 
@@ -187,7 +187,7 @@ __device__ __forceinline__ bool tile_pixel_value(const unsigned long long* tile,
             if (v != R3D_EMPTY_U64) { neighbors += 1; sum = add(sum, bits_dbl(v)); }
         }
     if (neighbors == 0) return false;
-    val = __ddiv_rn(sum, (double)neighbors);
+    val = mean_div(sum, neighbors);
     return true;
 }
 

@@ -4,11 +4,14 @@
 // Two passes over the float4 points instead of the seven of the first version (ingest, grid count, index count, grid
 // scatter, index scatter, min/max, projection):
 //   k_ingest_count     A1 + A2 (r, elevation, azimuth bin cached), min / max elevation of the scan, per-cell /
-//                      per-column COUNTS of the three CSR indices, z-buffer cleared on the side
+//                      per-column-group COUNTS of the three CSR indices, z-buffer cleared on the side
 //   k_bucket_scan3     exclusive scans of the three count arrays (one launch)
 //   k_scatter_project  CSR scatter of the three indices + A3 (pix ids, 64-bit atomicMin z-buffer)
-// Consecutive points of a spinning LiDAR fall into the same 0.5 m cell / image column, so the histogram atomics are
+// Consecutive points of a spinning LiDAR fall into the same 0.5 m cell / column group, so the histogram atomics are
 // aggregated per warp with __match_any_sync: one atomic per distinct key of the warp instead of one per point.
+// Timing-only ablations for tools/gpu_prepass_ab.sh (variant builds only, their outputs are wrong): R3D_ABLATE_COL_IDX
+// drops the col_idx store, R3D_ABLATE_COL_ATOMICS the column count / slot atomics (and with them the col_idx store),
+// R3D_ABLATE_GRID_STORES the two grid-entry stores.
 __device__ __forceinline__ void agg_count(int* arr, int key, bool active) {
     const unsigned act = __ballot_sync(0xffffffffu, active);
     if (!active) return;
@@ -84,7 +87,7 @@ __global__ void __launch_bounds__(STREAM_THREADS) k_ingest_count(EngineDev e, in
     const size_t base = (size_t)b * e.P;
     int* cell = e.gcell + (size_t)b * e.G * e.G;
     int* acell = e.acell + (size_t)b * e.G * e.G;
-    int* coff = e.col_off + (size_t)b * (e.cols + 1);
+    int* coff = e.col_off + (size_t)b * (col_groups(e.cols) + 1);
     unsigned long long lmin = R3D_EMPTY_U64, lmax = 0ull;
     const bool excl = grids_exclusive(e);
     const float4* __restrict__ src = e.xyzi + (size_t)b * e.max_points;
@@ -123,7 +126,9 @@ __global__ void __launch_bounds__(STREAM_THREADS) k_ingest_count(EngineDev e, in
         const bool in_g = in && (double)v.z > -3.0 && any_surface_label(e, lab);         // od/fs:154-155
         if (excl) agg_count2(acell, cell, gc, in_g ? 1 : (in_a ? 0 : -1));
         else { agg_count(acell, gc, in_a); agg_count(cell, gc, in_g); }
-        agg_count(coff, cc, in);
+#ifndef R3D_ABLATE_COL_ATOMICS
+        agg_count(coff, cc / COL_GROUP, in);
+#endif
     }
     __shared__ unsigned long long s_min[STREAM_THREADS / 32], s_max[STREAM_THREADS / 32];
     for (int o = 16; o > 0; o >>= 1) {
@@ -139,12 +144,12 @@ __global__ void __launch_bounds__(STREAM_THREADS) k_ingest_count(EngineDev e, in
     }
 }
 
-// the three exclusive scans (surface grid, all-points grid, image columns) in one launch: blockIdx.y selects the array
+// the three exclusive scans (surface grid, all-points grid, column groups) in one launch: blockIdx.y selects the array
 __global__ void __launch_bounds__(1024) k_bucket_scan3(EngineDev e, int n_scans) {
     const size_t gg = (size_t)e.G * e.G;
     if (blockIdx.y == 0) bucket_scan_body(e.gcell, gg, (int)gg, n_scans);
     else if (blockIdx.y == 1) bucket_scan_body(e.acell, gg, (int)gg, n_scans);
-    else bucket_scan_body(e.col_off, (size_t)e.cols + 1, e.cols, n_scans);
+    else bucket_scan_body(e.col_off, (size_t)col_groups(e.cols) + 1, col_groups(e.cols), n_scans);
 }
 
 __global__ void __launch_bounds__(STREAM_THREADS) k_scatter_project(EngineDev e, int n_scans) {
@@ -163,7 +168,7 @@ __global__ void __launch_bounds__(STREAM_THREADS) k_scatter_project(EngineDev e,
     const size_t base = (size_t)b * e.P;
     int* cell = e.gcell + (size_t)b * e.G * e.G;
     int* acell = e.acell + (size_t)b * e.G * e.G;
-    int* coff = e.col_off + (size_t)b * (e.cols + 1);
+    int* coff = e.col_off + (size_t)b * (col_groups(e.cols) + 1);
     float4* out = e.gpts + (size_t)b * e.max_points;
     float4* aout = e.apts + (size_t)b * e.max_points;
     int* cidx = e.col_idx + (size_t)b * e.max_points;
@@ -202,7 +207,11 @@ __global__ void __launch_bounds__(STREAM_THREADS) k_scatter_project(EngineDev e,
                 ta[u] = agg_issue(acell, gc[u], in_a);
                 tg[u] = agg_issue(cell, gc[u], in_g);
             }
-            tc[u] = agg_issue(coff, col[u], in[u]);
+#ifndef R3D_ABLATE_COL_ATOMICS
+            tc[u] = agg_issue(coff, col[u] / COL_GROUP, in[u]);
+#else
+            tc[u] = AggTicket{0u, 0};
+#endif
         }
 #pragma unroll
         for (int u = 0; u < 2; ++u) {
@@ -216,15 +225,22 @@ __global__ void __launch_bounds__(STREAM_THREADS) k_scatter_project(EngineDev e,
         }
 #pragma unroll
         for (int u = 0; u < 2; ++u) {
-            const int sa = agg_finish(ta[u]);
+            const int sa = agg_finish(ta[u]), sg = agg_finish(tg[u]);
+#ifndef R3D_ABLATE_GRID_STORES
             if (sa >= 0) {
                 if (which[u] == 1) out[sa] = make_float4(v[u].x, v[u].y, v[u].z, __uint_as_float(lab[u]));
                 else aout[sa] = make_float4(v[u].x, v[u].y, v[u].z, apt_tag(e, lab[u], p[u]));
             }
-            const int sg = agg_finish(tg[u]);
             if (sg >= 0) out[sg] = make_float4(v[u].x, v[u].y, v[u].z, __uint_as_float(lab[u]));
+#else
+            if (sa + sg == -3) cidx[0] = p[u];          // never true: keeps the grid slot atomics returning ones
+#endif
             const int sc = agg_finish(tc[u]);
+#ifndef R3D_ABLATE_COL_IDX
             if (sc >= 0) cidx[sc] = p[u];
+#else
+            if (sc == -2) cidx[0] = p[u];                // never true: keeps the slot atomic a returning one
+#endif
         }
     }
 }

@@ -10,9 +10,9 @@ __device__ __forceinline__ bool pix_removed(const EngineDev& e, int b, const Sca
 
 // Slot update, one CTA per scan (A11/A12 + the decision how the range image is refreshed):
 //  1. scene = scene[pix_id not in vis_px] (od/ins:488-501, 545).  vis_px lies inside the pixel rectangle select_emit
-//     recorded, so only the points whose azimuth bin falls in that column range are visited (CSR by column, built once
-//     per scan) plus the inserted tail: O(window) instead of O(N).  Notes whether a removed point held the scene's
-//     min / max elevation.
+//     recorded, so only the points whose azimuth bin falls in the column groups of that range are visited (CSR by
+//     COL_GROUP columns, built once per scan) plus the inserted tail: O(window) instead of O(N).  Notes whether a
+//     removed point held the scene's min / max elevation.
 //  2. full re-projection or in-place patch?  The image geometry (od/ins:97-98) depends only on the scene's min / max
 //     elevation; if neither moved, every surviving point keeps its pixel and only the pixels of vis_px change.
 //  3. patch: the z-buffer changes only at the pixels of vis_px — all their scene points were removed (od/ins:491)
@@ -42,13 +42,14 @@ __device__ __forceinline__ bool apply_vis_mask(const EngineDev& e, int b, ScanSt
     const double* T = e.poses + (size_t)b * 16;
     const size_t base = (size_t)b * e.P;
     bool extreme = false;
-    const int* off = e.col_off + (size_t)b * (e.cols + 1);
+    const int* off = e.col_off + (size_t)b * (col_groups(e.cols) + 1);
     const int* idx = e.col_idx + (size_t)b * e.max_points;
     int c0 = s.d_c0, c1 = s.d_c1;
     if (e.far_arr[b]) { c0 = 0; c1 = e.cols - 1; }          // od/ins:486 quirk: covered pixels can be anywhere
     const unsigned long long lo = s.min_el_bits, hi = s.max_el_bits;
     if (c1 >= c0) {
-        const int beg = c0 > 0 ? off[c0 - 1] : 0, end = off[c1];           // off[c] = END of column c's bucket
+        const int g0 = c0 / COL_GROUP, g1 = c1 / COL_GROUP;                 // the column groups that hold c0 .. c1
+        const int beg = g0 > 0 ? off[g0 - 1] : 0, end = off[g1];           // off[g] = END of group g's bucket
         // index -> alive / pix -> mask word is a chain of dependent loads: four points per thread in flight
         for (int i = beg + tid; i < end; i += 4 * nthr) {
             int p[4], px[4];

@@ -179,7 +179,7 @@ __device__ R3D_WALK_FN void walk_close_fill(const EngineDev& e, int b, const int
                         if (m & 2u) { neighbors += 1; sum = add(sum, bits_dbl(s_raw[sr + dr][sc])); }
                         if (m & 4u) { neighbors += 1; sum = add(sum, bits_dbl(s_raw[sr + dr][sc + 1])); }
                     }
-                    if (neighbors > 0) tv = __ddiv_rn(sum, (double)neighbors);   // cl:57
+                    if (neighbors > 0) tv = mean_div(sum, neighbors);   // cl:57
                 }
                 out[(size_t)r * W + c] = tv;
                 far |= tv > kEmptyRange;

@@ -599,6 +599,17 @@ class Real3DEngine:
                                                         vis.ctypes.data), "debug_candidates")
         return flags, level, vis
 
+    def debug_col_index(self, scan):
+        """(group, off, idx, col) of the column index of scan `scan`'s original points: bucket g holds the point indices
+        idx[off[g - 1]:off[g]] (off[-1] read as 0), col = every point's azimuth bin."""
+        group = C.c_int32(0)
+        _lib.check(self.lib.r3d_engine_debug_col_index(self.handle, scan, C.byref(group), None, None, None), "debug_col_index")
+        off = np.zeros(-(-self.cols // group.value) + 1, np.int32)
+        idx, col = np.zeros(self.max_points, np.int32), np.zeros(self.max_points, np.uint16)
+        _lib.check(self.lib.r3d_engine_debug_col_index(self.handle, scan, C.byref(group), off.ctypes.data, idx.ctypes.data,
+                                                       col.ctypes.data), "debug_col_index")
+        return group.value, off, idx, col
+
     def close(self):
         if getattr(self, 'handle', None):
             self.lib.r3d_engine_destroy(self.handle)
