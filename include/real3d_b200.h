@@ -452,6 +452,25 @@ int r3d_engine_set_object_targets(r3d_engine* eng, const float* dims3, const int
 int r3d_engine_targets_device(r3d_engine* eng, const r3d_resident_store* store, const float* scene_box7,
                               const int32_t* scene_class, int32_t max_targets, float* out_box7, int32_t* out_class,
                               int32_t* out_count);
+/* Points of the augmented clouds in their detection targets, on the target buffers box7 / cls / count (DEVICE,
+ * [n][max_targets][7], [n][max_targets], [n]) that r3d_engine_targets_device filled for the last run, and on the
+ * engine's output rows (r3d_engine_output_device), so the test sees the frame and values a trainer gets, world
+ * transform included.  A point (x, y, z) is inside a box (cx, cy, cz, dx, dy, dz, h) iff |z - cz| <= dz / 2,
+ * |lx| < dx / 2 and |ly| < dy / 2, with c = cos h, s = sin h, u = x - cx, v = y - cy, lx = c u + s v, ly = -s u + c v
+ * (OpenPCDet's points_in_boxes: z from the centre, the z bound closed, the xy bounds open), evaluated in fp64 on the
+ * float32 values; a float pre-test only culls boxes the point is provably outside of.
+ *   out_points [n][max_targets] (DEVICE): output rows of the scan inside each target (a point inside two boxes counts
+ *     in both); zero past count.
+ *   out_point_gt (DEVICE, one per output row): the index of the first target of the row's scan that contains it, or -1.
+ *   min_points >= 0: afterwards every target with fewer points is dropped, scene and inserted alike; the kept rows of
+ *     box7 / cls / out_points move down in order, count shrinks, rows past it are zero, and out_point_gt refers to the
+ *     kept rows (a point in a dropped box takes the next kept box that contains it).  0 drops nothing.
+ * Enqueued on the engine stream; no host synchronisation.  Errors, reported before anything is enqueued: a null
+ * pointer, no run yet, a batch not loaded by r3d_engine_load_resident, a semseg engine, min_points < 0,
+ * max_targets < 1, no r3d_engine_targets_device since the batch was loaded, or more than 2048 possible targets in a scan
+ * (R3D_ERR_CAPACITY). */
+int r3d_engine_target_points_device(r3d_engine* eng, int32_t max_targets, float* box7, int32_t* cls, int32_t* count,
+                                    int32_t min_points, int32_t* out_points, int32_t* out_point_gt);
 
 /* debug / parity taps on the resident state of one scan (device -> host), used by the tests */
 int r3d_engine_debug_image(r3d_engine* eng, int scan, double* smooth_out /* rows*cols */);

@@ -148,6 +148,8 @@ PROTOTYPES = {
     "r3d_engine_set_object_targets": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "r3d_engine_targets_device": (C.c_int, [C.c_void_p, C.POINTER(ResidentStore), C.c_void_p, C.c_void_p, C.c_int32,
                                             C.c_void_p, C.c_void_p, C.c_void_p]),
+    "r3d_engine_target_points_device": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                                  C.c_void_p, C.c_void_p]),
 }
 
 _lib = None

@@ -129,6 +129,10 @@ struct r3d_engine {
     DevBuf<int> class_target;
     const int* kept_src = nullptr;
     std::vector<int> kept;
+    // most targets a scan of the loaded batch can have (kept scene boxes + max_events), set by the batch's
+    // r3d_engine_targets_device (0: not yet), and the [B][cap + 1] remap scratch of r3d_engine_target_points_device
+    int targets_bound = 0;
+    DevBuf<int> tp_remap;
     // profiling
     bool profile = false;
     double prof_ms[KID_COUNT] = {0};
@@ -769,6 +773,7 @@ extern "C" int r3d_engine_load_resident(r3d_engine* eng, const r3d_resident_stor
     d.world = eng->world_on ? eng->world.p : nullptr;
     eng->world_loaded = eng->world_on;
     eng->from_store = true;
+    eng->targets_bound = 0;
     eng->batch_idx.assign(indices, indices + n);
     TRY(r3d_check_launch("r3d_engine_load_resident"));
     eng->batch_loaded = true;
@@ -1173,15 +1178,40 @@ extern "C" int r3d_engine_targets_device(r3d_engine* eng, const r3d_resident_sto
             for (int j = s->h_box_offsets[i]; j < s->h_box_offsets[i + 1]; ++j) eng->kept[i] += cls[j] != 0;
         eng->kept_src = scene_class;
     }
+    int bound = 0;
     for (int i : eng->batch_idx) {
         if (i < 0 || i >= s->n_scans) return r3d_fail(R3D_ERR_ARG, "r3d_engine_targets_device: batch index outside this store");
         if ((long long)eng->kept[i] + d.max_events - 1 > max_targets)
             return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_targets_device: max_targets below a scan's kept scene boxes + max_events - 1");
+        bound = std::max(bound, eng->kept[i] + d.max_events);
     }
+    eng->targets_bound = bound;
     launch_gt_targets(eng->idx_dev.p, s->box_offsets, scene_box7, scene_class, eng->dev.st, eng->dev.inserted, eng->dev.inserted_box,
                       d.max_events, eng->obj_dims3.p, eng->class_target.p, eng->world_loaded ? eng->world.p : nullptr, eng->n_scans,
                       max_targets, out_box7, out_class, out_count, eng->stream);
     return r3d_check_launch("r3d_engine_targets_device");
+}
+
+extern "C" int r3d_engine_target_points_device(r3d_engine* eng, int32_t max_targets, float* box7, int32_t* cls, int32_t* count,
+                                               int32_t min_points, int32_t* out_points, int32_t* out_point_gt) {
+    if (!bind(eng) || !box7 || !cls || !count || !out_points || !out_point_gt)
+        return r3d_fail(R3D_ERR_ARG, "r3d_engine_target_points_device: null argument");
+    if (!eng->ran) return r3d_fail(R3D_ERR_ARG, "r3d_engine_target_points_device: run first");
+    if (!eng->from_store)
+        return r3d_fail(R3D_ERR_ARG, "r3d_engine_target_points_device: the batch was not loaded from a resident store");
+    const EngineDev& d = eng->dev;
+    if (d.task != 0) return r3d_fail(R3D_ERR_ARG, "r3d_engine_target_points_device: detection targets need an object detection engine");
+    if (min_points < 0) return r3d_fail(R3D_ERR_ARG, "r3d_engine_target_points_device: min_points < 0");
+    if (max_targets < 1) return r3d_fail(R3D_ERR_ARG, "r3d_engine_target_points_device: max_targets < 1");
+    if (eng->targets_bound == 0)
+        return r3d_fail(R3D_ERR_ARG, "r3d_engine_target_points_device: no r3d_engine_targets_device for this batch");
+    const int cap = std::min(max_targets, eng->targets_bound);
+    if (cap > TARGET_POINTS_MAX_BOXES)
+        return r3d_fail(R3D_ERR_CAPACITY, "r3d_engine_target_points_device: more than 2048 targets in a scan");
+    if (min_points > 0 && (size_t)d.B * (cap + 1) > eng->tp_remap.n) TRY(eng->tp_remap.alloc((size_t)d.B * (cap + 1)));
+    R3D_CUDA(launch_target_points(eng->out_xyzi.p, eng->out_off.p, eng->n_scans, eng->max_n0 + d.max_inserted, box7, cls, count,
+                                  max_targets, cap, min_points, out_points, out_point_gt, eng->tp_remap.p, eng->stream));
+    return r3d_check_launch("r3d_engine_target_points_device");
 }
 
 extern "C" int r3d_engine_fetch(r3d_engine* eng, r3d_batch_result* res) {

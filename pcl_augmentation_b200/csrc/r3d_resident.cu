@@ -9,6 +9,8 @@ namespace r3d {
 constexpr int GATHER_CHUNK = 4096;       // points per CTA: the (chunk, scan) grid of k_widen_labels
 constexpr int GATHER_THREADS = 256;
 constexpr int DRAW_WARPS = 4;            // warps per CTA of k_draw_schedule
+constexpr int TP_THREADS = 256;          // k_target_points / k_target_remap: CTA of 8 warps ...
+constexpr int TP_CHUNK = 8192;           // ... over TP_CHUNK output rows of one scan
 
 // ------------------------------------------------------------------------------------------------ gathers
 // A pure copy: per point one 16-byte load + store of xyzi and a 2-byte label read widened to the engine's u32 row.
@@ -294,6 +296,171 @@ __global__ void k_gt_targets(const int* __restrict__ idx, const int* __restrict_
     if (lane == 0) out_count[b] = m;
 }
 
+// ------------------------------------------------------------------------------------------ points in targets
+// OpenPCDet's points_in_boxes test in fp64 on the float32 point and box: |z - cz| <= dz / 2, |lx| < dx / 2 and
+// |ly| < dy / 2 with (lx, ly) = (c u + s v, -s u + c v), u = x - cx, v = y - cy, c = cos h, s = sin h.  Every operation
+// is rounded on its own (no contraction), in the order of oracle/target_points.py.
+__device__ __forceinline__ bool point_in_target(float x, float y, float z, float cx, float cy, float cz, float dx, float dy,
+                                                float dz, double c, double s) {
+    if (!(fabs(__dsub_rn((double)z, (double)cz)) <= __dmul_rn((double)dz, 0.5))) return false;
+    const double u = __dsub_rn((double)x, (double)cx), v = __dsub_rn((double)y, (double)cy);
+    const double lx = __dadd_rn(__dmul_rn(c, u), __dmul_rn(s, v));
+    const double ly = __dadd_rn(-__dmul_rn(s, u), __dmul_rn(c, v));
+    return fabs(lx) < __dmul_rn((double)dx, 0.5) && fabs(ly) < __dmul_rn((double)dy, 0.5);
+}
+
+// Shared memory of k_target_points per box slot: c, s (fp64), the float box centre / sizes, the six float bounds of
+// the pre-test and the counter.
+constexpr int TP_BOX_BYTES = 2 * 8 + 6 * 4 + 6 * 4 + 4;
+size_t target_points_smem(int cap) { return (size_t)cap * TP_BOX_BYTES; }
+
+// One CTA per (TP_CHUNK output rows, scan): every warp takes 32 consecutive rows at a time, which are ring neighbours
+// of the scan, reduces their x / y / z extent and tests it against the pre-test bounds of every box (lane k takes
+// boxes k, k + 32, ...).  Only the boxes that survive get the exact test on all 32 rows, in target order, so the first
+// hit of a row is its point_gt.  Pre-test bounds: the box's circumscribed square in xy and its z slab, widened by
+// 2^-20 (|centre| + half extent) + 2^-30 and rounded outwards; the fp64 expression errs by less than 2^-50 of those
+// magnitudes, so a culled box never contains the point by the exact test.  Counts go to shared counters, then one
+// global atomic per (CTA, box) into points (zeroed before the launch).
+__global__ void __launch_bounds__(TP_THREADS) k_target_points(const float4* __restrict__ xyzi, const long long* __restrict__ out_off,
+                                                              const float* __restrict__ box7, const int* __restrict__ count,
+                                                              int max_targets, int cap, int* points, int* point_gt) {
+    extern __shared__ double s_tp[];
+    double* sc = s_tp;
+    double* ss = sc + cap;
+    float* f = reinterpret_cast<float*>(ss + cap);     // cx cy cz dx dy dz | xlo xhi ylo yhi zlo zhi, each [cap]
+    int* cnt = reinterpret_cast<int*>(f + 12 * cap);
+    const int b = blockIdx.y;
+    const long long r_beg = out_off[b], r_end = out_off[b + 1];
+    const long long c0 = r_beg + (long long)blockIdx.x * TP_CHUNK;
+    if (c0 >= r_end) return;
+    const int m = min(count[b], cap);
+    const float* bx = box7 + (size_t)b * max_targets * 7;
+    for (int j = threadIdx.x; j < m; j += TP_THREADS) {
+        const float* q = bx + (size_t)j * 7;
+        const float cx = q[0], cy = q[1], cz = q[2], dx = q[3], dy = q[4], dz = q[5];
+        sc[j] = cos((double)q[6]); ss[j] = sin((double)q[6]);
+        f[j] = cx; f[cap + j] = cy; f[2 * cap + j] = cz; f[3 * cap + j] = dx; f[4 * cap + j] = dy; f[5 * cap + j] = dz;
+        const float hx = dx * 0.5f, hy = dy * 0.5f, hz = dz * 0.5f;
+        const float R = __fsqrt_ru(__fadd_ru(__fmul_ru(hx, hx), __fmul_ru(hy, hy)));
+        const float px = __fadd_ru(__fmul_ru(__fadd_ru(fabsf(cx), R), 0x1p-20f), 0x1p-30f);
+        const float py = __fadd_ru(__fmul_ru(__fadd_ru(fabsf(cy), R), 0x1p-20f), 0x1p-30f);
+        const float pz = __fadd_ru(__fmul_ru(__fadd_ru(fabsf(cz), fabsf(hz)), 0x1p-20f), 0x1p-30f);
+        f[6 * cap + j] = __fsub_rd(__fsub_rd(cx, R), px);  f[7 * cap + j] = __fadd_ru(__fadd_ru(cx, R), px);
+        f[8 * cap + j] = __fsub_rd(__fsub_rd(cy, R), py);  f[9 * cap + j] = __fadd_ru(__fadd_ru(cy, R), py);
+        f[10 * cap + j] = __fsub_rd(__fsub_rd(cz, hz), pz); f[11 * cap + j] = __fadd_ru(__fadd_ru(cz, hz), pz);
+        cnt[j] = 0;
+    }
+    __syncthreads();
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    constexpr int SLICE = TP_CHUNK / (TP_THREADS / 32);
+    const long long q0 = c0 + (long long)w * SLICE, q1 = min(q0 + SLICE, min(c0 + TP_CHUNK, r_end));
+    for (long long q = q0; q < q1; q += 32) {
+        const long long r = q + lane;
+        const bool live = r < q1;
+        float4 p = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (live) p = __ldcs(xyzi + r);
+        float xl = live ? p.x : INFINITY, xh = live ? p.x : -INFINITY, yl = live ? p.y : INFINITY, yh = live ? p.y : -INFINITY;
+        float zl = live ? p.z : INFINITY, zh = live ? p.z : -INFINITY;
+        for (int o = 16; o > 0; o >>= 1) {
+            xl = fminf(xl, __shfl_xor_sync(0xffffffffu, xl, o)); xh = fmaxf(xh, __shfl_xor_sync(0xffffffffu, xh, o));
+            yl = fminf(yl, __shfl_xor_sync(0xffffffffu, yl, o)); yh = fmaxf(yh, __shfl_xor_sync(0xffffffffu, yh, o));
+            zl = fminf(zl, __shfl_xor_sync(0xffffffffu, zl, o)); zh = fmaxf(zh, __shfl_xor_sync(0xffffffffu, zh, o));
+        }
+        int first = -1;
+        for (int j0 = 0; j0 < m; j0 += 32) {
+            const int j = j0 + lane;
+            const bool cand = j < m && !(xl > f[7 * cap + j] || xh < f[6 * cap + j] || yl > f[9 * cap + j] ||
+                                         yh < f[8 * cap + j] || zl > f[11 * cap + j] || zh < f[10 * cap + j]);
+            for (unsigned bits = __ballot_sync(0xffffffffu, cand); bits; bits &= bits - 1u) {
+                const int k = j0 + __ffs(bits) - 1;
+                const bool in = live && point_in_target(p.x, p.y, p.z, f[k], f[cap + k], f[2 * cap + k], f[3 * cap + k],
+                                                        f[4 * cap + k], f[5 * cap + k], sc[k], ss[k]);
+                const unsigned hits = __ballot_sync(0xffffffffu, in);
+                if (lane == 0 && hits) atomicAdd(cnt + k, __popc(hits));
+                if (in && first < 0) first = k;
+            }
+        }
+        if (live) __stcs(point_gt + r, first);
+    }
+    __syncthreads();
+    for (int j = threadIdx.x; j < m; j += TP_THREADS)
+        if (cnt[j]) atomicAdd(points + (size_t)b * max_targets + j, cnt[j]);
+}
+
+// One warp per scan drops the targets with fewer than min_points points: the kept rows of box7 / class / points move
+// down in order (ballots, as k_gt_targets), the freed rows become zero and count shrinks.  remap[b][j] is the new
+// index of a kept target j, and -1 - (new index of the first kept target after j) for a dropped one; remap[b][cap] is
+// the first dropped target (-1: none, point_gt stays as it is).
+__global__ void k_target_filter(float* box7, int* cls, int* count, int* points, int n, int max_targets, int cap, int min_points,
+                                int* remap) {
+    const int b = (int)((blockIdx.x * (size_t)blockDim.x + threadIdx.x) >> 5);
+    const int lane = threadIdx.x & 31;
+    if (b >= n) return;                                       // whole warps: n * 32 threads of whole CTAs
+    const int m = min(count[b], cap);
+    float* ob = box7 + (size_t)b * max_targets * 7;
+    int* oc = cls + (size_t)b * max_targets;
+    int* op = points + (size_t)b * max_targets;
+    const unsigned below = (1u << lane) - 1u;
+    int* rb = remap + (size_t)b * (cap + 1);
+    int kept = 0, first_drop = -1;
+    for (int j0 = 0; j0 < m; j0 += 32) {
+        const int j = j0 + lane;
+        float o[7] = {};
+        int c = 0, pts = 0;
+        if (j < m) {
+            for (int q = 0; q < 7; ++q) o[q] = ob[(size_t)j * 7 + q];
+            c = oc[j]; pts = op[j];
+        }
+        const bool keep = j < m && pts >= min_points;
+        const unsigned km = __ballot_sync(0xffffffffu, keep);
+        const unsigned dm = __ballot_sync(0xffffffffu, j < m && !keep);
+        if (first_drop < 0 && dm) first_drop = j0 + __ffs(dm) - 1;
+        __syncwarp();                                         // every row of this group is read before any is moved
+        const int pos = kept + __popc(km & below);
+        if (keep) {
+            for (int q = 0; q < 7; ++q) ob[(size_t)pos * 7 + q] = o[q];
+            oc[pos] = c; op[pos] = pts;
+        }
+        if (j < m) rb[j] = keep ? pos : -1 - pos;
+        kept += __popc(km);
+        __syncwarp();
+    }
+    for (int p = kept + lane; p < m; p += 32) {
+        for (int q = 0; q < 7; ++q) ob[(size_t)p * 7 + q] = 0.f;
+        oc[p] = 0; op[p] = 0;
+    }
+    if (lane == 0) { count[b] = kept; rb[cap] = first_drop; }
+}
+
+// point_gt after k_target_filter, for the scans that dropped a target: a row in a target before the first dropped one
+// keeps its index, a row in a later kept target takes its new index, and a row in a dropped target is tested again
+// against the kept targets after it, in order (rare: a dropped target holds fewer than min_points rows).
+__global__ void __launch_bounds__(TP_THREADS) k_target_remap(const float4* __restrict__ xyzi, const long long* __restrict__ out_off,
+                                                             const float* __restrict__ box7, const int* __restrict__ count,
+                                                             int max_targets, int cap, const int* __restrict__ remap, int* point_gt) {
+    const int b = blockIdx.y;
+    const int* rb = remap + (size_t)b * (cap + 1);
+    const int first_drop = rb[cap];
+    if (first_drop < 0) return;
+    const long long c0 = out_off[b] + (long long)blockIdx.x * TP_CHUNK, r_end = min(c0 + TP_CHUNK, out_off[b + 1]);
+    const float* bx = box7 + (size_t)b * max_targets * 7;
+    const int m = count[b];
+    for (long long r = c0 + threadIdx.x; r < r_end; r += TP_THREADS) {
+        const int g = point_gt[r];
+        if (g < first_drop) continue;
+        int v = rb[g];
+        if (v < 0) {
+            const float4 p = xyzi[r];
+            int k = -1 - v;
+            for (v = -1; k < m && v < 0; ++k) {
+                const float* q = bx + (size_t)k * 7;
+                if (point_in_target(p.x, p.y, p.z, q[0], q[1], q[2], q[3], q[4], q[5], cos((double)q[6]), sin((double)q[6]))) v = k;
+            }
+        }
+        point_gt[r] = v;
+    }
+}
+
 // ------------------------------------------------------------------------------------------------ launchers
 void launch_gather_points(const r3d_resident_store& s, const int* idx, int n, int max_n0, float4* xyzi, int max_points,
                           unsigned* label, int P, int od, unsigned road_label, cudaStream_t st) {
@@ -355,6 +522,27 @@ void launch_gt_targets(const int* idx, const int* box_off, const float* scene_bo
                                                                   E, dims3, class_target, world, n, max_targets, out_box7,
                                                                   out_class, out_count);
     r3d_count_launch();
+}
+
+cudaError_t launch_target_points(const float4* xyzi, const long long* out_off, int n, int max_rows, float* box7, int* cls,
+                                 int* count, int max_targets, int cap, int min_points, int* points, int* point_gt, int* remap,
+                                 cudaStream_t st) {
+    const size_t smem = target_points_smem(cap);
+    cudaError_t err = cudaFuncSetAttribute(k_target_points, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (err != cudaSuccess) return err;
+    err = cudaMemsetAsync(points, 0, (size_t)n * max_targets * sizeof(int), st);
+    if (err != cudaSuccess) return err;
+    const dim3 grid((max_rows + TP_CHUNK - 1) / TP_CHUNK, n);
+    k_target_points<<<grid, TP_THREADS, smem, st>>>(xyzi, out_off, box7, count, max_targets, cap, points, point_gt);
+    r3d_count_launch();
+    if (min_points > 0) {
+        constexpr int WARPS = 4;
+        k_target_filter<<<(n + WARPS - 1) / WARPS, WARPS * 32, 0, st>>>(box7, cls, count, points, n, max_targets, cap, min_points,
+                                                                        remap);
+        k_target_remap<<<grid, TP_THREADS, 0, st>>>(xyzi, out_off, box7, count, max_targets, cap, remap, point_gt);
+        r3d_count_launch(2);
+    }
+    return cudaSuccess;
 }
 
 }  // namespace r3d

@@ -40,5 +40,14 @@ void launch_gt_targets(const int* idx, const int* box_off, const float* scene_bo
                        const int* inserted, const double* inserted_box, int E, const float* dims3, const int* class_target,
                        const float* world, int n, int max_targets, float* out_box7, int* out_class, int* out_count,
                        cudaStream_t st);
+// Points of the output rows xyzi (scan b: rows out_off[b] .. out_off[b + 1], at most max_rows) inside the first
+// min(count[b], cap) targets of box7 / cls / count (r3d_engine_target_points_device): points [n][max_targets] and
+// point_gt per row; with min_points > 0 the targets below it are dropped in place and point_gt refers to the kept ones.
+// remap: [n][cap + 1] scratch.  Dynamic shared memory: target_points_smem(cap), cap <= TARGET_POINTS_MAX_BOXES.
+constexpr int TARGET_POINTS_MAX_BOXES = 2048;
+size_t target_points_smem(int cap);
+cudaError_t launch_target_points(const float4* xyzi, const long long* out_off, int n, int max_rows, float* box7, int* cls,
+                                 int* count, int max_targets, int cap, int min_points, int* points, int* point_gt, int* remap,
+                                 cudaStream_t st);
 
 }  // namespace r3d

@@ -477,6 +477,21 @@ class Real3DEngine:
         _lib.check(self.lib.r3d_engine_targets_device(self.handle, C.byref(store.abi), ptr(box7), ptr(cls), m,
                                                       gb.data_ptr(), gc.data_ptr(), ng.data_ptr()), "targets_device")
 
+    def target_points_device(self, out, min_points, point_gt):
+        """Enqueue on the engine stream, for the targets ``targets_device`` wrote into ``out`` for the last run:
+        ``out['gt_points']`` (int32 [>= n, max_targets]) = output rows of the scan inside each target, and ``point_gt``
+        (int32 CUDA tensor with one entry per output row at least) = index of the first target of the row's scan that
+        contains the row, or -1 (inside test: include/real3d_b200.h, ``oracle.target_points``).  Targets
+        with fewer than ``min_points`` points are then dropped from ``out`` in place, order kept, and ``point_gt``
+        refers to the kept rows; 0 drops nothing."""
+        gb, gc, ng, gp = out['gt_boxes'], out['gt_classes'], out['n_gt'], out['gt_points']
+        m = int(gb.shape[1])
+        assert all(t.is_contiguous() for t in (gb, gc, ng, gp, point_gt))
+        assert tuple(gp.shape[1:]) == (m,) and gp.shape[0] >= self._n_scans
+        _lib.check(self.lib.r3d_engine_target_points_device(self.handle, m, gb.data_ptr(), gc.data_ptr(), ng.data_ptr(),
+                                                            int(min_points), gp.data_ptr(), point_gt.data_ptr()),
+                   "target_points_device")
+
     def unpack(self, buffers, raise_on_error=True):
         """Per-scan output records in the reference's formats."""
         out = []

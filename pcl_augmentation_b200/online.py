@@ -238,6 +238,10 @@ class AugmentedBatch:
     gt_classes: object = None # int32 [n, max_targets]: 1-based into target_classes, 0 = padding
     n_gt: object = None       # int32 [n]
     world: object = None      # float32 [n, 8]: with world_aug, (fx, fy, theta, c, s, k, 0, 0) of each scan
+    # with target_points: output rows inside each target of gt_boxes, and per row the first target of its scan that
+    # contains it (-1: none); targets with fewer than target_points points are already dropped from gt_*
+    gt_points: object = None  # int32 [n, max_targets]; zero past n_gt
+    point_gt: object = None   # int32 [total]: index into gt_boxes[s] of the row's scan s, or -1
 
 
 class OnlineAugmenter:
@@ -245,9 +249,16 @@ class OnlineAugmenter:
     batch k + 1 is augmented while the consumer still works on batch k."""
 
     def __init__(self, task, config, db, dataset, *, batch_size, seed, yaw_steps=360, depth=2, rank=0, world=1,
-                 target_classes=None, world_aug=None, **engine_kwargs):
+                 target_classes=None, world_aug=None, target_points=None, **engine_kwargs):
         """``target_classes`` (object detection): the class names of ``gt_boxes`` / ``gt_classes``; every insertion
-        class must be one of them.  ``world_aug``: a ``WorldAug`` applied to every batch (None: off)."""
+        class must be one of them.  ``world_aug``: a ``WorldAug`` applied to every batch (None: off).
+        ``target_points`` (needs ``target_classes``): None (off) or min_points K >= 0: every batch also gets
+        ``gt_points`` / ``point_gt`` on the augmented cloud, and targets with fewer than K points are dropped."""
+        if target_points is not None:
+            if target_classes is None:
+                raise ValueError("target_points needs target_classes")
+            if isinstance(target_points, bool) or int(target_points) != target_points or target_points < 0:
+                raise ValueError(f"target_points must be None or an integer >= 0, got {target_points!r}")
         torch = _lib.require_cuda()
         from .dataset_driver import _objects_per_frame
         assert dataset.task == task and depth >= 1
@@ -281,6 +292,12 @@ class OnlineAugmenter:
                 self._targets.append({'gt_boxes': torch.zeros((self.batch_size, self.max_targets, 7), dtype=torch.float32, device=dev),
                                       'gt_classes': torch.zeros((self.batch_size, self.max_targets), dtype=torch.int32, device=dev),
                                       'n_gt': torch.zeros(self.batch_size, dtype=torch.int32, device=dev)})
+        self.target_points = None if target_points is None else int(target_points)
+        if self.target_points is not None:
+            rows = self.batch_size * (self.engines[0].max_points + self.engines[0].max_inserted + 16)   # output capacity
+            for tg in self._targets:
+                tg['gt_points'] = torch.zeros((self.batch_size, self.max_targets), dtype=torch.int32, device=dev)
+                tg['point_gt'] = torch.zeros(rows, dtype=torch.int32, device=dev)
 
     def _submit(self, indices, epoch):
         torch = self._torch
@@ -317,6 +334,9 @@ class OnlineAugmenter:
             eng.targets_device(self.dataset, tg)
             n = len(idx)
             extra.update(gt_boxes=tg['gt_boxes'][:n], gt_classes=tg['gt_classes'][:n], n_gt=tg['n_gt'][:n])
+            if self.target_points is not None:
+                eng.target_points_device(tg, self.target_points, tg['point_gt'])
+                extra.update(gt_points=tg['gt_points'][:n], point_gt=tg['point_gt'][:int(out['offsets'][n])])
         if self.world_aug is not None:
             extra['world'] = eng.world_device()
         ready = torch.cuda.Event()

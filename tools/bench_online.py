@@ -7,6 +7,7 @@ intensities are redrawn (2.2 GB of points + labels: larger than L2, so the gathe
     python tools/bench_online.py [--batches 20] [--warmup 2] [--depth 3] [--out DIR]            rates
     python tools/bench_online.py --profile [--out DIR]                                           kernel times + copies
     python tools/bench_online.py --targets [--world-aug] [--rounds 3] [--out DIR]                 variants A/B
+    python tools/bench_online.py --targets --target-points K [--rounds 3] [--out DIR]            points in targets A/B
 
 Rates (scans/s, host clock around work that ends in a device synchronise):
   * online     OnlineAugmenter.epochs over the store, a new epoch each pass (gather + device schedule draw + run), and
@@ -18,6 +19,11 @@ bytes per second against a device-to-device copy measured in the same run, and e
 --targets / --world-aug: the online rate of plain batches, of batches with detection targets (targets_device) and, with
 --world-aug, of batches with targets and world augmentation, alternating the variants round by round on the same
 engines; with --profile, the kernel times of a plain epoch and of an epoch with the variant's options, in one process.
+--target-points K: the targets-only rate against targets + points in targets with min_points K (OnlineAugmenter
+target_points), alternating round by round; then the device time of the new kernels per batch, the streaming kernel's
+algorithmic bytes (16 B read + 4 B written per output row) over its time against the copy peak of the same run, and on
+one epoch of the store without the filter, the fraction of scene targets whose point count went down, reached 0 or
+fell below K compared with the same box on the raw store scan.
 """
 from __future__ import annotations
 
@@ -48,7 +54,7 @@ def card():
 TARGETS = ["Car", "Pedestrian", "Cyclist"]
 
 
-def setup(depth, targets=False, world_aug=None):
+def setup(depth, targets=False, world_aug=None, target_points=None):
     import bench
     from pcl_augmentation_b200.engine import scan_input_from_case
     from pcl_augmentation_b200.online import OnlineAugmenter, ResidentDataset
@@ -66,13 +72,14 @@ def setup(depth, targets=False, world_aug=None):
     kw.pop("max_scans"), kw.pop("map_data")
     c0 = base[0]
     aug = OnlineAugmenter("od", c0.config, c0.db, store, batch_size=BATCH, seed=2024, depth=depth,
-                          target_classes=TARGETS if targets else None, world_aug=world_aug, **kw)
+                          target_classes=TARGETS if targets else None, world_aug=world_aug, target_points=target_points, **kw)
     return aug, store, scans
 
 
-def set_variant(aug, targets, world_aug):
+def set_variant(aug, targets, world_aug, target_points=None):
     """Switch an augmenter built with targets between the variants (its target buffers stay allocated)."""
     aug.target_classes = TARGETS if targets else None
+    aug.target_points = target_points
     aug.world_aug = world_aug
     for e in aug.engines:
         e.set_world_aug(world_aug)
@@ -81,23 +88,25 @@ def set_variant(aug, targets, world_aug):
 def variants(args):
     import torch
     from pcl_augmentation_b200.online import WorldAug
-    aug, store, _ = setup(args.depth, targets=True)
-    names = {"online": (False, None), "online_targets": (True, None)}
+    aug, store, _ = setup(args.depth, targets=True, target_points=args.target_points)
+    names = {"online": (False, None, None), "online_targets": (True, None, None)}
     if args.world_aug:
-        names["online_targets_world"] = (True, WorldAug())
+        names["online_targets_world"] = (True, WorldAug(), None)
+    if args.target_points is not None:
+        names["online_targets_points"] = (True, None, args.target_points)
     per_epoch = N_STORE // BATCH
     n_epochs = -(-args.batches // per_epoch)
     out = {"card": card(), "store_scans": N_STORE, "batch": BATCH, "rounds": args.rounds}
-    for name, (t, w) in names.items():                  # warm every variant
-        set_variant(aug, t, w)
+    for name, (t, w, k) in names.items():               # warm every variant
+        set_variant(aug, t, w, k)
         for _ in aug.epochs(range(10_000, 10_000 + -(-args.warmup // per_epoch))):
             pass
     torch.cuda.synchronize()
     rates_by = {k: [] for k in names}
     epoch = 0
     for _ in range(args.rounds):
-        for name, (t, w) in names.items():
-            set_variant(aug, t, w)
+        for name, (t, w, k) in names.items():
+            set_variant(aug, t, w, k)
             torch.cuda.synchronize()
             t0 = time.perf_counter()
             n = 0
@@ -111,7 +120,66 @@ def variants(args):
         out[name + "_median"] = float(np.median(r))
     for name in names:
         out[name + "_over_online"] = out[name + "_median"] / out["online_median"]
+    if args.target_points is not None:
+        out["online_targets_points_over_targets"] = out["online_targets_points_median"] / out["online_targets_median"]
+        out.update(target_points_measure(aug, store, args.target_points))
     aug.close()
+    return out
+
+
+def copy_peak():
+    """Bytes per second of a device-to-device copy of 2 GiB (read + write) on this card."""
+    import torch
+    src = torch.empty(1 << 31, dtype=torch.uint8, device="cuda")
+    dst = torch.empty_like(src)
+    dst.copy_(src)
+    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    ev0.record()
+    for _ in range(10):
+        dst.copy_(src)
+    ev1.record()
+    torch.cuda.synchronize()
+    return 10 * 2 * src.numel() / (ev0.elapsed_time(ev1) * 1e-3)
+
+
+def target_points_measure(aug, store, k):
+    """Kernel times of the points-in-targets variant and the scene targets that lost points (see the module doc)."""
+    import torch
+    from oracle.target_points import points_in_boxes
+    set_variant(aug, True, None, k)
+    rows = []
+    for b in aug.epoch(97):
+        rows.append(int(b.offsets[-1]))
+    torch.cuda.synchronize()
+    kern, n_batches = kernel_times(aug, 96)
+    copy_bps = copy_peak()
+    us = {name: float(np.mean(v)) for name, v in kern.items()}
+    rows_per_batch = float(np.mean(rows))
+    tp_bps = rows_per_batch * 20 / (us["k_target_points"] * 1e-6)
+    out = {"target_points_k": k, "target_points_kernels_us_per_launch": {n: {"mean": us[n], "launches": len(kern[n])}
+                                                                       for n in kern if n.startswith("k_target")},
+           "target_points_us_per_batch": sum(us[n] * len(kern[n]) for n in kern if n.startswith("k_target")) / n_batches,
+           "output_rows_per_batch": rows_per_batch, "k_target_points_bytes_per_s": tp_bps, "copy_peak_bytes_per_s": copy_bps,
+           "k_target_points_over_copy_peak": tp_bps / copy_bps}
+    # scene targets of one epoch (counts only, no filter) against the same boxes on the raw store scans
+    set_variant(aug, True, None, 0)
+    n_scene = went_down = to_zero = below_k = 0
+    for b in aug.epoch(95):
+        n_gt, n_ins = b.n_gt.cpu().numpy(), b.n_inserted.cpu().numpy()
+        gp, gb = b.gt_points.cpu().numpy(), b.gt_boxes.cpu().numpy()
+        for s, i in enumerate(b.indices):
+            m = int(n_gt[s] - n_ins[s])
+            if m == 0:
+                continue
+            a, e = int(store.h_point_offsets[i]), int(store.h_point_offsets[i + 1])
+            raw = points_in_boxes(store.xyzi[a:e, :3].cpu().numpy(), gb[s, :m]).sum(axis=0)
+            aug_c = gp[s, :m]
+            n_scene += m
+            went_down += int((aug_c < raw).sum())
+            to_zero += int(((aug_c == 0) & (raw > 0)).sum())
+            below_k += int(((aug_c < k) & (raw >= k)).sum())
+    out.update(scene_targets=n_scene, scene_fraction_fewer_points=went_down / max(n_scene, 1),
+               scene_fraction_emptied=to_zero / max(n_scene, 1), scene_fraction_fell_below_k=below_k / max(n_scene, 1))
     return out
 
 
@@ -177,18 +245,7 @@ def profile(args):
     for _ in aug.epoch(99):
         pass
     torch.cuda.synchronize()
-    # copy peak of this card: a device-to-device copy of 2 GiB (read + write)
-    src = torch.empty(1 << 31, dtype=torch.uint8, device="cuda")
-    dst = torch.empty_like(src)
-    dst.copy_(src)
-    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    ev0.record()
-    for _ in range(10):
-        dst.copy_(src)
-    ev1.record()
-    torch.cuda.synchronize()
-    copy_bps = 10 * 2 * src.numel() / (ev0.elapsed_time(ev1) * 1e-3)
-    del src, dst
+    copy_bps = copy_peak()
     n_batches = 0
     with tprofile(activities=[ProfilerActivity.CUDA, ProfilerActivity.CPU]) as prof:
         for b in aug.epoch(0):
@@ -229,7 +286,7 @@ def profile(args):
 
 
 KERNELS = ("k_gather_points", "k_draw_schedule", "k_gather_boxes", "k_gather_scan_meta", "k_inserted_targets", "k_draw_world",
-           "k_gt_targets", "k_out_write")
+           "k_gt_targets", "k_out_write", "k_target_points", "k_target_filter", "k_target_remap")
 
 
 def kernel_times(aug, epoch):
@@ -262,6 +319,8 @@ def main():
     ap.add_argument("--profile", action="store_true")
     ap.add_argument("--targets", action="store_true", help="detection targets for every batch (see the module doc)")
     ap.add_argument("--world-aug", action="store_true", help="world flip / rotation / scaling (WorldAug defaults)")
+    ap.add_argument("--target-points", type=int, default=None, metavar="K",
+                    help="--targets: also batches with points in targets and min_points K (see the module doc)")
     ap.add_argument("--rounds", type=int, default=3, help="--targets: alternations of the variants")
     ap.add_argument("--out", default=None, help="directory for the JSON result (printed either way)")
     args = ap.parse_args()
@@ -270,6 +329,8 @@ def main():
     _lib.require_cuda()
     if args.world_aug and not args.targets and not args.profile:
         ap.error("--world-aug is measured as online + targets + world aug: pass --targets too")
+    if args.target_points is not None and (not args.targets or args.profile or args.target_points < 0):
+        ap.error("--target-points K (K >= 0) is measured against --targets: pass --targets, not --profile")
     res = profile(args) if args.profile else variants(args) if args.targets else rates(args)
     line = json.dumps(res)
     print(line)
@@ -278,6 +339,7 @@ def main():
         name = "bench_online_profile" if args.profile else "bench_online"
         name += "_targets" if args.targets else ""
         name += "_world" if args.world_aug else ""
+        name += f"_points{args.target_points}" if args.target_points is not None else ""
         with open(os.path.join(args.out, name + ".json"), "w") as f:
             f.write(line + "\n")
 
